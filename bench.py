@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ProtoASNet prototype-head hot path on B200 (contract: see DESIGN.md 'Measurement').
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one prototype-head forward (BASELINE config 3: feature map 512x4x7x7 bf16, D=256, P=40, K=4) over a
@@ -11,6 +11,9 @@ region); ``push`` = seconds for one push / prototype projection over 50 000 clip
 (fused similarity+argmin, one NCCL all-reduce(MIN) of packed keys + one all-reduce(SUM) of winner rows).
 ``--impl reference`` times the reference algorithm's CPU port (oracle/, op-for-op the reference's PyTorch ops) on
 the host cores of the box.
+``--dump-outputs DIR`` writes what the last timed step returned (rank 0: logits, similarity, occurrence_map) as
+DIR/<name>.npy in float32 (32 MB for the batch of 1024); inputs and weights are seeded, so two builds can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -210,6 +213,13 @@ def _bind_host_memory_to_gpu_node(dev):
         return None
 
 
+def dump_outputs(directory, outputs):
+    """outputs: (logits, similarity, occurrence_map) as a caller of the head receives them -> DIR/<name>.npy, float32."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in zip(("logits", "similarity", "occurrence_map"), outputs):
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_reference(args, rank):
     from protoasnet_b200 import synth
 
@@ -228,8 +238,10 @@ def run_reference(args, rank):
         t0 = time.perf_counter()
         for _ in range(args.steps):
             for _ in range(sample // 64):
-                fwd(x)
+                out = fwd(x)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     v = args.steps * sample / dt
     what = "the reference's own Video_XProtoNet class (oracle/_ref, identity backbone)" if kind == "reference" else \
         "oracle port of the reference's ops"
@@ -254,7 +266,10 @@ def main():
     ap.add_argument("--push-clips", type=int, default=PUSH_CLIPS)
     ap.add_argument("--no-push", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -318,6 +333,7 @@ def main():
         barrier()
         ms_total = e0.elapsed_time(e1)
         launches = int(lib.pasn_debug_launch_count() - l0)
+        last_out = out
         # dominant kernel, per launch, CUDA events recorded inside the library on the launch stream
         lib.pasn_debug_time_main_kernel(1)
         main_ms = []
@@ -483,6 +499,9 @@ def main():
             push["cpu_baseline"] = {"value": s50, "unit": "s per 50k clips (extrapolated)", "cores": cores, "kind": "port",
                                     "sample": f"restated reference push loop, batch 5, {n_sample} clips in {dt:.1f} s, "
                                               "extrapolated linearly to 50 000"}
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_out)
 
     if rank == 0:
         # whole-head algorithmic FLOPs over the time in which all of them run (the step), against the burst peak for a
