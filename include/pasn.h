@@ -42,7 +42,13 @@ typedef enum {
                              /* everything computed since are invalid                 */
 } pasn_status;
 
-typedef enum { PASN_F32 = 0, PASN_BF16 = 1 } pasn_dtype;
+/* element type of the feature map (and of the occurrence map, which is returned in the same type).
+ * PASN_F16 (torch.autocast's default) runs on the tensor-core families only (fused or tiled, see pasn_path); a shape that only
+ * the generic CUDA-core path takes, or dims.path = PASN_PATH_GENERIC, is refused with PASN_ERR_UNSUPPORTED (and a
+ * workspace size of 0): the CUDA-core path is the fp32 correctness path.  In fp16 mode the feature map is read exactly, the
+ * first-layer weights (add_on_layers.0.weight, occurrence_module.0.weight) are rounded to fp16, and everything after the
+ * first layer is bf16 mode's arithmetic.  An fp16 occurrence map saturates to inf above 65504, as any fp16 tensor does. */
+typedef enum { PASN_F32 = 0, PASN_BF16 = 1, PASN_F16 = 2 } pasn_dtype;
 
 /* memory format of the backbone feature map handed to the head */
 typedef enum {
@@ -56,11 +62,13 @@ typedef enum { PASN_OCC_ABS = 0 } pasn_occ_act;
 
 /* which kernel family computes the head */
 typedef enum {
-  PASN_PATH_AUTO = 0,    /* fused kernel when dims/dtype qualify, else tiled, else generic                      */
-  PASN_PATH_GENERIC = 1, /* CUDA-core FFMA kernels, fp32 accumulate, every shape/dtype                          */
-  PASN_PATH_TCGEN05 = 2, /* fused tcgen05/TMEM token kernel (bf16 operands, fp32 accumulate; D = 256, S >= 128) */
+  PASN_PATH_AUTO = 0,    /* fused kernel when dims/dtype qualify, else tiled, else generic (fp16: never generic) */
+  PASN_PATH_GENERIC = 1, /* CUDA-core FFMA kernels, fp32 accumulate, every shape; fp32 / bf16 only              */
+  PASN_PATH_TCGEN05 = 2, /* fused tcgen05/TMEM token kernel (bf16 operands, fp32 accumulate; D = 256, S >= 128; */
+                         /* fp16 maps: first layer fp16 x fp16)                                                 */
   PASN_PATH_TILED = 3    /* chain of TMA-fed tcgen05 GEMMs: any S / P, D % 128 == 0, C % 64 == 0; bf16 feature   */
-                         /* maps in bf16, fp32 feature maps as a 3-pass bf16 hi/lo split (fp32-grade results)   */
+                         /* maps in bf16, fp16 maps with an fp16 x fp16 first layer, fp32 feature maps as a     */
+                         /* 3-pass bf16 hi/lo split (fp32-grade results)                                        */
 } pasn_path;
 
 typedef struct {
@@ -80,8 +88,8 @@ typedef struct {
  *   add_on_layers.{0,2}.{weight,bias}, occurrence_module.{0,2}.{weight,bias}, occurrence_module.4.weight,
  *   prototype_vectors, last_layer.weight
  * (src/models/Video_XProtoNet.py:27-80; src/models/XProtoNet.py:17-49).  In PASN_BF16 mode the conv
- * weights and biases are rounded to bf16 (round-to-nearest-even) on the fly; prototypes and
- * last_layer always stay fp32. */
+ * weights and biases are rounded to bf16 (round-to-nearest-even) on the fly (PASN_F16 mode: the two first-layer weights
+ * addon_w1 / occ_w1 to fp16, the rest as in bf16 mode); prototypes and last_layer always stay fp32. */
 typedef struct {
   const float* addon_w1; /* [D][C]   */
   const float* addon_b1; /* [D]      */
@@ -122,7 +130,7 @@ int pasn_tcgen05_supported(const pasn_dims* dims);
 /* scratch needed by pasn_head_forward / pasn_occurrence_only for these dims */
 size_t pasn_head_workspace_bytes(const pasn_dims* dims);
 
-/* size of / fill the derived bf16 weight cache of the tensor-core path that serves these dims (fused: stage images in
+/* size of / fill the derived bf16 (fp16 mode: first layer fp16) weight cache of the tensor-core path that serves these dims (fused: stage images in
  * shared-memory byte order; tiled: row-major bf16 planes); depends on dims.dtype and dims.path; never saved in checkpoints */
 size_t pasn_packed_weights_bytes(const pasn_dims* dims);
 int pasn_pack_weights(const pasn_weights* w, const pasn_dims* dims, void* packed, void* stream);
@@ -152,10 +160,11 @@ int pasn_occurrence_only(const void* feat, const pasn_weights* w, const void* pa
 /* Backward of the head (training: loss.backward() through Video_XProtoNet.forward, src/agents/XProtoNet_Base.py:397,
  * src/agents/Video_XProtoNet_e2e.py:138, and through compute_occurence_map, src/loss/loss.py:302).  Forward
  * intermediates are recomputed, nothing has to be saved by the forward call.  Gradients of the fp32 formulation on the
- * given inputs (a bf16 feature map is read exactly, weights are not rounded); sub-gradients as in PyTorch (relu'(0) = 0,
+ * given inputs (a bf16 or fp16 feature map is read exactly, weights are not rounded); sub-gradients as in PyTorch (relu'(0) = 0,
  * d|x|/dx(0) = 0, clamped norms constant).  Shapes the tiled path takes (C % 64 = 0, D % 128 = 0) run on the tensor cores
  * as three-pass bf16 hi/lo GEMMs (fp32-grade products, fp32 accumulation) unless dims.path is PASN_PATH_GENERIC; the
- * rest runs on fp32 CUDA-core kernels.  grad_logits = grad_similarity = NULL: only the occurrence branch is recomputed
+ * rest runs on fp32 CUDA-core kernels.  fp16 feature maps take the tensor-core chain only (PASN_ERR_UNSUPPORTED and a
+ * workspace size of 0 otherwise).  grad_logits = grad_similarity = NULL: only the occurrence branch is recomputed
  * and differentiated (backward of pasn_occurrence_only); the other parameter gradients are left untouched.
  *   grad_logits      [N,K] fp32 or NULL     grad_similarity [N,P] fp32 or NULL     grad_occurrence [N,P,S] fp32 or NULL
  *   grads            every pointer non-NULL, same shapes as pasn_weights; gradients are ADDED to the buffers
@@ -182,7 +191,7 @@ int pasn_similarity_stats(const float* similarity, const int64_t* labels, int32_
                           int32_t n_specific, int32_t top_specific, int32_t top_rest, float* class_max, int32_t* class_arg,
                           double* sums, uint64_t* counts, double* sim_cumsum, void* stream);
 /* sum[0] += sum over rows of ||occ[row, 0:S]||_p (p = 1 or 2; L_norm over the spatial dims, src/loss/loss.py:236-250);
- * row_norm[row] = that norm (or NULL).  occ is [rows][S] in `dtype`. */
+ * row_norm[row] = that norm (or NULL).  occ is [rows][S] in `dtype` (any pasn_dtype). */
 int pasn_occurrence_lnorm(const void* occ, int32_t dtype, int64_t rows, int32_t S, int32_t p, double* sum, float* row_norm,
                           void* stream);
 

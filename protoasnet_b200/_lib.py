@@ -9,10 +9,12 @@ import ctypes as C
 import os
 from typing import Optional
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpasn_b200.so")
 
-PASN_F32, PASN_BF16 = 0, 1
+PASN_F32, PASN_BF16, PASN_F16 = 0, 1, 2
 PASN_LAYOUT_NCS, PASN_LAYOUT_NSC = 0, 1
 PASN_OCC_ABS = 0
 PASN_PATH_AUTO, PASN_PATH_GENERIC, PASN_PATH_TCGEN05, PASN_PATH_TILED = 0, 1, 2, 3
@@ -28,6 +30,10 @@ SYMBOLS = [
     "pasn_head_backward_workspace_bytes", "pasn_head_backward", "pasn_similarity_stats", "pasn_occurrence_lnorm",
     "pasn_debug_tc_gemm_desc_bytes", "pasn_debug_tc_gemm", "pasn_debug_set_gemm_trace",
 ]
+
+
+# torch dtype -> pasn_dtype of the feature / occurrence maps the library takes
+DTYPES = {torch.float32: PASN_F32, torch.bfloat16: PASN_BF16, torch.float16: PASN_F16}
 
 
 class PasnDims(C.Structure):

@@ -8,7 +8,7 @@ static bool dims_ok(const pasn_dims* d) {
   if (!d) return false;
   if (d->N < 0 || d->C <= 0 || d->D <= 0 || d->P <= 0 || d->K <= 0 || d->S <= 0) return false;
   if (d->D % 2 != 0) return false;  // occurrence_module hidden width is D // 2
-  if (d->dtype != PASN_F32 && d->dtype != PASN_BF16) return false;
+  if (d->dtype != PASN_F32 && d->dtype != PASN_BF16 && d->dtype != PASN_F16) return false;
   if (d->layout != PASN_LAYOUT_NCS && d->layout != PASN_LAYOUT_NSC) return false;
   if (d->occ_act != PASN_OCC_ABS) return false;
   if (d->path < PASN_PATH_AUTO || d->path > PASN_PATH_TILED) return false;
@@ -16,9 +16,16 @@ static bool dims_ok(const pasn_dims* d) {
 }
 
 // which kernel family serves these dims: 0 generic, 1 fused token kernel, 2 tiled GEMM chain; *err when an explicitly
-// requested family cannot run them
+// requested family cannot run them.  fp16 feature maps are served by the tensor-core families only (the CUDA-core path is
+// the fp32 correctness path): without one of them *err is PASN_ERR_UNSUPPORTED.
 enum { FAM_GENERIC = 0, FAM_FUSED = 1, FAM_TILED = 2 };
+static int resolve_family_any(const pasn_dims& d, int* err);
 static int resolve_family(const pasn_dims& d, int* err) {
+  const int fam = resolve_family_any(d, err);
+  if (d.dtype == PASN_F16 && fam == FAM_GENERIC) *err = PASN_ERR_UNSUPPORTED;
+  return fam;
+}
+static int resolve_family_any(const pasn_dims& d, int* err) {
   *err = PASN_OK;
   switch (d.path) {
     case PASN_PATH_GENERIC: return FAM_GENERIC;
@@ -102,17 +109,20 @@ extern "C" int pasn_similarity_stats(const float* similarity, const int64_t* lab
 extern "C" int pasn_occurrence_lnorm(const void* occ, int32_t dtype, int64_t rows, int32_t S, int32_t p, double* sum,
                                      float* row_norm, void* stream) {
   if (rows < 0 || S <= 0 || !sum || (rows > 0 && !occ)) return PASN_ERR_INVALID;
-  if (dtype != PASN_F32 && dtype != PASN_BF16) return PASN_ERR_INVALID;
+  if (dtype != PASN_F32 && dtype != PASN_BF16 && dtype != PASN_F16) return PASN_ERR_INVALID;
   return launch_occ_lnorm(occ, dtype, rows, S, p, sum, row_norm, reinterpret_cast<cudaStream_t>(stream));
 }
 
+// fp16 feature maps: tensor-core backward only
+static bool backward_ok(const pasn_dims* d) { return dims_ok(d) && (d->dtype != PASN_F16 || tiled_backward_supported(*d)); }
 extern "C" size_t pasn_head_backward_workspace_bytes(const pasn_dims* dims) {
-  return dims_ok(dims) ? backward_workspace_bytes(*dims) : 0;
+  return backward_ok(dims) ? backward_workspace_bytes(*dims) : 0;
 }
 extern "C" int pasn_head_backward(const void* feat, const pasn_weights* w, const pasn_dims* dims, const float* grad_logits,
                                   const float* grad_similarity, const float* grad_occurrence, const pasn_grads* grads,
                                   float* grad_feat, void* workspace, size_t workspace_bytes, void* stream) {
   if (!dims_ok(dims) || !w || !grads) return PASN_ERR_INVALID;
+  if (!backward_ok(dims)) return PASN_ERR_UNSUPPORTED;
   if (faulted()) return PASN_ERR_FAULT;
   if (dims->N == 0) return PASN_OK;
   if (!feat || !workspace) return PASN_ERR_INVALID;
@@ -160,15 +170,17 @@ extern "C" const char* pasn_strerror(int status) {
 extern "C" int pasn_tcgen05_supported(const pasn_dims* dims) {
   if (!dims_ok(dims)) return 0;
   int err;
-  return resolve_family(*dims, &err) != FAM_GENERIC ? 1 : 0;
+  const int fam = resolve_family(*dims, &err);
+  return fam != FAM_GENERIC && err == PASN_OK ? 1 : 0;
 }
 
 extern "C" size_t pasn_head_workspace_bytes(const pasn_dims* dims) {
   if (!dims_ok(dims)) return 0;
   int err;
   const int fam = resolve_family(*dims, &err);
+  if (dims->dtype == PASN_F16 && err) return 0;   // no family can run them
   size_t need = generic_workspace_bytes(*dims);   // the generic path stays available as the NULL-`packed` fallback
-  if (dims->path == PASN_PATH_TCGEN05 || dims->path == PASN_PATH_TILED) need = 0;
+  if (dims->path == PASN_PATH_TCGEN05 || dims->path == PASN_PATH_TILED || dims->dtype == PASN_F16) need = 0;
   if (fam == FAM_FUSED) { const size_t t = sm100_workspace_bytes(*dims); need = t > need ? t : need; }
   if (fam == FAM_TILED) {   // (pasn_occurrence_only runs in the same family as the forward)
     const size_t t = tiled_workspace_bytes(*dims);
@@ -207,7 +219,7 @@ extern "C" int pasn_head_forward(const void* feat, const pasn_weights* w, const 
   int fam = resolve_family(*dims, &err);
   if (err) return err;
   if (fam != FAM_GENERIC && packed == nullptr) {
-    if (dims->path != PASN_PATH_AUTO) return PASN_ERR_UNSUPPORTED;
+    if (dims->path != PASN_PATH_AUTO || dims->dtype == PASN_F16) return PASN_ERR_UNSUPPORTED;
     fam = FAM_GENERIC;
   }
   if (fam == FAM_FUSED)
@@ -230,7 +242,7 @@ extern "C" int pasn_occurrence_only(const void* feat, const pasn_weights* w, con
   int fam = resolve_family(*dims, &err);   // same family (and therefore the same packed weights) as pasn_head_forward
   if (err) return err;
   if (fam != FAM_GENERIC && packed == nullptr) {
-    if (dims->path != PASN_PATH_AUTO) return PASN_ERR_UNSUPPORTED;
+    if (dims->path != PASN_PATH_AUTO || dims->dtype == PASN_F16) return PASN_ERR_UNSUPPORTED;
     fam = FAM_GENERIC;
   }
   if (fam == FAM_FUSED)

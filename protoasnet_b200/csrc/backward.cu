@@ -244,8 +244,9 @@ int head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, c
   s.Opre = q; q += PS * nbm; s.O = q; q += PS * nbm;    s.FE = q; q += PD * nbm;   s.gFE = q; q += PD * nbm;
   s.gO = q; q += PS * nbm;   s.gF = q; q += DS * nbm;   s.gH1 = q; q += DS * nbm;  s.gG2 = q; q += D2S * nbm;
   s.gG1 = q;
+  if (d.dtype == PASN_F16) return PASN_ERR_UNSUPPORTED;   // fp16 feature maps: tensor-core backward only
   const bool xbf = d.dtype == PASN_BF16;
-  const size_t elt = xbf ? 2 : 4;
+  const size_t elt = dtype_bytes(d.dtype);
   // strides of the feature map seen as B[k = channel][n = voxel] per clip
   const long long x_sk = d.layout == PASN_LAYOUT_NSC ? 1 : S, x_sn = d.layout == PASN_LAYOUT_NSC ? C : 1;
 

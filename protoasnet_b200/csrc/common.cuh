@@ -1,6 +1,7 @@
 // Shared device/host helpers for libpasn_b200 (sm_100a only).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -16,12 +17,17 @@ namespace pasn {
 __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// bytes per element of a feature / occurrence map of this pasn_dtype (the one place that knows the element sizes)
+__host__ __device__ inline size_t dtype_bytes(int dtype) { return dtype == PASN_F32 ? 4 : 2; }
+
 template <typename T>
 __device__ __forceinline__ float to_f32(T v);
 template <>
 __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <>
 __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <>
+__device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }
 
 __device__ __forceinline__ float round_bf16(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 

@@ -152,6 +152,7 @@ size_t generic_workspace_bytes(const pasn_dims& d) {
 int generic_head_forward(const void* feat, const pasn_weights& w, const pasn_dims& d, float* logits, float* sim,
                          void* occ, float* feats, float* dist, const pasn_push_args* push, void* ws, size_t ws_bytes,
                          cudaStream_t st) {
+  if (d.dtype == PASN_F16) return PASN_ERR_UNSUPPORTED;   // the CUDA-core path is the fp32 / bf16 correctness path
   if (ws_bytes < generic_workspace_bytes(d)) return PASN_ERR_WORKSPACE;
   const int nb_max = chunk_clips(d);
   const int D2 = d.D / 2;
@@ -160,7 +161,7 @@ int generic_head_forward(const void* feat, const pasn_weights& w, const pasn_dim
   float* G2 = F + (size_t)nb_max * d.D * d.S;
   float* O = G2 + (size_t)nb_max * D2 * d.S;
   float* FE = O + (size_t)nb_max * d.P * d.S;
-  const size_t elt = d.dtype == PASN_BF16 ? 2 : 4;
+  const size_t elt = dtype_bytes(d.dtype);
   main_kernel_begin(st);  // generic path: the "dominant kernel" is the whole GEMM chain
   for (int n0 = 0; n0 < d.N; n0 += nb_max) {
     const int nb = (d.N - n0 < nb_max) ? d.N - n0 : nb_max;
@@ -202,12 +203,13 @@ int generic_head_forward(const void* feat, const pasn_weights& w, const pasn_dim
 
 int generic_occurrence_only(const void* feat, const pasn_weights& w, const pasn_dims& d, void* occ, void* ws,
                             size_t ws_bytes, cudaStream_t st) {
+  if (d.dtype == PASN_F16) return PASN_ERR_UNSUPPORTED;   // the CUDA-core path is the fp32 / bf16 correctness path
   if (ws_bytes < generic_workspace_bytes(d)) return PASN_ERR_WORKSPACE;
   const int nb_max = chunk_clips(d);
   const int D2 = d.D / 2;
   float* H = reinterpret_cast<float*>(ws);
   float* G2 = H + (size_t)2 * nb_max * d.D * d.S;
-  const size_t elt = d.dtype == PASN_BF16 ? 2 : 4;
+  const size_t elt = dtype_bytes(d.dtype);
   for (int n0 = 0; n0 < d.N; n0 += nb_max) {
     const int nb = (d.N - n0 < nb_max) ? d.N - n0 : nb_max;
     const char* x = reinterpret_cast<const char*>(feat) + (size_t)n0 * d.C * d.S * elt;

@@ -399,9 +399,10 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
 }
 
 // =================================================================================================
-// weight packing: fp32 state_dict tensors -> bf16 stage images in the exact smem byte order
+// weight packing: fp32 state_dict tensors -> bf16 stage images in the exact smem byte order (f16: the layer-1 images W3 / W1
+// in fp16, the operand type of an fp16 feature map)
 // =================================================================================================
-__global__ void pack_weights_kernel(pasn_weights w, int C, int P, uint8_t* out) {
+__global__ void pack_weights_kernel(pasn_weights w, int C, int P, int f16, uint8_t* out) {
   const PackedLayout PL = packed_layout(C);
   const int nkc = C / 64;
   const size_t n_l1 = (size_t)2 * nkc * 256 * 64, n_w4 = (size_t)4 * 128 * 64, n_w5 = (size_t)2 * 64 * 64;
@@ -413,7 +414,9 @@ __global__ void pack_weights_kernel(pasn_weights w, int C, int P, uint8_t* out) 
       const int stage = (int)(j / (256 * 64)), e = (int)(j % (256 * 64));
       const int r = e / 64, k = e % 64, kc = stage >> 1, pass = stage & 1;
       const float v = (pass ? w.addon_w1 : w.occ_w1)[(size_t)r * C + kc * 64 + k];
-      *reinterpret_cast<__nv_bfloat16*>(out + PL.off_l1 + (size_t)stage * 32768 + off_kmajor_sw128(r, k)) = __float2bfloat16_rn(v);
+      uint8_t* dst = out + PL.off_l1 + (size_t)stage * 32768 + off_kmajor_sw128(r, k);
+      if (f16) *reinterpret_cast<__half*>(dst) = __float2half_rn(v);
+      else *reinterpret_cast<__nv_bfloat16*>(dst) = __float2bfloat16_rn(v);
       continue;
     }
     j -= n_l1;
@@ -479,9 +482,10 @@ void sm100_set_k1_variant(int variant) { g_k1_variant = variant; }
 
 bool sm100_supported(const pasn_dims& d) {
   // fp32 feature maps take the fused path only on explicit request (bf16 compute: inputs are rounded on the fly)
-  // channels_last ([N,S,C]) feature maps: bf16 only
-  if (d.layout != PASN_LAYOUT_NCS && !(d.layout == PASN_LAYOUT_NSC && d.dtype == PASN_BF16)) return false;
-  if (d.dtype != PASN_BF16 && !(d.dtype == PASN_F32 && d.path == PASN_PATH_TCGEN05)) return false;
+  // channels_last ([N,S,C]) feature maps: bf16 and fp16 only
+  const bool half = d.dtype == PASN_BF16 || d.dtype == PASN_F16;
+  if (d.layout != PASN_LAYOUT_NCS && !(d.layout == PASN_LAYOUT_NSC && half)) return false;
+  if (!half && !(d.dtype == PASN_F32 && d.path == PASN_PATH_TCGEN05)) return false;
   if (d.D != DD) return false;
   if (d.C % 64 != 0 || d.C < 64 || d.C > 1024) return false;
   if (d.P < 1 || d.P > PP_MAX) return false;
@@ -556,7 +560,7 @@ __global__ void sum_groups_kernel(const float* __restrict__ fev, float* __restri
 
 int sm100_pack_weights(const pasn_weights& w, const pasn_dims& d, void* packed, cudaStream_t st) {
   if (((uintptr_t)packed & 15) != 0) return PASN_ERR_ALIGN;
-  pack_weights_kernel<<<148 * 4, 256, 0, st>>>(w, d.C, d.P, reinterpret_cast<uint8_t*>(packed));
+  pack_weights_kernel<<<148 * 4, 256, 0, st>>>(w, d.C, d.P, d.dtype == PASN_F16 ? 1 : 0, reinterpret_cast<uint8_t*>(packed));
   PASN_LAUNCH_CHECK();
   count_launch();
   return PASN_OK;
@@ -588,6 +592,7 @@ int sm100_head_forward(const void* feat, const pasn_weights& w, const void* pack
   }();
   K1Params k1{};
   k1.f32_in = d.dtype == PASN_F32;
+  k1.f16_in = d.dtype == PASN_F16;
   k1.nsc = d.layout == PASN_LAYOUT_NSC;
   k1.feat = reinterpret_cast<const __nv_bfloat16*>(feat);
   k1.feat32 = reinterpret_cast<const float*>(feat);

@@ -73,10 +73,12 @@ __device__ __forceinline__ void split_points(int nkc, int& a1, int& a2) {  // wh
 // Everything that is fixed per launch is a template parameter: the kernel is ~7 k instructions for five warp roles, and code
 // of orders / input kinds / experiments that do not run still spreads the ones that do over more instruction-cache lines
 // (ncu: 8 % of the issue slots lost to instruction fetch before; serial bf16 NCDHW instantiation 8256 -> ~5.5 k instructions).
-// IN: 0 = bf16 [N,C,S], 1 = bf16 channels_last [N,S,C], 2 = fp32 [N,C,S] (rounded to bf16 on the fly).
+// IN: 0 = bf16 [N,C,S], 1 = bf16 channels_last [N,S,C], 2 = fp32 [N,C,S] (rounded to bf16 on the fly), 3 = fp16 [N,C,S],
+// 4 = fp16 channels_last.  fp16 maps are gathered byte for byte like bf16 ones; only the layer-1 MMAs (fp16 x fp16 against
+// fp16 weight images: kind::f16 takes no mixed fp16 / bf16 operands) and the map store differ.
 template <int PP, bool TRACE, bool TWO_PHASE, int IN>
 __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Params p) {
-  constexpr bool nsc = IN == 1, f32_in = IN == 2;
+  constexpr bool nsc = IN == 1 || IN == 4, f32_in = IN == 2, f16_in = IN == 3 || IN == 4;
   const int dbg_skip = PASN_K1_EXPERIMENTS ? p.dbg_skip : 0, x_drain = PASN_K1_EXPERIMENTS ? p.x_drain : 0,
             flush_sleep = PASN_K1_EXPERIMENTS ? p.flush_sleep : 0, flush_kmajor = PASN_K1_EXPERIMENTS ? p.flush_kmajor : 1,
             l2_hints = PASN_K1_EXPERIMENTS ? p.l2_hints : 1;
@@ -169,8 +171,9 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       };
       // X tile: MN-major (voxels contiguous) for NCDHW input, K-major (channels contiguous) for channels_last input
       const uint32_t x_mn = nsc ? 0u : 1u;
-      const uint32_t idesc_g = make_idesc_bf16(128, 256, x_mn, 0);    // A = X tile, B = W3 chunk (K-major)
-      const uint32_t idesc_a = make_idesc_bf16(128, 128, 0, x_mn);    // A = W1 half chunk (K-major), B = X tile
+      // A = X tile, B = W3 chunk (K-major) / A = W1 half chunk (K-major), B = X tile; fp16 maps: both operands fp16
+      const uint32_t idesc_g = f16_in ? make_idesc_16(128, 256, 0, 0, x_mn, 0) : make_idesc_bf16(128, 256, x_mn, 0);
+      const uint32_t idesc_a = f16_in ? make_idesc_16(128, 128, 0, 0, 0, x_mn) : make_idesc_bf16(128, 128, 0, x_mn);
       const uint32_t xk = nsc ? 2u : 128u;                          // descriptor advance per K step of 16 channels
       const uint32_t idesc_g2 = make_idesc_bf16(128, 128, 0, 0);
       const uint32_t idesc_o = make_idesc_bf16(128, 64, 0, 0);
@@ -637,7 +640,12 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
             const int vc = c_begin + clipl, rc = vc / p.G, vg = vc - rc * p.G;
             const size_t o0 = ((size_t)rc * p.P) * p.SR + (size_t)vg * S + s;
             const unsigned char* src = os + off_mnmajor_nosw(slot * PP, tok, NPOOL);
-            if (!f32_in) {
+            if constexpr (f16_in) {   // O is bf16 in Os; the map leaves in the feature map's type
+              __half* orow = reinterpret_cast<__half*>(p.occ) + o0;
+#pragma unroll 8
+              for (int pp = 0; pp < p.P; ++pp)
+                orow[(size_t)pp * p.SR] = __float2half_rn(__bfloat162float(*reinterpret_cast<const __nv_bfloat16*>(src + (pp >> 3) * 128 + (pp & 7) * 2)));
+            } else if (!f32_in) {
               __nv_bfloat16* orow = p.occ + o0;
 #pragma unroll 8
               for (int pp = 0; pp < p.P; ++pp)
@@ -975,9 +983,11 @@ static int launch_inst(const K1Params& k1, int grid, cudaStream_t st) {
 template <int PP>
 static int launch_one(const K1Params& k1, int grid, cudaStream_t st) {
   // The instrumented instantiation (clock reads on the issue path) only runs while a trace buffer is installed.  The
-  // two-phase order (an A/B variant, slower) and the trace exist for bf16 maps; fp32 maps always run the plain serial kernel.
+  // two-phase order (an A/B variant, slower) and the trace exist for bf16 maps; fp32 and fp16 maps always run the plain
+  // serial kernel.
   const bool tr = k1.trace != nullptr;
   if (k1.f32_in) return launch_inst<PP, false, false, 2>(k1, grid, st);
+  if (k1.f16_in) return k1.nsc ? launch_inst<PP, false, false, 4>(k1, grid, st) : launch_inst<PP, false, false, 3>(k1, grid, st);
   if (k1.nsc) return tr ? launch_inst<PP, true, false, 1>(k1, grid, st) : launch_inst<PP, false, false, 1>(k1, grid, st);
   if (k1.phases != 1) return tr ? launch_inst<PP, true, true, 0>(k1, grid, st) : launch_inst<PP, false, true, 0>(k1, grid, st);
   return tr ? launch_inst<PP, true, false, 0>(k1, grid, st) : launch_inst<PP, false, false, 0>(k1, grid, st);

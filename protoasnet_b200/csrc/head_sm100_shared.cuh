@@ -37,7 +37,7 @@ struct K1Params {
   const float* feat32;         // same buffer seen as fp32 when f32_in (bf16-compute mode for fp32 feature maps)
   float* occ32;                // occurrence map as fp32 when f32_in
   int f32_in;
-  int nsc;                     // feature map is [N][S][C] (channels_last): two-phase kernel file only, bf16 only
+  int nsc;                     // feature map is [N][S][C] (channels_last): bf16 or fp16
   const uint8_t* packed;
   __nv_bfloat16* occ;          // [N][P][S] or null
   uint8_t* feimg;              // K2 operand images, FE_TILE_BYTES per K2 tile
@@ -61,6 +61,7 @@ struct K1Params {
   int flush_sleep;             // ns slept after every fourth prototype row of a clip flush (0: none)
   int x_drain;                 // 1: feature-gather warps publish everything in flight before they block on a full ring
   int spin;                    // Ctx::spin
+  int f16_in;                  // fp16 feature map (read as it is; layer-1 MMAs fp16 x fp16 with fp16 weight images), map in fp16
 };
 
 // 1: build the timing experiments of profiles/README.md into the fused kernels (PASN_DBG_SKIP, PASN_X_DRAIN, PASN_FLUSH_SLEEP,

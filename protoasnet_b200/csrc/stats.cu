@@ -134,7 +134,9 @@ int launch_occ_lnorm(const void* occ, int dtype, long long rows, int S, int p, d
   if (rows <= 0) return PASN_OK;
   if (p != 1 && p != 2) return PASN_ERR_INVALID;
   const unsigned grid = (unsigned)((rows + 7) / 8);
-  if (dtype == PASN_BF16)
+  if (dtype == PASN_F16)
+    occ_lnorm_kernel<__half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(occ), rows, S, p, sums, row_norm);
+  else if (dtype == PASN_BF16)
     occ_lnorm_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(occ), rows, S, p, sums, row_norm);
   else
     occ_lnorm_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(occ), rows, S, p, sums, row_norm);

@@ -131,7 +131,9 @@ enum {
   E_BIT_DIRECT = 8,   // plain stores (unaligned / channel-major outputs), two outputs split between the warp groups
   E_BIT_OUT = 16,     // any output at all
   E_BIT_ABSOUT = 32,  // |value| on the second output
+  E_BIT_F16 = 64,     // fp16 outputs (OUT_F16): only in the instantiation that needs them, the others keep their code
   EPI_FULL = 63,
+  EPI_F16 = EPI_FULL | E_BIT_F16,
   EPI_LEAN = E_BIT_OUT,                   // bias / rank-1 term / activation, TMA-stored outputs
   EPI_STAT = E_BIT_STAT,                  // no output, row statistics only
   EPI_DIRECT = E_BIT_OUT | E_BIT_DIRECT,
@@ -143,7 +145,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
   constexpr bool PAIR = MODE >= 1, QUAD = MODE == 2;
   constexpr bool E_AUX = (EPI & E_BIT_AUX) != 0, E_PSUM = (EPI & E_BIT_PSUM) != 0, E_STAT = (EPI & E_BIT_STAT) != 0,
                  E_DIRECT = (EPI & E_BIT_DIRECT) != 0, E_OUT = (EPI & E_BIT_OUT) != 0, E_ABSOUT = (EPI & E_BIT_ABSOUT) != 0,
-                 E_SPLIT = E_DIRECT;
+                 E_SPLIT = E_DIRECT, E_F16 = (EPI & E_BIT_F16) != 0;
   extern __shared__ __align__(1024) unsigned char smem[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BAR);
   uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + SM_MISC);
@@ -281,7 +283,8 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
   } else if (warp == 1 && rank == 0) {
     // ------------------------------------------------------------------ MMA issuer (leader CTA of a pair)
     if (elect_one()) {
-      const uint32_t id = make_idesc_16(BMP, (uint32_t)bn, 1u, 1u, g.a_mn_major ? 1u : 0u, g.b_mn_major ? 1u : 0u);
+      const uint32_t ab_bf16 = g.ab_f16 ? 0u : 1u;   // one element type for both operands (launch() checks npass == 1)
+      const uint32_t id = make_idesc_16(BMP, (uint32_t)bn, ab_bf16, ab_bf16, g.a_mn_major ? 1u : 0u, g.b_mn_major ? 1u : 0u);
       auto mma = [&](uint32_t d, uint32_t alo, uint32_t ahi, uint32_t blo, uint32_t bhi, uint32_t acc) {
         if constexpr (PAIR) mma_ss2_x(d, alo, ahi, blo, bhi, id, acc);
         else mma_ss_x(d, alo, ahi, blo, bhi, id, acc);
@@ -390,7 +393,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
     int i = 0;
     // one 64-column group of one output leaves through the staging slab(s) + TMA store(s)
     auto store_tma = [&](const Output& o, int mi, const float (&v)[64], int col0, int row0, int b) {
-      const int nbox = o.mode == OUT_BF16 ? 1 : 2;
+      const int nbox = (o.mode == OUT_BF16 || (E_F16 && o.mode == OUT_F16)) ? 1 : 2;
 #pragma unroll
       for (int bx = 0; bx < 2; ++bx) {
         if (bx >= nbox) break;
@@ -405,6 +408,18 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
             asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v[32 * bx + 4 * c]),
                          "f"(v[32 * bx + 4 * c + 1]), "f"(v[32 * bx + 4 * c + 2]), "f"(v[32 * bx + 4 * c + 3])
                          : "memory");
+          }
+        } else if (E_F16 && o.mode == OUT_F16) {
+#pragma unroll
+          for (int c = 0; c < 8; ++c) {
+            uint32_t pk[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const __half2 h2 = __floats2half2_rn(v[8 * c + 2 * j], v[8 * c + 2 * j + 1]);
+              pk[j] = *reinterpret_cast<const uint32_t*>(&h2);
+            }
+            const uint32_t a = rowaddr + (uint32_t)((c ^ (lane & 7)) << 4);
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(pk[0]), "r"(pk[1]), "r"(pk[2]), "r"(pk[3]) : "memory");
           }
         } else if (o.mode == OUT_BF16_HILO && bx == 1) {
 #pragma unroll
@@ -461,6 +476,11 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
           for (int j = 0; j < 64; ++j)
             if (j < nv) p[j * cstep] = v[j];
         }
+      } else if (E_F16 && o.mode == OUT_F16) {
+        __half* p = reinterpret_cast<__half*>(o.ptr) + base + (long long)col0 * cstep;
+#pragma unroll
+        for (int j = 0; j < 64; ++j)
+          if (j < nv) p[j * cstep] = __float2half_rn(v[j]);
       } else {
         __nv_bfloat16* p = reinterpret_cast<__nv_bfloat16*>(o.ptr) + base + (long long)col0 * cstep;
         const bool lo = o.mode == OUT_BF16_HILO;
@@ -752,9 +772,12 @@ void set_trace(void* dev_buf) { g_trace = reinterpret_cast<long long*>(dev_buf);
 int launch(const Gemm& g, cudaStream_t st) {
   if (g.M <= 0 || g.N <= 0 || g.K <= 0 || g.batch <= 0) return PASN_OK;
   if (g.npass < 1 || g.npass > 4 || (g.bn != 64 && g.bn != 128 && g.bn != 256)) return PASN_ERR_INVALID;
+  if (g.ab_f16 && g.npass != 1) return PASN_ERR_INVALID;   // fp16 operands have no lo planes
+  const bool f16_out = g.out[0].mode == OUT_F16 || g.out[1].mode == OUT_F16;
   static bool attr_done = false;
   if (!attr_done) {
     const void* fns[] = {(const void*)tc_gemm_kernel<0, EPI_FULL>, (const void*)tc_gemm_kernel<1, EPI_FULL>, (const void*)tc_gemm_kernel<2, EPI_FULL>,
+                         (const void*)tc_gemm_kernel<0, EPI_F16>, (const void*)tc_gemm_kernel<1, EPI_F16>,
                          (const void*)tc_gemm_kernel<0, EPI_LEAN>, (const void*)tc_gemm_kernel<1, EPI_LEAN>,
                          (const void*)tc_gemm_kernel<0, EPI_STAT>, (const void*)tc_gemm_kernel<1, EPI_STAT>,
                          (const void*)tc_gemm_kernel<0, EPI_DIRECT>, (const void*)tc_gemm_kernel<1, EPI_DIRECT>,
@@ -776,7 +799,7 @@ int launch(const Gemm& g, cudaStream_t st) {
   // shape 602 vs 1005: the stage hand-back needs both pairs' commits and the 4-deep ring cannot cover the extra cluster
   // round trip -- so it is opt-in only.
   static const int quad_env = [] { const char* e = getenv("PASN_GEMM_QUAD"); return e ? atoi(e) : 0; }();
-  const bool quad = pair && quad_env != 0 && g.bn == 256 && g.M > 2 * BM;
+  const bool quad = pair && quad_env != 0 && g.bn == 256 && g.M > 2 * BM && !f16_out;
   const int cl = quad ? 4 : (pair ? 2 : 1);
   // tall tiles for long main loops: two sub-tiles per CTA share every B stage (and take both accumulator buffers, so the
   // epilogue no longer overlaps the MMAs -- negligible when K is long): a quarter less L2 -> SM traffic per flop
@@ -806,22 +829,23 @@ int launch(const Gemm& g, cudaStream_t st) {
   }
   const bool split_k = g.k_rows_per_batch > 0;
   if (split_k && !(g.a_mn_major && g.b_mn_major)) return PASN_ERR_INVALID;
+  const CUtensorMapDataType ab_dt = g.ab_f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
   if (!g.a_mn_major) {
-    if (!make_map(&kp.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, g.A, (unsigned long long)g.ka, (unsigned long long)g.M,
+    if (!make_map(&kp.tmA, ab_dt, 2, g.A, (unsigned long long)g.ka, (unsigned long long)g.M,
                   g.a_batched ? g.batch : 1, (unsigned long long)g.lda * 2, (unsigned long long)g.a_bs * 2, BK, BM))
       return PASN_ERR_ALIGN;
   } else {   // [batch][K rows][ka columns], m contiguous: boxes of 64 m x 64 k
-    if (!make_map(&kp.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, g.A, (unsigned long long)g.ka,
+    if (!make_map(&kp.tmA, ab_dt, 2, g.A, (unsigned long long)g.ka,
                   (unsigned long long)(g.a_rows ? g.a_rows : g.K), (g.a_batched && !split_k) ? (g.group > 1 ? g.group_items : g.batch) : 1,
                   (unsigned long long)g.lda * 2, (unsigned long long)g.a_bs * 2, 64, BK))
       return PASN_ERR_ALIGN;
   }
   if (!g.b_mn_major) {
-    if (!make_map(&kp.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, g.B, (unsigned long long)g.kb,
+    if (!make_map(&kp.tmB, ab_dt, 2, g.B, (unsigned long long)g.kb,
                   (unsigned long long)(g.b_rows ? g.b_rows : g.N), g.b_batched ? g.batch : 1, (unsigned long long)g.ldb * 2, (unsigned long long)g.b_bs * 2, BK, (unsigned)(quad ? 64 : (pair ? g.bn / 2 : g.bn))))
       return PASN_ERR_ALIGN;
   } else {   // [batch][K rows][kb columns], n contiguous: boxes of 64 n x 64 k
-    if (!make_map(&kp.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, g.B, (unsigned long long)g.kb,
+    if (!make_map(&kp.tmB, ab_dt, 2, g.B, (unsigned long long)g.kb,
                   (unsigned long long)(g.b_rows ? g.b_rows : g.K), (g.b_batched && !split_k) ? (g.group > 1 ? g.group_items : g.batch) : 1, (unsigned long long)g.ldb * 2, (unsigned long long)g.b_bs * 2, 64, BK))
       return PASN_ERR_ALIGN;
   }
@@ -832,7 +856,8 @@ int launch(const Gemm& g, cudaStream_t st) {
     kp.tmO[2 * mi + 1] = kp.tmA;
     if (o.mode == OUT_NONE || o.trans_S > 0 || !out_aligned(o)) continue;
     const bool f32 = o.mode == OUT_F32;
-    const CUtensorMapDataType dt = f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const CUtensorMapDataType dt = f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                       : (o.mode == OUT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
     const int elt = f32 ? 4 : 2;
     const unsigned long long ncols = o.ncols ? o.ncols : g.N;
     bool okm = make_map(&kp.tmO[2 * mi], dt, elt, o.ptr, ncols, (unsigned long long)g.M, g.batch,
@@ -883,8 +908,8 @@ int launch(const Gemm& g, cudaStream_t st) {
     // (EPI_AUX: fwd+bwd of 256 clips 1.09-1.10 -> 1.06-1.07 ms; at 64 clips the step is launch-bound and moves with the box)
     static const int aux_env = [] { const char* e = getenv("PASN_GEMM_EPI_AUX"); return e ? atoi(e) : 1; }();
     static const int variants[] = {EPI_LEAN, EPI_STAT, EPI_DIRECT, EPI_PSUM, EPI_AUX};
-    int epi = EPI_FULL;
-    if (epi_env && !quad)
+    int epi = f16_out ? EPI_F16 : EPI_FULL;   // (fp16 outputs: the fp16 chain's occurrence-map stores only)
+    if (epi_env && !quad && !f16_out)
       for (int v : variants)
         if ((v & need) == need && (v != EPI_AUX || aux_env)) { epi = v; break; }
     cudaError_t e;
@@ -895,6 +920,7 @@ int launch(const Gemm& g, cudaStream_t st) {
     else if (epi == EPI_DIRECT) e = TCG_LAUNCH(EPI_DIRECT);
     else if (epi == EPI_PSUM) e = TCG_LAUNCH(EPI_PSUM);
     else if (epi == EPI_AUX) e = TCG_LAUNCH(EPI_AUX);
+    else if (epi == EPI_F16) e = TCG_LAUNCH(EPI_F16);
     else e = TCG_LAUNCH(EPI_FULL);
 #undef TCG_LAUNCH
     if (e != cudaSuccess) return PASN_ERR_CUDA;

@@ -5,7 +5,8 @@
 // with bf16 operands, fp32 accumulation in TMEM, and up to four operand passes: the hi/lo split for fp32 inputs,
 // x*w = (xh + xl)(wh + wl) with xh = bf16(x), xl = bf16(x - xh) -- 16 significant bits per operand at bf16's full range, all
 // four partial products kept.  (kind::f16 does not take an fp16 operand next to a bf16 one -- tried, the launch faults --
-// so the lo planes cannot carry fp16's 11 bits.)
+// so the lo planes cannot carry fp16's 11 bits.)  ab_f16 runs one pass with BOTH operands fp16 instead: the first layer of an
+// fp16 feature map against fp16 weight planes.  Every other GEMM stays bf16 x bf16, so no launch can mix the two types.
 #pragma once
 #include <cuda.h>
 
@@ -15,7 +16,7 @@ namespace pasn {
 namespace tcg {
 
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_ABS = 2 };
-enum { OUT_NONE = 0, OUT_BF16 = 1, OUT_BF16_HILO = 2, OUT_F32 = 3 };   // HILO: bf16 hi plane | bf16 lo plane
+enum { OUT_NONE = 0, OUT_BF16 = 1, OUT_BF16_HILO = 2, OUT_F32 = 3, OUT_F16 = 4 };   // HILO: bf16 hi plane | bf16 lo plane
 
 struct Output {
   void* ptr;          // base of the [batch][M][ld] array (element (b, m, n) at ptr + (b*bs + m*ld + n) * elt)
@@ -55,7 +56,8 @@ struct Gemm {
   int act;
   Output out[2];
   float* psum;                   // optional [batch*M][2*tiles_n]: row sums of the outputs per column half-tile ...
-  int psum_rounded;              // ... of the bf16-rounded values (what a bf16 consumer of out[0] will read) or of the fp32 values
+  int psum_rounded;              // ... of the bf16-rounded values (what a bf16 consumer of the outputs will read) or of the fp32
+                                 // values (an OUT_F16 output feeds no GEMM: the fp16 chain pools its bf16 copy)
   int pair;                      // 1: CTA pairs (cta_group::2): 256 x bn tiles, each CTA of a 2-CTA cluster loads its 128 rows of A
                                  // and half of the B tile -- a third less L2 -> SM traffic per flop (bn >= 128 only; else ignored)
   // optional per-row statistics of the final fp32 values (the prototype stage's reductions folded into the GEMM that produces
@@ -70,6 +72,8 @@ struct Gemm {
   int group, group_rows, group_items;
   long long stat_rows;           // rows of rowstat that exist (0: batch * M): rows past it are not written
   int dot_early;                 // dotvec is not written by the kernel in front on the stream: it may be read before that one has completed
+  int ab_f16;                    // 1: A and B are fp16 (kind::f16 with F16 x F16; npass must be 1), 0: both bf16.  Placed in the tail
+                                 // padding of the struct: sizeof(Gemm) is unchanged (448)
 };
 
 void set_trace(void* dev_buf);   // debug: 64 rows of 64 int64 globaltimer stamps of CTA 0, one row per launch (null = off)

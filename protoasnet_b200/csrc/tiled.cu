@@ -16,6 +16,7 @@
 //   cosine / (.+1)/2 / logits / 1-s / push keys: proto_stage.cu (fp32)
 // Hidden activations are bf16 in HBM between the GEMMs (hi|lo planes in fp32 mode).
 #include <cstdlib>
+#include <type_traits>
 
 #include "tc_gemm.cuh"
 
@@ -27,6 +28,7 @@ struct Plan {
   int ex;        // bf16 planes per activation / weight: 1 (bf16 mode), 2 (fp32 mode: hi | lo)
   int C, D, D2, P, K, S, Sp;   // Sp: column pitch of one plane of the pooling A operand (occurrence values)
   bool occ_direct;             // bf16 mode and 16-byte aligned rows: the pooling reads the occurrence_map buffer itself
+                               // (fp16 mode: the map is fp16, the pooling reads a bf16 copy of it, see DESIGN.md 2.7)
   bool w2_first;               // F = W2 H1 + b2 before the pooling (cheaper when S is small against P)
   bool tok_c;                  // few prototypes: O over all tokens at once (token-major), the map leaves channel-major per clip
   int Pp;                      // column pitch of one plane of the token-major occurrence values
@@ -42,7 +44,7 @@ Plan make_plan(const pasn_dims& d) {
   Plan p{};
   p.ex = d.dtype == PASN_F32 ? 2 : 1;
   p.C = d.C; p.D = d.D; p.D2 = d.D / 2; p.P = d.P; p.K = d.K; p.S = d.S;
-  p.occ_direct = p.ex == 1 && (d.S * 2) % 16 == 0;
+  p.occ_direct = d.dtype == PASN_BF16 && (d.S * 2) % 16 == 0;
   // MACs of the W2 stage per clip: S*D*D*passes before the pooling, P*D*D*passes after it (bf16 mode: the pooled vectors
   // go in as hi + lo planes, two passes; fp32 mode: three passes either way)
   p.w2_first = p.ex == 1 ? (d.S < 2 * d.P) : (d.S < d.P);
@@ -108,17 +110,22 @@ __global__ void pack_planes_kernel(const float* __restrict__ w, int rows, int co
     if (ex == 2) *(out + (size_t)r * ex * cols + cols + c) = __float2bfloat16_rn(v - __bfloat162float(hi));
   }
 }
+// fp16 mode's first-layer weights: fp32 [n] -> fp16 (the operand type of the fp16 feature map)
+__global__ void pack_f16_kernel(const float* __restrict__ w, long long n, __half* __restrict__ out) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    out[i] = __float2half_rn(w[i]);
+}
 __global__ void pack_bias_kernel(const float* __restrict__ b, int n, int round, float* __restrict__ out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = round ? round_bf16(b[i]) : b[i];
 }
 
-// feature map -> token-major bf16 planes XT[(n*S + s)][ex*C]
+// feature map -> token-major bf16 planes XT[(n*S + s)][ex*C] (O = __half: one fp16 plane, the fp16 chain's first-layer operand)
 //   NCS ([n][C][S]): 64-channel x 32-voxel tiles through shared memory: loads run along s (one channel row segment per warp
 //   instruction), stores along c (one full 128-byte line of bf16 channel pairs per token and plane);
-//   NSC fp32 ([n][S][C]): plane split only
-template <typename T>
-__global__ void __launch_bounds__(256) to_tokens_ncs_kernel(const T* __restrict__ x, int C, int S, int ex, __nv_bfloat16* __restrict__ out) {
+//   NSC fp32 / fp16 ([n][S][C]): plane split only
+template <typename T, typename O = __nv_bfloat16>
+__global__ void __launch_bounds__(256) to_tokens_ncs_kernel(const T* __restrict__ x, int C, int S, int ex, O* __restrict__ out) {
   __shared__ float tile[64][33];
   const int n = blockIdx.z, c0 = blockIdx.y * 64, s0 = blockIdx.x * 32;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -133,7 +140,10 @@ __global__ void __launch_bounds__(256) to_tokens_ncs_kernel(const T* __restrict_
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const int sl = warp * 4 + j, s = s0 + sl;
-    if (s < S && c < C) {
+    if constexpr (std::is_same<O, __half>::value) {
+      if (s < S && c < C)
+        *reinterpret_cast<__half2*>(out + ((size_t)n * S + s) * C + c) = __floats2half2_rn(tile[2 * lane][sl], tile[2 * lane + 1][sl]);
+    } else if (s < S && c < C) {
       const float v0 = tile[2 * lane][sl], v1 = tile[2 * lane + 1][sl];
       const __nv_bfloat16 h0 = __float2bfloat16_rn(v0), h1 = __float2bfloat16_rn(v1);
       __nv_bfloat16* row = out + ((size_t)n * S + s) * ex * C;
@@ -144,7 +154,7 @@ __global__ void __launch_bounds__(256) to_tokens_ncs_kernel(const T* __restrict_
     }
   }
 }
-// small bf16 clips (C*S*2 bytes fit in shared memory, e.g. the 7 x 7 image head): a clip's [C][S] block is one contiguous
+// small bf16 (or fp16: the kernel only moves bytes) clips (C*S*2 bytes fit in shared memory, e.g. the 7 x 7 image head): a clip's [C][S] block is one contiguous
 // run in memory, so it is copied in with 16-byte vectors and transposed out of shared memory (rows of S bf16 are not
 // 4-byte aligned, which makes the tiled kernel above read half-empty sectors).  One block per clip.
 __global__ void __launch_bounds__(256) to_tokens_small_bf16_kernel(const __nv_bfloat16* __restrict__ x, int C, int S,
@@ -163,12 +173,13 @@ __global__ void __launch_bounds__(256) to_tokens_small_bf16_kernel(const __nv_bf
   }
 }
 
-__global__ void to_tokens_nsc_f32_kernel(const float* __restrict__ x, long long rows, int C, __nv_bfloat16* __restrict__ out) {
+template <typename T>
+__global__ void to_tokens_nsc_split_kernel(const T* __restrict__ x, long long rows, int C, __nv_bfloat16* __restrict__ out) {
   const long long n = rows * C;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const long long r = i / C;
     const int c = (int)(i - r * C);
-    const float v = x[i];
+    const float v = to_f32<T>(x[i]);
     const __nv_bfloat16 hi = __float2bfloat16_rn(v);
     out[r * 2 * C + c] = hi;
     *(out + r * 2 * C + C + c) = __float2bfloat16_rn(v - __bfloat162float(hi));
@@ -229,8 +240,14 @@ int tiled_pack_weights(const pasn_weights& w, const pasn_dims& d, void* packed, 
     pack_planes_kernel<<<148 * 2, 256, 0, st>>>(src, rows, cols, ex, reinterpret_cast<__nv_bfloat16*>(pk + off));
     count_launch();
   };
-  planes(w.addon_w1, d.D, d.C, L.off_w13);
-  planes(w.occ_w1, d.D, d.C, L.off_w13 + (size_t)d.D * ex * d.C * 2);
+  if (d.dtype == PASN_F16) {   // first layer fp16 x fp16 (one plane, same bytes as bf16 mode's)
+    pack_f16_kernel<<<148 * 2, 256, 0, st>>>(w.addon_w1, (long long)d.D * d.C, reinterpret_cast<__half*>(pk + L.off_w13));
+    pack_f16_kernel<<<148 * 2, 256, 0, st>>>(w.occ_w1, (long long)d.D * d.C, reinterpret_cast<__half*>(pk + L.off_w13) + (size_t)d.D * d.C);
+    count_launch(2);
+  } else {
+    planes(w.addon_w1, d.D, d.C, L.off_w13);
+    planes(w.occ_w1, d.D, d.C, L.off_w13 + (size_t)d.D * ex * d.C * 2);
+  }
   planes(w.occ_w2, D2, d.D, L.off_w4);
   planes(w.occ_w3, d.P, D2, L.off_w5);
   planes(w.addon_w2, d.D, d.D, L.off_w2);
@@ -255,24 +272,25 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   const char* pk = reinterpret_cast<const char*>(packed);
   const int ex = p.ex, C = p.C, D = p.D, D2 = p.D2, P = p.P, S = p.S;
   const long long T = (long long)nb * S;
-  const size_t elt = d.dtype == PASN_BF16 ? 2 : 4;
+  const size_t elt = dtype_bytes(d.dtype);
+  const bool f16 = d.dtype == PASN_F16;   // layer 1 fp16 x fp16, the map stored in fp16; everything else as bf16 mode
   int rc;
 
   // ---- tokens
   const __nv_bfloat16* xt;
   const char* x = reinterpret_cast<const char*>(feat) + (size_t)n0 * C * S * elt;
-  // bf16 NCDHW feature maps with 16-byte aligned channel rows need no transposition: [C][S] per clip IS the MN-major form
+  // bf16 / fp16 NCDHW feature maps with 16-byte aligned channel rows need no transposition: [C][S] per clip IS the MN-major form
   // of the A operand (voxels contiguous), which the TMA unit tiles straight out of the caller's buffer
   const bool x_direct = d.layout == PASN_LAYOUT_NCS && ex == 1 && (S * 2) % 16 == 0 && ((uintptr_t)x & 15) == 0;
   if (d.layout == PASN_LAYOUT_NSC && ex == 1) {
-    xt = reinterpret_cast<const __nv_bfloat16*>(x);   // channels_last bf16 feature map: already token-major
+    xt = reinterpret_cast<const __nv_bfloat16*>(x);   // channels_last bf16 / fp16 feature map: already token-major
     if (((uintptr_t)xt & 15) != 0) return PASN_ERR_ALIGN;
   } else if (x_direct) {
     xt = reinterpret_cast<const __nv_bfloat16*>(x);
   } else {
     __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(ws + p.off_xt);
     if (d.layout == PASN_LAYOUT_NSC) {
-      to_tokens_nsc_f32_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, dst);
+      to_tokens_nsc_split_kernel<float><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, dst);
     } else {
       dim3 grid(ceil_div(S, 32), ceil_div(C, 64), nb);
       const size_t clip_bytes = (size_t)C * S * 2;
@@ -284,6 +302,9 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
           attr_done = true;
         }
         to_tokens_small_bf16_kernel<<<nb, 256, clip_bytes, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, dst);
+      } else if (f16) {
+        to_tokens_ncs_kernel<__half, __half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 1,
+                                                                   reinterpret_cast<__half*>(dst));
       } else if (ex == 1) {
         to_tokens_ncs_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, ex, dst);
       } else {
@@ -329,6 +350,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.M = (int)T; g.N = nA; g.K = C; g.batch = 1; g.bn = 256;
     set_passes(g, ex, C, C);
     g.bias = occ_only ? b13 + D : b13; g.act = tcg::ACT_RELU;
+    g.ab_f16 = f16 ? 1 : 0;   // X and [W1; W3] both fp16 (pack: tiled_pack_weights)
     g.out[0] = {Y, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * nA, 0, nA};
     if (x_direct) {   // one GEMM per clip: rows = its S voxels, operand [C rows][S] as it lies in the feature map
       g.a_mn_major = 1; g.lda = S; g.a_bs = (long long)C * S; g.a_batched = 1; g.ka = S; g.a_rows = C;
@@ -351,6 +373,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   }
   // ---- (C) O[n] = |W5 G2[n]^T|  -> occurrence_map [n][P][S] (+ the pooling operand copy when the map cannot serve as one)
   void* occ_user = occ ? reinterpret_cast<char*>(occ) + (size_t)n0 * P * S * elt : nullptr;
+  const int occ_mode = ex == 2 ? tcg::OUT_F32 : (f16 ? tcg::OUT_F16 : tcg::OUT_BF16);   // the map in the feature map's type
   const __nv_bfloat16* pool_a = nullptr;     // pooling A operand
   long long pool_lda = 0;
   // W2-after-pooling order: the row sums over s then come from a small column-sum kernel below.  (fp32 maps keep the
@@ -369,7 +392,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.act = tcg::ACT_ABS;
     int no = 0;
     if (occ_user != nullptr) {
-      g.out[no] = {occ_user, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_F32, (long long)S, (long long)P * S, 0, P, 0, S};
+      g.out[no] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0, P, 0, S};
       ++no;
     }
     if (!occ_only) {
@@ -396,7 +419,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     int no = 0;
     const bool need_copy = !occ_only && !(p.occ_direct && occ_user != nullptr);
     if (occ_user != nullptr) {
-      g.out[no] = {occ_user, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_F32, (long long)S, (long long)P * S, 0};
+      g.out[no] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0};
       g.out[no].ncols = S;
       ++no;
     }
@@ -555,7 +578,8 @@ int tiled_occurrence_only(const void* feat, const pasn_weights& w, const void* p
 namespace {
 
 struct BPlan {
-  int C, D, D2, P, Pp, K, S, xe;   // xe: planes of the token-major feature copy (1: bf16 input is exact, 2: fp32 input)
+  int C, D, D2, P, Pp, K, S, xe;   // xe: planes of the token-major feature copy (1: bf16 input is exact, 2: fp32 input, or
+                                   // fp16 input: its 11 significant bits are exact in a bf16 hi | lo pair)
   int nb;
   size_t off_pk, off_xt, off_y, off_g2, off_os, off_oa, off_f, off_fe, off_gfe, off_rs, off_go, off_gf, off_gy, off_gg2,
       off_part, part_bytes, total;
@@ -574,7 +598,7 @@ inline int split_parts(long long T, int tiles, int* kper) {
 BPlan make_bplan(const pasn_dims& d) {
   BPlan b{};
   b.C = d.C; b.D = d.D; b.D2 = d.D / 2; b.P = d.P; b.Pp = (d.P + 7) / 8 * 8; b.K = d.K; b.S = d.S;
-  b.xe = d.dtype == PASN_F32 ? 2 : 1;
+  b.xe = d.dtype == PASN_BF16 ? 1 : 2;
   pasn_dims d2 = d;
   d2.dtype = PASN_F32;
   const size_t pk = align_up(pack_layout(d2).total, 1024);
@@ -796,7 +820,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
   float* FE = reinterpret_cast<float*>(ws + b.off_fe);
   float4* RS = reinterpret_cast<float4*>(ws + b.off_rs);
   float* PART = reinterpret_cast<float*>(ws + b.off_part);
-  const size_t elt = d.dtype == PASN_BF16 ? 2 : 4;
+  const size_t elt = dtype_bytes(d.dtype);
   const bool x_lo = xe == 2;
   // No gradient arrives through logits / similarity: backward of compute_occurence_map alone (TransformLoss re-entry,
   // src/loss/loss.py:302) -- only the occurrence branch is recomputed and differentiated.
@@ -846,11 +870,13 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       xt = reinterpret_cast<const __nv_bfloat16*>(x);
       if (((uintptr_t)xt & 15) != 0) return PASN_ERR_ALIGN;
     } else if (d.layout == PASN_LAYOUT_NSC) {
-      to_tokens_nsc_f32_kernel<<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, XT);
+      if (d.dtype == PASN_F16) to_tokens_nsc_split_kernel<__half><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const __half*>(x), T, C, XT);
+      else to_tokens_nsc_split_kernel<float><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, XT);
       count_launch();
     } else {
       dim3 grid(ceil_div(S, 32), ceil_div(C, 64), nb);
       if (xe == 1) to_tokens_ncs_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, 1, XT);
+      else if (d.dtype == PASN_F16) to_tokens_ncs_kernel<__half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 2, XT);
       else to_tokens_ncs_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(x), C, S, 2, XT);
       count_launch();
     }

@@ -82,8 +82,8 @@ class _HeadRuntime:
         m = self.owner
         if not x.is_cuda:
             raise _lib.PasnError("protoasnet_b200 head needs a CUDA tensor: there is no CPU implementation of this path")
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            raise _lib.PasnError(f"unsupported feature dtype {x.dtype} (fp32 or bf16)")
+        if x.dtype not in _lib.DTYPES:
+            raise _lib.PasnError(f"unsupported feature dtype {x.dtype} (fp32, bf16 or fp16)")
         nd = x.dim() - 2
         if nd not in (2, 3):
             raise _lib.PasnError("feature map must be [N,C,H,W] or [N,C,T,H,W]")
@@ -100,8 +100,14 @@ class _HeadRuntime:
         for v in spatial:
             S *= int(v)
         P, D = int(m.prototype_shape[0]), int(m.prototype_shape[1])
-        dims = PasnDims(int(x.shape[0]), int(x.shape[1]), D, P, int(m.num_classes), S,
-                        _lib.PASN_BF16 if x.dtype == torch.bfloat16 else _lib.PASN_F32, layout, _lib.PASN_OCC_ABS, path)
+        dims = PasnDims(int(x.shape[0]), int(x.shape[1]), D, P, int(m.num_classes), S, _lib.DTYPES[x.dtype], layout,
+                        _lib.PASN_OCC_ABS, path)
+        if dims.dtype == _lib.PASN_F16 and not _lib.load().pasn_tcgen05_supported(C.byref(dims)):
+            raise _lib.PasnError(
+                f"fp16 feature maps run on the tensor-core paths only (fused: D = 256, C % 64 == 0, C <= 1024, P <= 48, "
+                f"S % 4 == 0, S >= 128; tiled: C % 64 == 0, D % 128 == 0; kernel_path not GENERIC), and this head "
+                f"(C = {dims.C}, D = {D}, P = {P}, S = {S}, kernel_path = {path}) takes neither: pass x.float() or "
+                f"x.bfloat16()")
         return dims, x, spatial
 
     def run(self, x: torch.Tensor, want_occ=True, want_feats=False, want_dist=False, push: Optional[dict] = None):

@@ -123,7 +123,7 @@ class _OccNorm(torch.autograd.Function):
             raise _lib.PasnError("protoasnet_b200.metrics needs CUDA tensors: there is no CPU implementation of this path")
         lib = _lib.load()
         o = occ.detach()
-        if o.dtype not in (torch.float32, torch.bfloat16):
+        if o.dtype not in _lib.DTYPES:
             o = o.to(torch.float32)
         o = o.contiguous()
         rows = int(o.shape[0] * o.shape[1])
@@ -131,7 +131,7 @@ class _OccNorm(torch.autograd.Function):
         total = torch.zeros(1, dtype=torch.float64, device=o.device)
         norms = torch.empty(rows, dtype=torch.float32, device=o.device)
         with torch.cuda.device(o.device):
-            _lib.check(lib.pasn_occurrence_lnorm(o.data_ptr(), _lib.PASN_BF16 if o.dtype == torch.bfloat16 else _lib.PASN_F32,
+            _lib.check(lib.pasn_occurrence_lnorm(o.data_ptr(), _lib.DTYPES[o.dtype],
                                                  rows, s, int(p), total.data_ptr(), norms.data_ptr(), _stream(o.device)),
                        "pasn_occurrence_lnorm")
         ctx.save_for_backward(occ, norms)
