@@ -220,6 +220,24 @@ int pasn_push_merge_peers(const uint64_t* peer_records, const uint64_t* peer_fla
 /* prototype_vectors[p,:] = vec[p,:] where valid[p] != 0 (else unchanged) */
 int pasn_push_write_prototypes(float* prototypes, const float* vec, const int32_t* valid, int32_t P, int32_t D,
                                void* stream);
+/* Winner side data captured on the device, in the pass that produced the minimum (push_abs_revision.py:301-307): for every
+ * prototype p whose best_key[p] names a clip of this call (global index idx in [global_offset, global_offset + N)), copy
+ * row (idx - global_offset, p) of each slot's source into row p of its destination; every other row is left untouched.
+ *   src row address = src + (idx - global_offset) * clip_stride_bytes + p * proto_stride_bytes   (proto_stride 0: per-clip data)
+ *   dst row address = dst + p * row_bytes
+ * Called after the scan of a batch on the same stream: keys only decrease and ties go to the lowest global index, so
+ * best_key[p] names a clip of the batch exactly when that batch improved p, and the row that survives belongs to the final key.
+ * Rows are copied as bytes (16-byte vectors when src, dst and row_bytes are 16-byte aligned). */
+#define PASN_CAPTURE_MAX_SLOTS 8
+typedef struct {
+  const void* src;
+  void* dst;
+  int64_t row_bytes;
+  int64_t clip_stride_bytes;
+  int64_t proto_stride_bytes;
+} pasn_capture_slot;
+int pasn_push_capture(const uint64_t* best_key, int32_t P, int64_t global_offset, int32_t N,
+                      const pasn_capture_slot* slots_host, int32_t nslots, void* stream);
 
 /* measurement hooks used by bench.py (not part of the reference-facing contract):
  *   launch_count          number of kernels this library has launched in the process so far

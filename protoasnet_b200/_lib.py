@@ -24,7 +24,7 @@ SYMBOLS = [
     "pasn_abi_version", "pasn_strerror", "pasn_tcgen05_supported", "pasn_head_workspace_bytes",
     "pasn_packed_weights_bytes", "pasn_pack_weights", "pasn_head_forward", "pasn_occurrence_only",
     "pasn_push_record_bytes", "pasn_push_init", "pasn_push_decode", "pasn_push_reduce", "pasn_push_write_prototypes",
-    "pasn_push_merge_peers",
+    "pasn_push_merge_peers", "pasn_push_capture",
     "pasn_debug_launch_count", "pasn_debug_time_main_kernel", "pasn_debug_last_main_kernel_ms",
     "pasn_debug_sm100_error", "pasn_debug_set_trace", "pasn_debug_set_k1_variant", "pasn_debug_fault", "pasn_debug_set_fault",
     "pasn_head_backward_workspace_bytes", "pasn_head_backward", "pasn_similarity_stats", "pasn_occurrence_lnorm",
@@ -53,6 +53,14 @@ class PasnGrads(C.Structure):
 class PasnPushArgs(C.Structure):
     _fields_ = [("labels", C.c_void_p), ("proto_class", C.c_void_p), ("global_offset", C.c_int64),
                 ("best_key", C.c_void_p), ("best_vec", C.c_void_p)]
+
+
+PASN_CAPTURE_MAX_SLOTS = 8
+
+
+class PasnCaptureSlot(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("row_bytes", C.c_int64), ("clip_stride_bytes", C.c_int64),
+                ("proto_stride_bytes", C.c_int64)]
 
 
 class PasnError(RuntimeError):
@@ -99,6 +107,8 @@ def load() -> C.CDLL:
     lib.pasn_push_reduce.argtypes = [vp, i32, i32, i32, vp, vp, vp, vp, vp]
     lib.pasn_push_merge_peers.restype = C.c_int
     lib.pasn_push_merge_peers.argtypes = [vp, vp, i32, i32, C.c_uint32, i32, i32, vp, vp, vp, vp, vp]
+    lib.pasn_push_capture.restype = C.c_int
+    lib.pasn_push_capture.argtypes = [vp, i32, i64, i32, C.POINTER(PasnCaptureSlot), i32, vp]
     lib.pasn_push_write_prototypes.restype = C.c_int
     lib.pasn_push_write_prototypes.argtypes = [vp, vp, vp, i32, i32, vp]
     lib.pasn_debug_launch_count.restype = C.c_ulonglong

@@ -423,6 +423,32 @@ __global__ void push_write_kernel(float* protos, const float* vec, const int32_t
   if (valid[i / D]) protos[i] = vec[i];
 }
 
+// Winner side data (pasn_push_capture): block (p, slot, part) copies part of row p of one slot when best_key[p] names a
+// clip of this call.  The slots travel by value in the kernel parameters, so the call needs no host->device copy.
+struct CaptureSlots {
+  pasn_capture_slot s[PASN_CAPTURE_MAX_SLOTS];
+};
+__global__ void __launch_bounds__(256) push_capture_kernel(const unsigned long long* __restrict__ best_key, long long offset,
+                                                           int N, const CaptureSlots slots) {
+  const int p = blockIdx.x;
+  const unsigned long long key = best_key[p] ^ PASN_KEY_SIGN;
+  if (key == PASN_KEY_NONE) return;
+  const long long idx = (long long)(key & 0xFFFFFFFFull);
+  if (idx < offset || idx >= offset + N) return;
+  const pasn_capture_slot& sl = slots.s[blockIdx.y];
+  const char* src = reinterpret_cast<const char*>(sl.src) + (idx - offset) * sl.clip_stride_bytes + (long long)p * sl.proto_stride_bytes;
+  char* dst = reinterpret_cast<char*>(sl.dst) + (long long)p * sl.row_bytes;
+  const long long n = sl.row_bytes;
+  const long long t0 = (long long)blockIdx.z * blockDim.x + threadIdx.x, step = (long long)gridDim.z * blockDim.x;
+  if ((((uintptr_t)src | (uintptr_t)dst | (uintptr_t)n) & 15) == 0) {
+    const uint4* s4 = reinterpret_cast<const uint4*>(src);
+    uint4* d4 = reinterpret_cast<uint4*>(dst);
+    for (long long i = t0; i < n / 16; i += step) d4[i] = s4[i];
+  } else {
+    for (long long i = t0; i < n; i += step) dst[i] = src[i];
+  }
+}
+
 }  // namespace pasn
 
 using namespace pasn;
@@ -472,6 +498,30 @@ extern "C" int pasn_push_write_prototypes(float* prototypes, const float* vec, c
   if (!prototypes || !vec || !valid || P <= 0 || D <= 0) return PASN_ERR_INVALID;
   long long n = (long long)P * D;
   push_write_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(prototypes, vec, valid, P, D);
+  PASN_LAUNCH_CHECK();
+  count_launch();
+  return PASN_OK;
+}
+extern "C" int pasn_push_capture(const uint64_t* best_key, int32_t P, int64_t global_offset, int32_t N,
+                                 const pasn_capture_slot* slots_host, int32_t nslots, void* stream) {
+  if (!best_key || P <= 0 || N < 0 || global_offset < 0 || global_offset + N > 0xFFFFFFFFll || !slots_host || nslots <= 0 ||
+      nslots > PASN_CAPTURE_MAX_SLOTS)
+    return PASN_ERR_INVALID;
+  CaptureSlots cs{};
+  long long max_row = 0;
+  for (int i = 0; i < nslots; ++i) {
+    const pasn_capture_slot& s = slots_host[i];
+    if (s.row_bytes < 0 || s.clip_stride_bytes < 0 || s.proto_stride_bytes < 0) return PASN_ERR_INVALID;
+    if (s.row_bytes > 0 && (!s.src || !s.dst)) return PASN_ERR_INVALID;
+    cs.s[i] = s;
+    if (s.row_bytes > max_row) max_row = s.row_bytes;
+  }
+  if (N == 0 || max_row == 0) return PASN_OK;
+  // a whole input clip can be megabytes: split long rows over up to 32 blocks (16 KB each) so one SM does not copy it alone
+  long long parts = (max_row + 16383) / 16384;
+  if (parts > 32) parts = 32;
+  push_capture_kernel<<<dim3(P, nslots, (unsigned)parts), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const unsigned long long*>(best_key), (long long)global_offset, N, cs);
   PASN_LAUNCH_CHECK();
   count_launch();
   return PASN_OK;

@@ -481,22 +481,18 @@ class PrototypeHeadMixin:
         r = self._rt.run(x, want_occ=True, want_feats=True, want_dist=True)
         return r["features_extracted"], r["distance"], r["occurrence_map"], r["logits"]
 
-    # ---- B200 extension used by push (no per-batch D2H, no occurrence-map store) ----
-    def push_scan(self, x, labels, proto_class, global_offset, best_key, backbone=True, best_vec=None):
+    # ---- B200 extension used by push (no per-batch D2H; the occurrence map is stored only on request) ----
+    def push_scan(self, x, labels, proto_class, global_offset, best_key, backbone=True, best_vec=None, want_occ=False):
         """Fused similarity + class-restricted running argmin over one batch; updates ``best_key`` (and, when given,
-        the winners' ``features_extracted`` rows ``best_vec`` [P,D] fp32) in place."""
+        the winners' ``features_extracted`` rows ``best_vec`` [P,D] fp32) in place.  Returns the batch's ``logits``
+        (and ``occurrence_map`` with ``want_occ``) from the same pass, for the winners' side data."""
         if backbone:
             x = self.cnn_backbone(x)
         if best_vec is not None and (best_vec.dtype != torch.float32 or not best_vec.is_contiguous()):
             raise _lib.PasnError("best_vec must be a contiguous fp32 [P,D] tensor")
-        return self._rt.run(x, want_occ=False, push=dict(labels=labels, proto_class=proto_class,
-                                                           global_offset=global_offset, best_key=best_key,
-                                                           best_vec=best_vec))
-
-    def _rt_push_forward_features(self, feats_in):
-        """push_forward on an already-computed backbone feature map (winner re-fetch in push pass 2)."""
-        r = self._rt.run(feats_in, want_occ=True, want_feats=True, want_dist=True)
-        return r["features_extracted"], r["distance"], r["occurrence_map"], r["logits"]
+        return self._rt.run(x, want_occ=want_occ, push=dict(labels=labels, proto_class=proto_class,
+                                                              global_offset=global_offset, best_key=best_key,
+                                                              best_vec=best_vec))
 
     def __repr__(self):
         rep = ("PPNet(\n\tcnn_backbone: {},\n\timg_size: {},\n\tprototype_shape: {},\n\tproto_layer_rf_info: {},\n"

@@ -3,18 +3,26 @@
 Mirrors ``push_prototypes`` of the reference (src/utils/push_abs_revision.py:181-348) and the agent wrapper
 ``XProtoNet_Base.push`` (src/agents/XProtoNet_Base.py:149-167), re-designed for B200:
 
-  scan    every rank walks its contiguous shard of the unshuffled ``train_push`` set; per batch ONE fused launch pair
-          computes the head, folds the class-restricted running argmin into packed keys
+  load    a map-style DataLoader's batches are drawn once on rank 0 from its batch sampler and broadcast; rank r loads only
+          its contiguous slice of them (``shard_bounds``), through a DataLoader over the same dataset with the same
+          collation and workers.  Batches keep their single-process composition and global offsets.  A loader without a
+          batch sampler (IterableDataset) is walked whole by every rank, each computing on its own slice.
+  scan    per batch ONE fused launch pair computes the head, folds the class-restricted running argmin into packed keys
           ``orderable(fp32 dist) << 32 | global index`` AND keeps the winner's ``features_extracted`` row -- both in one
           device record ``[keys P x u64 | vectors P x D x f32]``.  The winner is captured in the pass that saw it, as the
           reference does (push_abs_revision.py:299-307): its push loader draws a random window per ``__getitem__``
           (src/data/as_dataloader.py:246-255), so a clip cannot be fetched a second time.  No per-batch D2H of features,
           distances, occurrence maps or input clips (push_abs_revision.py:278-285).
-  merge   ONE collective: all-gather of the records (41 KB per rank at P=40, D=256); every rank then picks, per
-          prototype, the record with the smallest key (lowest distance, ties -> lowest global index) and overwrites
-          ``prototype_vectors`` identically (push_abs_revision.py:342-346).
-  side    with a Dataset loader the data the reference pickles (occurrence map, logits, label, filename, input clip;
-          push_abs_revision.py:301-325) is taken from the batch that improved a prototype, while it is still in memory.
+  side    with a save directory, the data the reference pickles (occurrence map, logits, input clip;
+          push_abs_revision.py:301-325) is copied on the device by ``pasn_push_capture`` right after the scan of each
+          batch, into per-prototype stashes; labels and file names stay on the host.  No host synchronisation per batch.
+  merge   ONE collective: all-gather of the records (41 KB per rank at P=40, D=256), or one kernel over peer memory;
+          every rank then picks, per prototype, the record with the smallest key (lowest distance, ties -> lowest global
+          index) and overwrites ``prototype_vectors`` identically (push_abs_revision.py:342-346).  The loader path waits
+          at a barrier first, so loader skew between ranks is absorbed there.
+  pickle  the host reads the winners' indices once; the rank whose shard holds a winner copies its side rows to the host,
+          one gather_object brings them to rank 0 (copied, never summed: bit-identical), and rank 0 writes the one
+          ``prototypes_info.pickle``, identical to a single-process push over the same batches.
 
 Defined behaviour where the reference crashes: a class-specific prototype whose class never occurs keeps its old
 vector and reports index -1 (SURVEY.md section 7 'Empty class').  Rendering of prototype images / mp4s
@@ -268,6 +276,131 @@ def push_resident(model, features: torch.Tensor, labels: torch.Tensor, global_of
     return finish_push(model, rec, replace_prototypes, group)
 
 
+def shard_bounds(n_batches: int, rank: int, world: int) -> Tuple[int, int]:
+    """Batches [lo, hi) of rank ``rank``: contiguous slices of ceil(n_batches / world) batches, so every batch has the
+    composition it has in a single-process run (the trailing ranks get an empty slice when there are fewer batches)."""
+    per = -(-n_batches // world)
+    return min(rank * per, n_batches), min((rank + 1) * per, n_batches)
+
+
+class ShardPlan:
+    """Who pushes which clips: from the sizes of ALL batches in loader order, rank r takes the batches
+    ``bounds[r]`` (``shard_bounds``) and so the global clips [starts[r], starts[r] + counts[r])."""
+
+    def __init__(self, sizes: Sequence[int], world: int):
+        self.sizes = [int(b) for b in sizes]
+        self.world = int(world)
+        cum = [0]
+        for b in self.sizes:
+            cum.append(cum[-1] + b)
+        self.n_total = cum[-1]
+        self.bounds = [shard_bounds(len(self.sizes), r, self.world) for r in range(self.world)]
+        self.starts = [cum[lo] for lo, _ in self.bounds]
+        self.counts = [cum[hi] - cum[lo] for lo, hi in self.bounds]
+
+    def owner(self, index: int) -> int:
+        """Rank whose shard holds global clip ``index``."""
+        if not 0 <= index < self.n_total:
+            raise ValueError(f"clip index {index} outside the push set [0, {self.n_total})")
+        return next(r for r in range(self.world) if self.starts[r] <= index < self.starts[r] + self.counts[r])
+
+
+def loader_batches(dataloader, group=None) -> Optional[list]:
+    """The batches (lists of dataset indices) a map-style DataLoader yields, drawn once from its batch sampler on rank 0
+    and broadcast, so that every rank agrees on them whatever the sampler.  None for a loader that has no batch sampler
+    to draw from (an IterableDataset, ``batch_size=None``, or any other iterable)."""
+    import torch.distributed as dist
+
+    if not isinstance(dataloader, torch.utils.data.DataLoader) or dataloader.batch_sampler is None or \
+            isinstance(dataloader.dataset, torch.utils.data.IterableDataset):
+        return None
+    rank, world = _world(group)
+    obj = [[list(b) for b in dataloader.batch_sampler] if rank == 0 else None]
+    if world > 1:
+        src = 0 if group is None else dist.get_global_rank(group, 0)
+        dist.broadcast_object_list(obj, src=src, group=group)
+    return obj[0]
+
+
+def shard_loader(dataloader, batches):
+    """A DataLoader over ``dataloader.dataset`` that yields exactly ``batches``, with the original's collation, workers
+    and memory pinning."""
+    kw = dict(collate_fn=dataloader.collate_fn, num_workers=dataloader.num_workers, pin_memory=dataloader.pin_memory,
+              worker_init_fn=dataloader.worker_init_fn, timeout=dataloader.timeout,
+              multiprocessing_context=dataloader.multiprocessing_context, persistent_workers=dataloader.persistent_workers)
+    if dataloader.num_workers > 0:
+        kw["prefetch_factor"] = dataloader.prefetch_factor
+    return torch.utils.data.DataLoader(dataloader.dataset, batch_sampler=batches, **kw)
+
+
+class _SideCapture:
+    """The side data the reference pickles for each prototype's winner (push_abs_revision.py:301-325), captured on the
+    device in the pass that produced the minimum: after each batch's scan, ``pasn_push_capture`` copies the rows of the
+    clips that improved a prototype into per-prototype stashes -- occurrence-map row [1,*spatial] (map dtype), logits [K]
+    (fp32), input clip (loader dtype).  Labels and file names are host data the loader hands over anyway; they are kept
+    per shard, by global position.  Nothing here waits for the device."""
+
+    def __init__(self, P: int, dev):
+        self.P, self.dev = P, dev
+        self.stash = None           # [occurrence rows, logits, clips], allocated at the first batch
+        self.start = None           # global index of this rank's first clip
+        self.targets, self.names = [], []
+
+    def batch(self, best_key, offset: int, x: torch.Tensor, out: dict, data_sample) -> None:
+        occ, logits = out["occurrence_map"], out["logits"]
+        x = x.contiguous()
+        N = int(x.shape[0])
+        if self.stash is None:
+            self.start = offset
+            self.stash = [torch.empty((self.P,) + tuple(t.shape[k:]), dtype=t.dtype, device=self.dev)
+                          for t, k in ((occ, 2), (logits, 1), (x, 1))]
+        elif tuple(x.shape[1:]) != tuple(self.stash[2].shape[1:]) or x.dtype != self.stash[2].dtype:
+            raise _lib.PasnError(f"push with a save directory needs clips of one shape and dtype: got {tuple(x.shape[1:])} "
+                                 f"{x.dtype} after {tuple(self.stash[2].shape[1:])} {self.stash[2].dtype}")
+        slots = (_lib.PasnCaptureSlot * 3)()
+        for s, src, dst, per_proto in zip(slots, (occ, logits, x), self.stash, (True, False, False)):
+            row = dst[0].numel() * dst.element_size()
+            s.src, s.dst, s.row_bytes = src.data_ptr(), dst.data_ptr(), row
+            s.clip_stride_bytes, s.proto_stride_bytes = (row * self.P, row) if per_proto else (row, 0)
+        lib = _lib.load()
+        with torch.cuda.device(self.dev):
+            _lib.check(lib.pasn_push_capture(best_key.data_ptr(), self.P, offset, N, slots, 3,
+                                             torch.cuda.current_stream(self.dev).cuda_stream), "pasn_push_capture")
+        self.targets.append(data_sample["target_AS"])
+        names = data_sample.get("filename", None)
+        self.names.extend(names[a] if names is not None else str(offset + a) for a in range(N))
+
+    def rows(self, index, protos) -> Dict[int, tuple]:
+        """Host copies of the side data of ``protos`` (winners in this rank's shard): p -> (occurrence-map row, logits,
+        clip, gt, file name).  Copied, never computed on, so they carry the captured bits (-0.0 included)."""
+        if not protos:
+            return {}
+        sel = torch.tensor(protos, dtype=torch.int64, device=self.dev)
+        occ, logits, clips = (t.index_select(0, sel) for t in self.stash)
+        occ, logits, clips = occ.float().cpu().numpy(), logits.cpu().numpy(), clips.cpu().numpy()
+        gts = torch.cat(self.targets).tolist()
+        return {p: (occ[t], logits[t], clips[t], int(gts[index[p] - self.start]), self.names[index[p] - self.start])
+                for t, p in enumerate(protos)}
+
+
+def _collect_side(cap: _SideCapture, res, plan: ShardPlan, group=None) -> Optional[Dict[int, tuple]]:
+    """Side data of every winner, on rank 0 (None on the other ranks): each rank takes the rows of the winners in its
+    shard off the device, and one gather_object brings them to rank 0, so the result is bit-identical to what a single
+    process captures."""
+    import torch.distributed as dist
+
+    rank, world = _world(group)
+    index = res["index"].cpu().tolist()                       # the one host read of the push
+    protos = [p for p in range(cap.P) if index[p] >= 0]
+    part = cap.rows(index, [p for p in protos if plan.owner(index[p]) == rank])
+    if world == 1:
+        return part
+    gathered = [None] * world if rank == 0 else None
+    with torch.cuda.device(cap.dev):
+        dist.gather_object(part, gathered, dst=0 if group is None else dist.get_global_rank(group, 0), group=group)
+    return {p: v for g in gathered for p, v in g.items()} if rank == 0 else None
+
+
 def push_prototypes(
     dataloader,
     model,
@@ -287,9 +420,12 @@ def push_prototypes(
 
     ``dataloader`` yields dicts with ``"cine"`` [B,3,(T),H,W], ``"target_AS"`` [B] and ``"filename"``, unshuffled
     (src/data/as_dataloader.py:65).  Every clip is seen exactly once: the winners' vectors and side data are captured
-    from the batch that produced them, so a loader whose ``__getitem__`` is random (as the reference's is) is fine.
-    Under torch.distributed every rank calls this with the SAME loader; rank r processes the batches whose global
-    clip range falls in its shard.
+    on the device from the batch that produced them, so a loader whose ``__getitem__`` is random (as the reference's
+    is) is fine, and no batch waits for the host.
+    Under torch.distributed every rank calls this with the SAME loader.  A map-style DataLoader's batches are drawn on
+    rank 0 and broadcast; rank r then loads only its contiguous slice of them (``shard_bounds``).  A loader without a
+    batch sampler is iterated whole by every rank, each computing its slice.  Rank 0 writes the one
+    ``prototypes_info.pickle`` and holds ``res["side"]``; it is ``{}`` on the other ranks.
     """
     model.eval()
     log(f"############## push at epoch {epoch_number} #################")
@@ -306,67 +442,69 @@ def push_prototypes(
     peers = _peer_records(model, P, D, dev, group)
     rec = peers.next_record() if peers is not None else PushRecord(P, D, dev)
     rank, world = _world(group)
-    n_batches = len(dataloader)
-    per = -(-n_batches // world)
-    b_lo, b_hi = min(rank * per, n_batches), min((rank + 1) * per, n_batches)
+    batches = None
+    if world > 1:
+        with torch.cuda.device(dev):
+            batches = loader_batches(dataloader, group)
+    if batches is not None:            # sharded loading: this rank fetches its own batches only
+        sizes = [len(b) for b in batches]
+        b_lo, b_hi = shard_bounds(len(sizes), rank, world)
+        source = enumerate(shard_loader(dataloader, batches[b_lo:b_hi]), start=b_lo)
+        offset = sum(sizes[:b_lo])
+    else:                              # every rank walks the whole loader and computes on its slice
+        sizes = []
+        b_lo, b_hi = shard_bounds(len(dataloader), rank, world)
+        source = enumerate(dataloader)
+        offset = 0
 
-    # side data of the current winner of each prototype (push_abs_revision.py:301-307), taken from the batch that
-    # improved it while that batch is still in memory
-    side = {j: None for j in range(P)}
-    want_side = proto_epoch_dir is not None
-    protos = []
-    offset = 0
+    cap = _SideCapture(P, dev) if proto_epoch_dir is not None else None
     with torch.no_grad():
-        for bi, data_sample in enumerate(dataloader):
+        for bi, data_sample in source:
             x = data_sample["cine"]
             B = x.shape[0]
+            if batches is None:
+                sizes.append(B)
+            elif B != sizes[bi]:
+                raise _lib.PasnError(f"batch {bi} holds {B} clips but its batch sampler listed {sizes[bi]} indices: "
+                                     f"the collate_fn must keep one clip per index")
             if b_lo <= bi < b_hi:
                 if preprocess_input_function is not None:
                     x = preprocess_input_function(x)
                 xd = x.to(dev, non_blocking=True)
                 y = data_sample["target_AS"].to(dev, non_blocking=True).to(torch.int64)
                 fmap = model.cnn_backbone(xd)
-                prev = rec.key.clone() if want_side else None
-                model.push_scan(fmap, y, pc, offset, rec.key, backbone=False, best_vec=rec.vec)
-                if want_side:
-                    changed = torch.nonzero(rec.key != prev).flatten()
-                    if changed.numel():                       # O(P log N) batches in total
-                        idx_now, _ = decode_keys(rec.key)
-                        local = (idx_now[changed] - offset)
-                        uniq, inv = torch.unique(local, return_inverse=True)
-                        _f, _d, occ, logits = model._rt_push_forward_features(fmap.index_select(0, uniq))
-                        occ_rows = occ[inv, changed].float().cpu().numpy()
-                        lg = logits[inv].float().cpu().numpy()
-                        names = data_sample.get("filename", None)
-                        for t, (j, a) in enumerate(zip(changed.tolist(), local.tolist())):
-                            side[j] = {"occurrence_map": occ_rows[t], "logits": lg[t], "image": np.asarray(x[a]),
-                                       "gt": int(data_sample["target_AS"][a]),
-                                       "filename": names[a] if names is not None else str(offset + a)}
+                out = model.push_scan(fmap, y, pc, offset, rec.key, backbone=False, best_vec=rec.vec,
+                                      want_occ=cap is not None)
+                if cap is not None:
+                    cap.batch(rec.key, offset, xd, out, data_sample)
             offset += B
 
+    if world > 1:
+        # ranks finish their shards at different times: wait here rather than in the merge, whose peer-memory wait is short
+        import torch.distributed as dist
+        with torch.cuda.device(dev):
+            dist.barrier(group=group)
     with torch.no_grad():
         res = finish_push(model, rec, replace_prototypes, group)
 
-    # side data in the reference's pickle schema (push_abs_revision.py:309-325); under DDP each rank writes the winners
-    # that its own shard produced
-    if want_side:
-        idx_local, _ = decode_keys(rec.key)
-        mine = (idx_local == res["index"]) & (res["index"] >= 0)
-        protos = [j for j in torch.nonzero(mine).flatten().tolist() if side[j] is not None]
-        if protos:
+    if cap is not None:
+        side = _collect_side(cap, res, ShardPlan(sizes, world), group)
+        if side:
+            protos = sorted(side)
+            occ, logits, clips, gts, names = (np.array([side[j][k] for j in protos]) for k in range(5))
+            # the reference's pickle schema (push_abs_revision.py:309-325)
             info = {
                 "prototype_ids": np.asarray(protos),
-                "prototypes_filenames": np.array([side[j]["filename"] for j in protos]),
-                "prototypes_src_imgs": np.array([side[j]["image"] for j in protos]),
-                "prototypes_gts": np.array([side[j]["gt"] for j in protos]),
-                "prototypes_preds": np.array([side[j]["logits"] for j in protos]),
-                "prototypes_occurrence_maps": np.array([side[j]["occurrence_map"] for j in protos]),
+                "prototypes_filenames": names,
+                "prototypes_src_imgs": clips,
+                "prototypes_gts": gts,
+                "prototypes_preds": logits,
+                "prototypes_occurrence_maps": occ,
                 "prototypes_similarity_to_src_ROIs": 1 - res["distance"][protos].double().cpu().numpy(),
             }
-            suffix = "" if world == 1 else f".rank{rank}"
-            with open(os.path.join(proto_epoch_dir, f"prototypes_info{suffix}.pickle"), "wb") as f:
+            with open(os.path.join(proto_epoch_dir, "prototypes_info.pickle"), "wb") as f:
                 pickle.dump(info, f)
-        res["side"] = {j: side[j] for j in protos}
+            res["side"] = {j: dict(zip(("occurrence_map", "logits", "image", "gt", "filename"), side[j])) for j in protos}
     log("\tpush time: \t{0}".format(time.time() - start))
     return res
 
