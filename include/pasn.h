@@ -257,10 +257,6 @@ int pasn_debug_sm100_error(const void* workspace, const pasn_dims* dims, void* s
 /* device buffer of 1024 int64: [0,768) clock64() stamps of CTA 0 of the token kernel per tile phase, [768,1024) globaltimer
  * stamps of the token kernel start/end and of CTA 0 of the prototype kernel (tools/trace_k1.py, trace_k2.py; NULL = off) */
 int pasn_debug_set_trace(void* device_buffer);
-/* tile order of the fused token kernel for the next calls (same results; kept for A/B timing and regression tests):
- * 1 = serial (default), 2 = two-phase (layer-1 phases overlapped with the previous tile's chain);
- * anything else = back to the default / PASN_K1_PHASES */
-int pasn_debug_set_k1_variant(int variant);
 /* Test hook for the building block of the tiled tensor-core path: one launch of the library's internal tcgen05 GEMM.
  * `desc_host` points at a pasn::tcg::Gemm (protoasnet_b200/csrc/tc_gemm.cuh; tests/test_tc_gemm_gpu.py mirrors it field
  * by field), `desc_bytes` must equal pasn_debug_tc_gemm_desc_bytes(). */

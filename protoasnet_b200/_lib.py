@@ -26,7 +26,7 @@ SYMBOLS = [
     "pasn_push_record_bytes", "pasn_push_init", "pasn_push_decode", "pasn_push_reduce", "pasn_push_write_prototypes",
     "pasn_push_merge_peers", "pasn_push_capture",
     "pasn_debug_launch_count", "pasn_debug_time_main_kernel", "pasn_debug_last_main_kernel_ms",
-    "pasn_debug_sm100_error", "pasn_debug_set_trace", "pasn_debug_set_k1_variant", "pasn_debug_fault", "pasn_debug_set_fault",
+    "pasn_debug_sm100_error", "pasn_debug_set_trace", "pasn_debug_fault", "pasn_debug_set_fault",
     "pasn_head_backward_workspace_bytes", "pasn_head_backward", "pasn_similarity_stats", "pasn_occurrence_lnorm",
     "pasn_debug_tc_gemm_desc_bytes", "pasn_debug_tc_gemm", "pasn_debug_set_gemm_trace",
 ]
@@ -127,8 +127,6 @@ def load() -> C.CDLL:
                                           vp, vp, vp, vp, vp, vp]
     lib.pasn_occurrence_lnorm.restype = C.c_int
     lib.pasn_occurrence_lnorm.argtypes = [vp, C.c_int32, C.c_int64, C.c_int32, C.c_int32, vp, vp, vp]
-    lib.pasn_debug_set_k1_variant.restype = C.c_int
-    lib.pasn_debug_set_k1_variant.argtypes = [C.c_int]
     lib.pasn_debug_fault.restype = C.c_int
     lib.pasn_debug_set_fault.restype = C.c_int
     lib.pasn_debug_set_fault.argtypes = [C.c_int]

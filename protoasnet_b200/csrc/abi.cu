@@ -139,7 +139,6 @@ extern "C" int pasn_debug_sm100_error(const void* workspace, const pasn_dims* di
 }
 
 extern "C" int pasn_debug_set_trace(void* device_buffer) { sm100_set_trace(device_buffer); return PASN_OK; }
-extern "C" int pasn_debug_set_k1_variant(int variant) { sm100_set_k1_variant(variant); return PASN_OK; }
 
 // test hook: one launch of the internal tiled tcgen05 GEMM (descriptor = pasn::tcg::Gemm, see csrc/tc_gemm.cuh)
 extern "C" size_t pasn_debug_tc_gemm_desc_bytes(void) { return sizeof(tcg::Gemm); }

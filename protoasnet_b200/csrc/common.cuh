@@ -144,7 +144,6 @@ int sm100_occurrence_only(const void* feat, const pasn_weights& w, const void* p
                           size_t ws_bytes, cudaStream_t st);
 int sm100_last_error(const void* ws, const pasn_dims& d, cudaStream_t st);
 void sm100_set_trace(void* dev_buf);
-void sm100_set_k1_variant(int variant);
 
 }  // namespace pasn
 

@@ -40,20 +40,13 @@ constexpr uint32_t K2_STAGE = 65536;                 // A_hi chunk 16 KB | A_lo 
 constexpr uint32_t K2_SM_V = 2 * K2_STAGE;           // prototypes fp32 [P][257]
 constexpr uint32_t K2_V_BYTES = PP_MAX * 257 * 4;    // 49344
 constexpr uint32_t K2_SM_MISC = K2_SM_V + 49408;     // 180480
-constexpr uint32_t K2_SM_ORD = K2_SM_MISC + 8192;     // uint16 tile order table (dynamic hand-out), K2_MAX_ORD entries
-constexpr int K2_MAX_ORD = 4096;
-constexpr uint32_t K2_SMEM = K2_SM_ORD + 2 * K2_MAX_ORD;
+constexpr uint32_t K2_SMEM = K2_SM_MISC + 8192;
 
 struct K2Params {
   const uint8_t* feimg; const float* osum; const uint8_t* packed; size_t off_w2, off_b2;
   const float* protos; const float* last_layer;
   float* logits; float* sim; float* dist; float* feats;
   const int64_t* labels; const int32_t* proto_class; long long global_offset; unsigned long long* best_key;
-  const int* ready;   // per-clip hand-off counters of the token kernel (null: wait for the whole grid instead)
-  int cpc, grid1;     // clips per token-kernel CTA and its grid (readiness order of the tiles)
-  int* queue;         // dynamic tile queue counter (zeroed per call)
-  int* tile_owner;    // [ntiles] CTA that processed a tile (push capture)
-  int a_kmajor, l2_hints;   // layout of the pooled-vector images (see K1Params::flush_kmajor); L2 eviction hints
   float* stash;   // push capture: [gridDim][P][256] fp32, FE row of this CTA's best clip per prototype (or null)
   int N, P, PP, K, cpt, ntiles;   // PP = padded P (row stride inside a tile), cpt = clips per tile = 128 / PP
   int* err;
@@ -84,7 +77,7 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
   float* s_v = reinterpret_cast<float*>(smem + K2_SM_V);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  Ctx ctx{p.err, abort_s, p.fault, 0};
+  Ctx ctx{p.err, abort_s, p.fault};
   if ((smem_u32(smem) & 1023u) != 0) {
     if (tid == 0) atomicCAS(p.err, 0, 901);
     return;
@@ -124,94 +117,25 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
   tc_fence_after();
   const uint32_t tbase = *tmem_ptr_s;
   const uint32_t st_base = smem_u32(smem);
-  // Tile hand-out.  With the clip-level hand-off (p.ready) tiles come from a global queue in the order in which the token
-  // kernel finishes their clips: every token-kernel CTA walks its `cpc` clips in order, so queue slot i stands for clip
-  // (i % grid1) * cpc + i / grid1, and a tile is handed out at the slot of its latest clip.  A CTA that becomes resident
-  // while stragglers of the token kernel are still running thus works on finished tiles, and late CTAs take fewer.
-  // Without it (PASN_K2_EARLY=0) the tiles are dealt round-robin after the whole token kernel has completed.
-  // The loader publishes each tile index (or -1) in a 4-slot ring guarded by mbarriers; MMA issuer and epilogue follow.
-  const bool dynamic = p.ready != nullptr && p.ntiles <= K2_MAX_ORD;
-  uint16_t* s_ord = reinterpret_cast<uint16_t*>(smem + K2_SM_ORD);
-  if (dynamic) {
-    // order table: walk the slots (round-major), keep the slot of each tile's latest clip.  Every CTA builds the same
-    // table: contiguous slot range per thread, count, block-wide exclusive scan, fill.
-    int* s_cnt = reinterpret_cast<int*>(smem);   // the stage ring is not in use yet
-    const int nslots = p.grid1 * p.cpc;
-    const int per = (nslots + K2_THREADS - 1) / K2_THREADS;
-    auto emit_tile = [&](int i) -> int {   // tile handed out at slot i, or -1
-      const int rnd = i / p.grid1, clip = (i - rnd * p.grid1) * p.cpc + rnd;
-      if (clip >= p.N) return -1;
-      const int t = clip / p.cpt, c0 = t * p.cpt;
-      int c1 = c0 + p.cpt;
-      if (c1 > p.N) c1 = p.N;
-      int key = 0;
-      for (int c = c0; c < c1; ++c) key = max(key, c % p.cpc);
-      int first = c0;
-      while (first % p.cpc != key) ++first;
-      return clip == first ? t : -1;
-    };
-    const int i0 = tid * per, i1 = min(nslots, i0 + per);
-    int cnt = 0;
-    for (int i = i0; i < i1; ++i) cnt += emit_tile(i) >= 0 ? 1 : 0;
-    s_cnt[tid] = cnt;
-    __syncthreads();
-    if (tid == 0) {
-      int run = 0;
-      for (int j = 0; j < K2_THREADS; ++j) { const int c = s_cnt[j]; s_cnt[j] = run; run += c; }
-    }
-    __syncthreads();
-    int pos = s_cnt[tid];
-    for (int i = i0; i < i1; ++i) {
-      const int t = emit_tile(i);
-      if (t >= 0) s_ord[pos++] = (uint16_t)t;
-    }
-    __syncthreads();
-  }
+  // Tiles are dealt round-robin once the whole token kernel has completed.  The loader publishes each tile index (or -1)
+  // in a 4-slot ring guarded by mbarriers; MMA issuer and epilogue follow.
   if (tid == 0) K2_TRACE(1);   // prologue done
 
   if (warp == 9) {
     // ---------------------------------------------------------------- loader
     if (lane == 0) {
-      if (p.ready == nullptr) griddep_wait();   // the pooled-vector images are written by the token kernel
+      griddep_wait();   // the pooled-vector images are written by the token kernel
       K2_TRACE(2);
       const uint64_t pol_first = l2_policy_evict_first();
       uint32_t u = 0;
       bool ok = true;
-      int dbg_grabs = 0;
       for (int it = 0; ok; ++it) {
-        int tile = -1;
-        if (dynamic) {
-          const int e = atomicAdd(p.queue, 1);
-          if (p.trace != nullptr && blockIdx.x == 0 && dbg_grabs < 4) {   // first grabs: (time, queue position)
-            p.trace[768 + 240 + 2 * dbg_grabs] = gtimer_ns();
-            p.trace[768 + 240 + 2 * dbg_grabs + 1] = e;
-            ++dbg_grabs;
-          }
-          tile = e < p.ntiles ? (int)s_ord[e] : -1;
-        } else {
-          tile = (int)blockIdx.x + it * (int)gridDim.x;
-          if (tile >= p.ntiles) tile = -1;
-        }
+        int tile = (int)blockIdx.x + it * (int)gridDim.x;
+        if (tile >= p.ntiles) tile = -1;
         s_tile[it & 3] = tile;
         mbar_arrive(&tbars[it & 3]);
         if (tile < 0) break;
-        if (p.tile_owner != nullptr) p.tile_owner[tile] = (int)blockIdx.x;
         const uint8_t* a_src = p.feimg + (size_t)tile * FE_TILE_BYTES;
-        if (p.ready != nullptr) {
-          // clip-level hand-off: the token kernel bumps ready[clip] (release) once per epilogue warp and once for the
-          // Osum row; acquire here, then order the bulk (async-proxy) reads after it
-          int c1 = tile * p.cpt + p.cpt;
-          if (c1 > p.N) c1 = p.N;
-          const long long t0 = clock64();
-          for (int c = tile * p.cpt; c < c1 && ok; ++c) {
-            while (ld_acquire_gpu(p.ready + c) < K1_READY_TARGET) {
-              __nanosleep(100);
-              if (*abort_s || clock64() - t0 > 8000000000ll) { *abort_s = 1; atomicCAS(p.err, 0, 612); if (p.fault) *reinterpret_cast<volatile int*>(p.fault) = 612; ok = false; break; }
-            }
-          }
-          if (!ok) break;
-          fence_proxy_async_all();
-        }
         K2_TRACE(16 + it * 8 + 7);
         if (p.trace != nullptr && blockIdx.x == 0 && it < 32) p.trace[768 + 200 + it] = tile;
         for (int kc = 0; kc < 4; ++kc, ++u) {
@@ -219,13 +143,9 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
           if (!(ok = bwait(&bars[2 + s], ph ^ 1, ctx, 611))) break;
           const uint32_t dst = st_base + s * K2_STAGE;
           mbar_arrive_expect_tx(&bars[s], K2_STAGE);
-          if (p.l2_hints) {   // the images were stored evict_last by the token kernel; read them once, then let them go
-            bulk_g2s_hint(dst, a_src + (size_t)kc * 16384, 16384, &bars[s], pol_first);
-            bulk_g2s_hint(dst + 16384, a_src + 65536 + (size_t)kc * 16384, 16384, &bars[s], pol_first);
-          } else {
-            bulk_g2s(dst, a_src + (size_t)kc * 16384, 16384, &bars[s]);
-            bulk_g2s(dst + 16384, a_src + 65536 + (size_t)kc * 16384, 16384, &bars[s]);
-          }
+          // the images were stored evict_last by the token kernel; read them once, then let them go
+          bulk_g2s_hint(dst, a_src + (size_t)kc * 16384, 16384, &bars[s], pol_first);
+          bulk_g2s_hint(dst + 16384, a_src + 65536 + (size_t)kc * 16384, 16384, &bars[s], pol_first);
           bulk_g2s(dst + 32768, p.packed + p.off_w2 + (size_t)kc * 32768, 16384, &bars[s]);
           bulk_g2s(dst + 49152, p.packed + p.off_w2 + (size_t)kc * 32768 + 16384, 16384, &bars[s]);
         }
@@ -235,9 +155,9 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
     // ---------------------------------------------------------------- MMA issuer (one elected thread, lean issue path:
     // see head_sm100_k1.cu -- descriptors as 32-bit halves in a single-thread region keep the UTCHMMAs back to back)
     if (elect_one()) {
-      // A (pooled vectors): K-major rows (k = d contiguous) or MN-major images, B (W2) K-major
-      const uint32_t idesc = make_idesc_bf16(128, 256, p.a_kmajor ? 0 : 1, 0);
-      const uint32_t a_lbo = p.a_kmajor ? 16u : 8192u, a_kstep = p.a_kmajor ? 2u : 128u;
+      // A (pooled vectors): K-major rows (k = d contiguous), B (W2) K-major
+      const uint32_t idesc = make_idesc_bf16(128, 256, 0, 0);
+      constexpr uint32_t a_lbo = 16u, a_kstep = 2u;
       constexpr uint32_t HI = desc_hi(1024, SWZ_128B);
       const uint32_t bar0 = smem_u32(bars);
       uint32_t u = 0;
@@ -273,7 +193,7 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
     const int q = warp & 3, ch = warp >> 2;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     const int r = q * 32 + lane;
-    if (p.ready == nullptr) griddep_wait();   // Osum is written by the token kernel
+    griddep_wait();   // Osum is written by the token kernel
     bool ok = true;
     for (int it = 0; ok; ++it) {
       if (!(ok = bwait(&tbars[it & 3], (it >> 2) & 1, ctx, 632))) break;
@@ -293,9 +213,6 @@ __global__ void __launch_bounds__(K2_THREADS, 1) proto_w2_kernel(const K2Params 
       if (!(ok = bwait(&bars[4 + buf], (it >> 1) & 1, ctx, 631))) break;
       tc_fence_after();
       if (tid == 0) K2_TRACE(16 + it * 8 + 5);
-      // the loader has seen this tile's clips handed over (the accumulator could not be full otherwise); acquire again
-      // in this thread before touching the Osum row the token kernel wrote
-      if (p.ready != nullptr && rvalid) (void)ld_acquire_gpu(p.ready + n);
       const float os = rvalid ? p.osum[(size_t)n * p.P + pp] : 0.f;
       const uint32_t ta = tbase + lane_base + 256u * buf + 128u * ch;
       float ff = 0.f, dot = 0.f;
@@ -456,18 +373,17 @@ __global__ void pack_weights_kernel(pasn_weights w, int C, int P, int f16, uint8
 
 // =================================================================================================
 // push capture: best_vec[p,:] = stash slot of the K2 CTA that processed the clip holding best_key[p], if that clip belongs
-// to this call (keys carry the global clip index).  One block per prototype.
+// to this call (keys carry the global clip index; K2 deals its tiles round-robin).  One block per prototype.
 // =================================================================================================
 __global__ void push_capture_stash_kernel(const unsigned long long* __restrict__ best_key, int P, long long offset, int N,
-                                          int cpt, int grid2, const int* __restrict__ tile_owner, const float* __restrict__ stash,
-                                          float* __restrict__ best_vec) {
+                                          int cpt, int grid2, const float* __restrict__ stash, float* __restrict__ best_vec) {
   const int pp = blockIdx.x;
   const unsigned long long key = best_key[pp] ^ PASN_KEY_SIGN;
   if (key == PASN_KEY_NONE) return;
   const long long idx = (long long)(key & 0xFFFFFFFFull);
   if (idx < offset || idx >= offset + N) return;
   const int tile = (int)((idx - offset) / cpt);
-  const int cta = tile_owner != nullptr ? tile_owner[tile] : tile % grid2;
+  const int cta = tile % grid2;
   const float* src = stash + ((size_t)cta * P + pp) * DD;
   for (int d = threadIdx.x; d < DD; d += blockDim.x) best_vec[(size_t)pp * DD + d] = src[d];
 }
@@ -477,8 +393,6 @@ __global__ void push_capture_stash_kernel(const unsigned long long* __restrict__
 // =================================================================================================
 static long long* g_trace = nullptr;
 void sm100_set_trace(void* dev_buf) { g_trace = reinterpret_cast<long long*>(dev_buf); }
-static int g_k1_variant = -1;   // -1: PASN_K1_PHASES / PASN_K1_PAIR from the environment, else the default
-void sm100_set_k1_variant(int variant) { g_k1_variant = variant; }
 
 bool sm100_supported(const pasn_dims& d) {
   // fp32 feature maps take the fused path only on explicit request (bf16 compute: inputs are rounded on the fly)
@@ -504,8 +418,6 @@ static inline int k2_ppad(const pasn_dims& d) {
 // tile, multiple of 4) whose pooled features are summed after K2.  G = 1 means no split.
 static inline int split_groups(const pasn_dims& d) {
   if (d.N <= 0 || d.N > 74) return 1;
-  static const int allow = [] { const char* e = getenv("PASN_NO_SPLIT"); return (e && atoi(e) != 0) ? 0 : 1; }();
-  if (!allow) return 1;
   int best = 1;
   for (int g = 2; g <= d.S / TILE_M; ++g) {
     if (d.S % g != 0) continue;
@@ -520,7 +432,7 @@ static inline int split_groups(const pasn_dims& d) {
 constexpr int K2_MAX_GRID = 160;   // upper bound of K2's grid (one CTA per SM)
 struct WsLayout {
   int G, Nv, Sv, tiles2;
-  size_t off_osum, off_err, off_ready, off_owner, off_stash, off_featsv, off_fe, off_simv, off_logv, total;
+  size_t off_osum, off_err, off_stash, off_featsv, off_fe, off_simv, off_logv, total;
 };
 static inline WsLayout ws_layout(const pasn_dims& d) {
   WsLayout L;
@@ -531,8 +443,6 @@ static inline WsLayout ws_layout(const pasn_dims& d) {
   size_t o = (size_t)L.tiles2 * FE_TILE_BYTES;
   L.off_osum = o; o += align_up((size_t)L.Nv * d.P * 4, 256);
   L.off_err = o; o += 256;
-  L.off_ready = o; o += align_up((size_t)L.Nv * 4, 256);   // directly behind err: one memset clears both
-  L.off_owner = o; o += align_up((size_t)L.tiles2 * 4, 256);
   L.off_stash = o; o += align_up((size_t)K2_MAX_GRID * d.P * DD * 4, 256);   // push capture: FE row of each K2 CTA's best clip per prototype
   L.off_featsv = L.off_fe = L.off_simv = L.off_logv = o;
   if (L.G > 1) {
@@ -583,7 +493,6 @@ int sm100_head_forward(const void* feat, const pasn_weights& w, const void* pack
   uint8_t* feimg = reinterpret_cast<uint8_t*>(wsp);
   float* osum = reinterpret_cast<float*>(wsp + L.off_osum);
   int* err = reinterpret_cast<int*>(wsp + L.off_err);
-  int* ready = reinterpret_cast<int*>(wsp + L.off_ready);
 
   static const int num_sms = [] {
     int dev = 0, n = 0;
@@ -607,35 +516,14 @@ int sm100_head_forward(const void* feat, const pasn_weights& w, const void* pack
   k1.err = err;
   k1.fault = fault_word();
   k1.trace = g_trace;
-  { const char* e = getenv("PASN_DBG_SKIP"); k1.dbg_skip = e ? atoi(e) : 0; }
-  static const int flush_kmajor = [] { const char* e = getenv("PASN_FLUSH_KMAJOR"); return (PASN_K1_EXPERIMENTS && e) ? atoi(e) : 1; }();
-  static const int l2_hints = [] { const char* e = getenv("PASN_L2_HINTS"); return (PASN_K1_EXPERIMENTS && e) ? atoi(e) : 1; }();
-  k1.flush_kmajor = flush_kmajor; k1.l2_hints = l2_hints;
-  static const int x_drain = [] { const char* e = getenv("PASN_X_DRAIN"); return e ? atoi(e) : 0; }();
-  k1.x_drain = x_drain;
-  static const int spin = [] { const char* e = getenv("PASN_K1_SPIN"); return e ? atoi(e) : 0; }();
-  k1.spin = spin;
-  static const int flush_sleep = [] { const char* e = getenv("PASN_FLUSH_SLEEP"); return e ? atoi(e) : 0; }();
-  k1.flush_sleep = flush_sleep;
-  // clip-level hand-off to the prototype kernel: an experiment (measured slower), only in builds with -DPASN_K1_EXPERIMENTS=1
-  static const int k2_early = [] { const char* e = getenv("PASN_K2_EARLY"); return (PASN_K1_EXPERIMENTS && e) ? atoi(e) : 0; }();
-  k1.ready = k2_early ? ready : nullptr;
-  // The workspace's error word (what pasn_debug_sm100_error reads; faults themselves go to the sticky fault word) and the
-  // hand-off counters are only cleared when somebody will look at them: a memset in front of every call is ~2 us of the step.
+  // The workspace's error word (what pasn_debug_sm100_error reads; faults themselves go to the sticky fault word) is only
+  // cleared when somebody will look at it: a memset in front of every call is ~2 us of the step.
   static const int dbg_sync = [] { const char* e = getenv("PASN_DEBUG_SYNC"); return e ? atoi(e) : 0; }();
-  if ((k2_early || dbg_sync) && cudaMemsetAsync(err, 0, 256 + (size_t)L.Nv * 4, st) != cudaSuccess) return PASN_ERR_CUDA;
+  if (dbg_sync && cudaMemsetAsync(err, 0, sizeof(int), st) != cudaSuccess) return PASN_ERR_CUDA;
   const int grid1 = ceil_div(L.Nv, k1.clips_per_cta);
   const int ppad = (d.P + 7) / 8 * 8;
-  // Token-kernel tile orders (same results; profiles/README.md): 1 = serial (default), 2 = two-phase
-  static const int env_variant = [] {
-    const char* e = getenv("PASN_K1_PHASES");
-    const int v = e ? atoi(e) : 1;
-    return v == 2 ? 2 : 1;
-  }();
-  const int variant = g_k1_variant == 2 ? 2 : (g_k1_variant == 1 ? 1 : env_variant);
-  k1.phases = variant;
   main_kernel_begin(st);
-  const int rc = launch_k1_two_phase(k1, ppad, grid1, st);
+  const int rc = launch_k1(k1, ppad, grid1, st);
   if (rc) return rc;
   main_kernel_end(st);
   count_launch();
@@ -663,10 +551,6 @@ int sm100_head_forward(const void* feat, const pasn_weights& w, const void* pack
   k2.err = err;
   k2.fault = k1.fault;
   k2.trace = g_trace;
-  k2.a_kmajor = flush_kmajor; k2.l2_hints = l2_hints;
-  k2.ready = k2_early ? ready : nullptr; k2.cpc = k1.clips_per_cta; k2.grid1 = grid1;
-  k2.queue = err + 1;
-  k2.tile_owner = k2_early ? reinterpret_cast<int*>(wsp + L.off_owner) : nullptr;
   const int grid2 = k2.ntiles < num_sms ? k2.ntiles : num_sms;   // <= K2_MAX_GRID
   {  // programmatic dependent launch: K2's prologue (TMEM, barriers, norms, the resident W2 images) overlaps K1's tail
     cudaLaunchConfig_t cfg{};
@@ -680,8 +564,7 @@ int sm100_head_forward(const void* feat, const pasn_weights& w, const void* pack
   PASN_LAUNCH_CHECK();
   count_launch();
   if (k2.stash) {
-    push_capture_stash_kernel<<<d.P, 128, 0, st>>>(k2.best_key, d.P, k2.global_offset, L.Nv, k2.cpt, grid2, k2.tile_owner, k2.stash,
-                                                   push->best_vec);
+    push_capture_stash_kernel<<<d.P, 128, 0, st>>>(k2.best_key, d.P, k2.global_offset, L.Nv, k2.cpt, grid2, k2.stash, push->best_vec);
     PASN_LAUNCH_CHECK();
     count_launch();
   }

@@ -1,25 +1,19 @@
-// K1 of the fused prototype head, third generation: "two-phase" token kernel (see head_sm100.cu for K2, packing and the
-// host side, and for the reference computation being replaced: src/models/Video_XProtoNet.py:82-98).
+// K1 of the fused prototype head: the token kernel (see head_sm100.cu for K2, packing and the host side, and for the
+// reference computation being replaced: src/models/Video_XProtoNet.py:82-98).  Measurements in profiles/README.md.
 //
-// What changed against the first tcgen05 kernel, and why (measurements in profiles/README.md):
 //   * add-on branch transposed.  acc_A^T[d, voxel] = W1 X^T  (weights are the A operand, the X tile the B operand), so
 //     H1^T = relu(. + b1) is converted to bf16 IN PLACE in TMEM (lane = channel d, bias is a per-lane scalar) and feeds
-//     the pooling MMA  FEpartial^T[d,(slot,p)] = H1^T O  as its TMEM A operand.  H1 no longer goes through shared
-//     memory: 64 KB of st.shared per tile, the 32 KB Hs buffer and its two hand-offs are gone.
-//   * with Hs gone the CTA needs 187 KB of shared memory, which keeps 60 KB of L1.  The NCDHW gather is done with
-//     cp.async (8-byte LDGSTS, three 16 KB chunks in flight per SM): 22 B/clk/SM measured against 11 B/clk/SM for
-//     the ld.global -> st.shared version (whose register loads all shared one scoreboard, i.e. one unit in flight)
-//     and 13 B/clk/SM for cp.async when only 28 KB of L1 were left.
-//   * layer 1 split in two phases per tile, G = X W3^T into TMEM columns [0,256) and A^T into [256,512), each streaming
-//     its own weights and gathering the X tile again (second read hits L2).  Only half of TMEM is written at a time,
-//     so the serial chain of tile i (G1 -> G2 -> O -> pooling) overlaps the other phase's MMAs instead of leaving the
-//     tensor pipe idle:  [G(i+1) | H1^T convert, pooling, drain of tile i]  [A(i+1) | G1, G2, O chain of tile i+1].
-//     `phases == 1` keeps the old order (both accumulators per chunk, X gathered once, chain serial) for comparison.
+//     the pooling MMA  FEpartial^T[d,(slot,p)] = H1^T O  as its TMEM A operand.  H1 never goes through shared memory.
+//   * the CTA needs 187 KB of shared memory, which keeps 60 KB of L1.  The NCDHW gather is done with cp.async (8-byte
+//     LDGSTS, three 16 KB chunks in flight per SM): 22 B/clk/SM measured against 11 B/clk/SM for an
+//     ld.global -> st.shared version (whose register loads all shared one scoreboard, i.e. one unit in flight) and
+//     13 B/clk/SM for cp.async when only 28 KB of L1 were left.
+//   * per tile, layer 1 issues both accumulators chunk by chunk from one gathered X chunk: acc_G = X W3^T into TMEM
+//     columns [0,256), acc_A^T into [256,512).  The serial chain G1 -> G2 -> O -> pooling follows; its MMAs come from a
+//     second issuing thread, so its waits on the epilogue stay off the layer-1 issuer's path.
 //
 // Warp roles (16 warps): 0 layer-1 MMA issuer, 1 weight producer (cp.async.bulk), 2 tail MMA issuer (G2, O, pooling),
 // 3 occurrence-map store + column sums, 4-7 X gather, 8-15 epilogue (TMEM lane quadrant = warp % 4, two per quadrant).
-#include <cstdlib>
-
 #include "head_sm100_shared.cuh"
 
 namespace pasn {
@@ -28,13 +22,7 @@ using namespace k1;
 
 namespace {
 
-#ifndef PASN_XSLOTS
-#define PASN_XSLOTS 4
-#endif
-#ifndef PASN_WSLOTS
-#define PASN_WSLOTS 3
-#endif
-constexpr int XSLOTS = PASN_XSLOTS, WSLOTS = PASN_WSLOTS, XDEPTH = XSLOTS - 1;   // XDEPTH chunks of cp.async in flight per producer warp
+constexpr int XSLOTS = 4, WSLOTS = 3, XDEPTH = XSLOTS - 1;   // XDEPTH chunks of cp.async in flight per producer warp
 constexpr uint32_t XSLOT_BYTES = 16384, WSLOT_BYTES = 32768;
 constexpr int K1_WARPS = 16, K1_THREADS = K1_WARPS * 32;
 constexpr int W_MMA = 0, W_WPROD = 1, W_TAIL = 2, W_OCC = 3, W_X0 = 4, W_EPI0 = 8;
@@ -47,11 +35,11 @@ constexpr uint32_t SM_BIAS = SM_OS + OS_BYTES_MAX;                // 188416  b3[
 constexpr uint32_t SM_BAR = SM_BIAS + (DD + DD + DH) * 4;         // 190976
 constexpr uint32_t SM_MISC = SM_BAR + 36 * 8;                     // 191232
 constexpr uint32_t K1_SMEM = SM_MISC + 64;                        // 191296
-static_assert(PASN_XSLOTS != 4 || PASN_WSLOTS != 3 || K1_SMEM <= 195 * 1024, "keep the 196 KB carve-out (60 KB of L1 for the cp.async gather)");
+static_assert(K1_SMEM <= 195 * 1024, "keep the 196 KB carve-out (60 KB of L1 for the cp.async gather)");
 
 enum {
   B_XFULL = 0, B_XEMPTY = XSLOTS, B_WFULL = 2 * XSLOTS, B_WEMPTY = 2 * XSLOTS + WSLOTS, B_GDONE = 2 * XSLOTS + 2 * WSLOTS, B_ADONE, B_G1READY, B_G2DONE, B_G2READY, B_ODONE,
-  B_OSREADY, B_OSEMPTY, B_H1TREADY, B_FEDONE0, B_FEFREE0, B_FEDONE1, B_GBFREE, B_ABFREE, B_W4RDY, B_W4BRDY, B_W5RDY, B_COUNT
+  B_OSREADY, B_OSEMPTY, B_H1TREADY, B_FEDONE0, B_FEDONE1, B_GBFREE, B_ABFREE, B_W4RDY, B_W4BRDY, B_W5RDY, B_COUNT
 };
 static_assert(B_COUNT <= 36, "barrier table");
 
@@ -63,25 +51,17 @@ static_assert(B_COUNT <= 36, "barrier table");
 //                 FEpartial^T fp32 at [320, 320 + 2*PP) (lane = d % 128), one channel half after the other
 constexpr uint32_t COL_AT = 256, COL_H1T0 = 256, COL_H1T1 = 448, COL_FE = 320;
 
-__device__ __forceinline__ void split_points(int nkc, int& a1, int& a2) {  // where G2 / O sit inside the A phase
-  a1 = (3 * nkc) / 8;
-  a2 = (6 * nkc) / 8;
-}
-
 }  // namespace
 
 // Everything that is fixed per launch is a template parameter: the kernel is ~7 k instructions for five warp roles, and code
-// of orders / input kinds / experiments that do not run still spreads the ones that do over more instruction-cache lines
-// (ncu: 8 % of the issue slots lost to instruction fetch before; serial bf16 NCDHW instantiation 8256 -> ~5.5 k instructions).
+// of input kinds that do not run still spreads the ones that do over more instruction-cache lines
+// (ncu: 8 % of the issue slots lost to instruction fetch before; bf16 NCDHW instantiation 8256 -> ~5.5 k instructions).
 // IN: 0 = bf16 [N,C,S], 1 = bf16 channels_last [N,S,C], 2 = fp32 [N,C,S] (rounded to bf16 on the fly), 3 = fp16 [N,C,S],
 // 4 = fp16 channels_last.  fp16 maps are gathered byte for byte like bf16 ones; only the layer-1 MMAs (fp16 x fp16 against
 // fp16 weight images: kind::f16 takes no mixed fp16 / bf16 operands) and the map store differ.
-template <int PP, bool TRACE, bool TWO_PHASE, int IN>
+template <int PP, bool TRACE, int IN>
 __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Params p) {
   constexpr bool nsc = IN == 1 || IN == 4, f32_in = IN == 2, f16_in = IN == 3 || IN == 4;
-  const int dbg_skip = PASN_K1_EXPERIMENTS ? p.dbg_skip : 0, x_drain = PASN_K1_EXPERIMENTS ? p.x_drain : 0,
-            flush_sleep = PASN_K1_EXPERIMENTS ? p.flush_sleep : 0, flush_kmajor = PASN_K1_EXPERIMENTS ? p.flush_kmajor : 1,
-            l2_hints = PASN_K1_EXPERIMENTS ? p.l2_hints : 1;
   extern __shared__ __align__(1024) unsigned char smem[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BAR);
   uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + SM_MISC);
@@ -100,8 +80,7 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
   const int ntok = ncl * S;
   const int ntiles = (ntok + TILE_M - 1) / TILE_M;
   const PackedLayout PL = packed_layout(p.C);
-  Ctx ctx{p.err, abort_s, p.fault, p.spin};
-  constexpr bool two_phase = TWO_PHASE;   // (compile-time: the serial order's kernel is 14 % smaller without the other order's code)
+  Ctx ctx{p.err, abort_s, p.fault};
 
   if ((smem_u32(smem) & 1023u) != 0) {  // swizzled layouts need the 1024-byte alignment we asked for
     if (tid == 0) atomicCAS(p.err, 0, 900);
@@ -122,10 +101,9 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
     mbar_init(&bars[B_OSEMPTY], 2);   // pooling MMAs retired + occurrence warp (map store and column sums)
     mbar_init(&bars[B_H1TREADY], 8);
     mbar_init(&bars[B_FEDONE0], 1);
-    mbar_init(&bars[B_FEFREE0], 4);
     mbar_init(&bars[B_FEDONE1], 1);
     mbar_init(&bars[B_GBFREE], 8);
-    mbar_init(&bars[B_ABFREE], 4);
+    mbar_init(&bars[B_ABFREE], 8);    // both channel halves drained their FEpartial^T columns
     mbar_init(&bars[B_W4RDY], 1);
     mbar_init(&bars[B_W4BRDY], 1);
     mbar_init(&bars[B_W5RDY], 1);
@@ -150,8 +128,6 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
   const uint32_t tbase = *tmem_ptr_s;
   const uint32_t x_base = smem_u32(smem + SM_X), w_base = smem_u32(smem + SM_W), os_base = smem_u32(smem + SM_OS);
   const int nkc = p.nkc;
-  int a1, a2;
-  split_points(nkc, a1, a2);
 
   if (warp == W_MMA) {
     // ------------------------------------------------------------------ MMA issuer (one elected thread)
@@ -175,17 +151,12 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       const uint32_t idesc_g = f16_in ? make_idesc_16(128, 256, 0, 0, x_mn, 0) : make_idesc_bf16(128, 256, x_mn, 0);
       const uint32_t idesc_a = f16_in ? make_idesc_16(128, 128, 0, 0, 0, x_mn) : make_idesc_bf16(128, 128, 0, x_mn);
       const uint32_t xk = nsc ? 2u : 128u;                          // descriptor advance per K step of 16 channels
-      const uint32_t idesc_g2 = make_idesc_bf16(128, 128, 0, 0);
-      const uint32_t idesc_o = make_idesc_bf16(128, 64, 0, 0);
-      const uint32_t idesc_pool = make_idesc_bf16(128, NPOOL, 0, 1);  // A = H1^T in TMEM, B = Os (MN-major, no swizzle)
-      constexpr uint32_t lbo_os = (uint32_t)(NPOOL / 8) * 128u;
       constexpr uint32_t HI_SW128 = desc_hi(1024, SWZ_128B);   // X tile (MN-major) and weight images (K-major): SBO 1024
-      constexpr uint32_t HI_OS = desc_hi(128, SWZ_NONE);       // Os: MN-major, no swizzle, SBO 128
       const uint32_t tb = tbase;
-      const uint32_t x_lo0 = desc_lo(x_base, nsc ? 16u : 8192u), w_lo0 = desc_lo(w_base, 16), os_lo0 = desc_lo(os_base, lbo_os);
+      const uint32_t x_lo0 = desc_lo(x_base, nsc ? 16u : 8192u), w_lo0 = desc_lo(w_base, 16);
       const uint32_t bar0 = smem_u32(bars);
       auto baddr = [&](int b) -> uint32_t { return bar0 + 8u * (uint32_t)b; };
-      const uint32_t njobs = (uint32_t)ntiles * (uint32_t)nkc * (two_phase ? 2u : 1u);
+      const uint32_t njobs = (uint32_t)ntiles * (uint32_t)nkc;
       uint32_t xs = 0, xph = 0, xcount = 0;   // X ring: slot and phase parity of the next job, jobs taken so far
       uint32_t ws = 0, wph = 0;               // weight ring
       bool xr = false, wr = false;            // "already seen full" for the next job / stage (probed early)
@@ -222,13 +193,12 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         wr = mbar_test_wait(&bars[B_WFULL + ws], wph);
         return r;
       };
-      auto issue_g = [&](int kc, uint32_t sx, uint32_t sw, bool free_x) {   // 4 MMAs: one 64-channel chunk into acc_G
+      auto issue_g = [&](int kc, uint32_t sx, uint32_t sw) {   // 4 MMAs: one 64-channel chunk into acc_G (X slot freed by issue_a)
         const uint32_t alo = x_lo0 + sx * (XSLOT_BYTES >> 4), blo = w_lo0 + sw * (WSLOT_BYTES >> 4);
         mma_ss_x(tb, alo, HI_SW128, blo, HI_SW128, idesc_g, kc ? 1u : 0u);
 #pragma unroll
         for (int k4 = 1; k4 < 4; ++k4) mma_ss_x(tb, alo + k4 * xk, HI_SW128, blo + k4 * 2, HI_SW128, idesc_g, 1u);
         mma_commit_a(baddr(B_WEMPTY) + 8u * sw);
-        if (free_x) mma_commit_a(baddr(B_XEMPTY) + 8u * sx);
       };
       auto issue_a = [&](int kc, uint32_t sx, uint32_t sw) {   // 8 MMAs: one chunk into both channel halves of acc_A^T
         const uint32_t blo = x_lo0 + sx * (XSLOT_BYTES >> 4), alo = w_lo0 + sw * (WSLOT_BYTES >> 4);
@@ -242,10 +212,10 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         mma_commit_a(baddr(B_WEMPTY) + 8u * sw);
         mma_commit_a(baddr(B_XEMPTY) + 8u * sx);
       };
-      auto chunk_g = [&](int kc, uint32_t sx, bool free_x) -> bool {
+      auto chunk_g = [&](int kc, uint32_t sx) -> bool {
         uint32_t sw;
         if (!take_w(sw)) return false;
-        issue_g(kc, sx, sw, free_x);
+        issue_g(kc, sx, sw);
         return true;
       };
       auto chunk_a = [&](int kc, uint32_t sx) -> bool {
@@ -279,72 +249,37 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         if (!(ok = bwait(&bars[B_GBFREE], tp ^ 1, ctx, 101))) break;   // G-branch columns of the previous tile consumed
         tc_fence_after();
         stamp(tile, 1);
-        if (two_phase) {
-          for (int kc = 0; kc < nkc && ok; ++kc) {
-            long long tc0 = 0;
-            if constexpr (TRACE) tc0 = clock64();
-            uint32_t sx;
-            ok = take_x(sx) && chunk_g(kc, sx, true);
-            chunk_time(tile, kc, tc0);
-          }
-          if (!ok) break;
-          mma_commit_a(baddr(B_GDONE));
-          stamp(tile, 2);
-          if constexpr (TRACE) {
-            if (p.trace != nullptr && blockIdx.x == 0 && tile < 16) {
-              p.trace[(0 * 16 + tile) * 16 + 13] = xwait;
-              p.trace[(0 * 16 + tile) * 16 + 14] = wwait;
-            }
-          }
-          if (!(ok = bwait(&bars[B_ABFREE], tp ^ 1, ctx, 111))) break;   // previous tile's pooling drained
-          tc_fence_after();
-          stamp(tile, 3);
-          for (int kc = 0; kc < nkc && ok; ++kc) {
-            if (kc == a1) ok = pass_w(1, B_W4RDY) && pass_w(1, B_W4BRDY);
-            if (ok && kc == a2) ok = pass_w(1, B_W5RDY);
-            if (!ok) break;
-            long long tc0 = 0;
-            if constexpr (TRACE) tc0 = clock64();
-            uint32_t sx;
-            ok = take_x(sx) && chunk_a(kc, sx);
-            chunk_time(tile, 8 + kc, tc0);
-          }
-          if (!ok) break;
-          mma_commit_a(baddr(B_ADONE));
-          stamp(tile, 6);
-        } else {
-          if (!(ok = bwait(&bars[B_ABFREE], tp ^ 1, ctx, 111))) break;
-          tc_fence_after();
-          stamp(tile, 3);
-          // (G, A) blocks per chunk, except that the last `skew` chunks issue their G blocks first: acc_G is then
-          // complete -- and G1's conversion can start -- while the add-on blocks of those chunks are still running
-          // (their X slots stay held a little longer; at the end of a tile the ring has nothing urgent to prefetch)
-          // skew <= XSLOTS - (XDEPTH - 1): a chunk is only published once the XDEPTH - 1 chunks after it were issued,
-          // and those need free slots while this thread still holds `skew` of them
-          constexpr int SKEW = XSLOTS - (XDEPTH - 1) < 3 ? XSLOTS - (XDEPTH - 1) : 3;
-          // (only for channels_last input: the NCDHW gather is the slower one and does not like waiting for two chunks
-          // before the add-on block of the first -- measured 159.6 vs 157.3 us -- while channels_last gains 2-4 %)
-          const int skew = !nsc ? 0 : (nkc < SKEW ? nkc : SKEW), k_skew = nkc - skew;
-          for (int kc = 0; kc < k_skew && ok; ++kc) {
-            long long tc0 = 0;
-            if constexpr (TRACE) tc0 = clock64();
-            uint32_t sx;
-            ok = take_x(sx) && chunk_g(kc, sx, false) && chunk_a(kc, sx);
-            chunk_time(tile, kc, tc0);
-          }
-          uint32_t sxs[3] = {0, 0, 0};
-          for (int j = 0; j < skew && ok; ++j) ok = take_x(sxs[j]) && chunk_g(k_skew + j, sxs[j], false);
-          if (!ok) break;
-          mma_commit_a(baddr(B_GDONE));
-          stamp(tile, 2);
-          for (int j = 0; j < skew && ok; ++j) ok = chunk_a(k_skew + j, sxs[j]);
-          if (!ok) break;
-          mma_commit_a(baddr(B_ADONE));
-          stamp(tile, 6);
-          // the two halves of W4 are handed over one by one: the first eight G2 MMAs only need the first (the stages of
-          // the chain are requested late -- their ring slots free when the last layer-1 blocks retire -- and land ~0.5 k cycles apart)
-          ok = pass_w(1, B_W4RDY) && pass_w(1, B_W4BRDY) && pass_w(1, B_W5RDY);
+        if (!(ok = bwait(&bars[B_ABFREE], tp ^ 1, ctx, 111))) break;   // previous tile's pooling drained
+        tc_fence_after();
+        stamp(tile, 3);
+        // (G, A) blocks per chunk, except that the last `skew` chunks issue their G blocks first: acc_G is then
+        // complete -- and G1's conversion can start -- while the add-on blocks of those chunks are still running
+        // (their X slots stay held a little longer; at the end of a tile the ring has nothing urgent to prefetch)
+        // skew <= XSLOTS - (XDEPTH - 1): a chunk is only published once the XDEPTH - 1 chunks after it were issued,
+        // and those need free slots while this thread still holds `skew` of them
+        constexpr int SKEW = XSLOTS - (XDEPTH - 1) < 3 ? XSLOTS - (XDEPTH - 1) : 3;
+        // (only for channels_last input: the NCDHW gather is the slower one and does not like waiting for two chunks
+        // before the add-on block of the first -- measured 159.6 vs 157.3 us -- while channels_last gains 2-4 %)
+        const int skew = !nsc ? 0 : (nkc < SKEW ? nkc : SKEW), k_skew = nkc - skew;
+        for (int kc = 0; kc < k_skew && ok; ++kc) {
+          long long tc0 = 0;
+          if constexpr (TRACE) tc0 = clock64();
+          uint32_t sx;
+          ok = take_x(sx) && chunk_g(kc, sx) && chunk_a(kc, sx);
+          chunk_time(tile, kc, tc0);
         }
+        uint32_t sxs[3] = {0, 0, 0};
+        for (int j = 0; j < skew && ok; ++j) ok = take_x(sxs[j]) && chunk_g(k_skew + j, sxs[j]);
+        if (!ok) break;
+        mma_commit_a(baddr(B_GDONE));
+        stamp(tile, 2);
+        for (int j = 0; j < skew && ok; ++j) ok = chunk_a(k_skew + j, sxs[j]);
+        if (!ok) break;
+        mma_commit_a(baddr(B_ADONE));
+        stamp(tile, 6);
+        // the two halves of W4 are handed over one by one: the first eight G2 MMAs only need the first (the stages of
+        // the chain are requested late -- their ring slots free when the last layer-1 blocks retire -- and land ~0.5 k cycles apart)
+        ok = pass_w(1, B_W4RDY) && pass_w(1, B_W4BRDY) && pass_w(1, B_W5RDY);
         if constexpr (TRACE) {
           if (p.trace != nullptr && blockIdx.x == 0 && tile < 16) {
             p.trace[(0 * 16 + tile) * 16 + 11] = xwait;
@@ -371,8 +306,7 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       const uint32_t bar0 = smem_u32(bars);
       auto baddr = [&](int b) -> uint32_t { return bar0 + 8u * (uint32_t)b; };
       const uint32_t stages_per_tile = 2u * (uint32_t)nkc + 3u;
-      const uint32_t off_w4 = two_phase ? (uint32_t)(nkc + a1) : 2u * (uint32_t)nkc;
-      const uint32_t off_w5 = two_phase ? (uint32_t)(nkc + a2 + 2) : 2u * (uint32_t)nkc + 2u;
+      const uint32_t off_w4 = 2u * (uint32_t)nkc, off_w5 = off_w4 + 2u;   // after the tile's layer-1 stages
       bool ok = true;
       // stages are handed over by the layer-1 issuer (B_W4RDY / B_W5RDY) once they have landed
 
@@ -417,15 +351,11 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         // ---- pooling FEpartial^T = H1^T O, one channel half after the other (they share the FEpartial^T columns)
 #pragma unroll
         for (int step = 0; step < 2; ++step) {
-          // two-phase: both halves go through columns [320, 320+NPOOL) (the G-branch columns already belong to the next
-          // tile), so half 1 waits for half 0 to be drained.  Serial order: half 1 lands in the idle G-branch columns
-          // [0, NPOOL) and is issued back to back.
-          if (step == 0) ok = bwait(&bars[B_H1TREADY], tp, ctx, 108) && bwait(&bars[B_OSREADY], tp, ctx, 109);
-          else if (two_phase) ok = bwait(&bars[B_FEFREE0], tp, ctx, 110);
-          if (!ok) break;
+          // half 0 lands in [320, 320+NPOOL), half 1 in the idle G-branch columns [0, NPOOL): issued back to back
+          if (step == 0 && !(ok = bwait(&bars[B_H1TREADY], tp, ctx, 108) && bwait(&bars[B_OSREADY], tp, ctx, 109))) break;
           tc_fence_after();
           const uint32_t a0 = step ? COL_H1T1 : COL_H1T0;
-          const uint32_t d0 = (step && !two_phase) ? 0u : COL_FE;
+          const uint32_t d0 = step ? 0u : COL_FE;
 #pragma unroll
           for (int ks = 0; ks < 8; ++ks)
             mma_ts_x(tb + d0, tb + a0 + 8u * ks, os_lo0 + ks * (2 * lbo_os / 16), HI_OS, idesc_pool, ks ? 1u : 0u);
@@ -437,9 +367,8 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
     }
   } else if (warp == W_WPROD) {
     // ------------------------------------------------------------------ weight producer (one thread)
-    // stage order = consumption order of the issuer.  two-phase: W3[0..nkc), then W1[0..nkc) with W4a,W4b before
-    // chunk a1 and W5 before chunk a2.  single-phase: (W3[k], W1[k]) pairs, for the
-    // last two chunks all W3 before all W1 (skewed issue order), then W4a, W4b, W5.
+    // stage order = consumption order of the issuer: (W3[k], W1[k]) pairs, for the last `skew` chunks all W3 before
+    // all W1 (skewed issue order), then W4a, W4b, W5.
     if (lane == 0) {
       uint32_t wst = 0;
       bool ok = true;
@@ -447,29 +376,19 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         const uint32_t ws = wst % WSLOTS, wph = (wst / WSLOTS) & 1;
         ++wst;
         if (!bwait(&bars[B_WEMPTY + ws], wph ^ 1, ctx, 201)) return false;
-        if (dbg_skip & 1) { mbar_arrive(&bars[B_WFULL + ws]); return true; }
         mbar_arrive_expect_tx(&bars[B_WFULL + ws], bytes);
         for (uint32_t o = 0; o < bytes; o += 16384)
           bulk_g2s(w_base + ws * WSLOT_BYTES + o, p.packed + src + o, 16384, &bars[B_WFULL + ws]);
         return true;
       };
       for (int tile = 0; tile < ntiles && ok; ++tile) {
-        if (two_phase) {
-          for (int kc = 0; kc < nkc && ok; ++kc) ok = put(PL.off_l1 + (size_t)(2 * kc) * 32768, 32768);
-          for (int kc = 0; kc < nkc && ok; ++kc) {
-            if (kc == a1) ok = put(PL.off_w4, 32768) && put(PL.off_w4 + 32768, 32768);
-            if (ok && kc == a2) ok = put(PL.off_w5, 16384);
-            if (ok) ok = put(PL.off_l1 + (size_t)(2 * kc + 1) * 32768, 32768);
-          }
-        } else {
-          constexpr int SKEW = XSLOTS - (XDEPTH - 1) < 3 ? XSLOTS - (XDEPTH - 1) : 3;
-          const int skew = !nsc ? 0 : (nkc < SKEW ? nkc : SKEW), k_skew = nkc - skew;
-          for (int kc = 0; kc < k_skew && ok; ++kc)
-            ok = put(PL.off_l1 + (size_t)(2 * kc) * 32768, 32768) && put(PL.off_l1 + (size_t)(2 * kc + 1) * 32768, 32768);
-          for (int kc = k_skew; kc < nkc && ok; ++kc) ok = put(PL.off_l1 + (size_t)(2 * kc) * 32768, 32768);
-          for (int kc = k_skew; kc < nkc && ok; ++kc) ok = put(PL.off_l1 + (size_t)(2 * kc + 1) * 32768, 32768);
-          ok = ok && put(PL.off_w4, 32768) && put(PL.off_w4 + 32768, 32768) && put(PL.off_w5, 16384);
-        }
+        constexpr int SKEW = XSLOTS - (XDEPTH - 1) < 3 ? XSLOTS - (XDEPTH - 1) : 3;
+        const int skew = !nsc ? 0 : (nkc < SKEW ? nkc : SKEW), k_skew = nkc - skew;
+        for (int kc = 0; kc < k_skew && ok; ++kc)
+          ok = put(PL.off_l1 + (size_t)(2 * kc) * 32768, 32768) && put(PL.off_l1 + (size_t)(2 * kc + 1) * 32768, 32768);
+        for (int kc = k_skew; kc < nkc && ok; ++kc) ok = put(PL.off_l1 + (size_t)(2 * kc) * 32768, 32768);
+        for (int kc = k_skew; kc < nkc && ok; ++kc) ok = put(PL.off_l1 + (size_t)(2 * kc + 1) * 32768, 32768);
+        ok = ok && put(PL.off_w4, 32768) && put(PL.off_w4 + 32768, 32768) && put(PL.off_w5, 16384);
       }
     }
   } else if (warp >= W_X0 && warp < W_X0 + 4) {
@@ -479,30 +398,10 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
     // operand layout (zero fill past the clip range).  XDEPTH chunks are in flight per warp; a chunk is published
     // (wait_group, cross-proxy fence, one arrive per warp) once the chunks issued after it are on their way.  The
     // 16-byte L1-bypassing form needs an alignment NCDHW rows (392-byte pitch) only have for every other channel; TMA
-    // needs 16-byte global strides.  In two-phase mode every chunk is gathered twice (job order = MMA order).
+    // needs 16-byte global strides.  Job g is chunk g % nkc of tile g / nkc.
     const int xw = warp - W_X0;
-    const uint32_t jobs_per_tile = (uint32_t)nkc * (two_phase ? 2u : 1u);
-    const uint32_t njobs = (uint32_t)ntiles * jobs_per_tile;
+    const uint32_t njobs = (uint32_t)ntiles * (uint32_t)nkc;
     bool ok = true;
-    // Wait for the ring slot of job g.  If it is not free yet the ring is full and this warp is about to stall (typically
-    // while the tile's serial chain runs): everything still in flight is waited for and published first, so that the
-    // issuer finds all XSLOTS chunks ready when layer 1 of the next tile starts (published chunks normally trail the
-    // issued ones by XDEPTH - 1).  The decision is made by lane 0 and broadcast: the publish protocol is warp-collective.
-    auto slot_free_or_drain = [&](uint32_t g, uint32_t xs, uint32_t xph, uint32_t& pub) -> bool {
-      const uint32_t full = __shfl_sync(0xffffffffu, mbar_test_wait(&bars[B_XEMPTY + xs], xph ^ 1) ? 0u : 1u, 0);
-      if (full && x_drain) {
-        if (pub < g) {
-          cp_async_wait<0>();
-          while (pub < g) {
-            fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&bars[B_XFULL + (pub % XSLOTS)]);
-            ++pub;
-          }
-        }
-      }
-      return bwait(&bars[B_XEMPTY + xs], xph ^ 1, ctx, 301);
-    };
     if (nsc) {
       // channels_last feature map [N][S][C]: a voxel's 64 channels of a chunk are 128 contiguous, 16-byte aligned bytes,
       // i.e. one row of the K-major SWIZZLE_128B operand image.  16-byte L1-bypassing cp.async: eight lanes per voxel row,
@@ -517,15 +416,15 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       const int sub = lane & 7, r4 = lane >> 3;
       for (uint32_t g = 0; g < njobs; ++g) {
         const uint32_t xs = g % XSLOTS, xph = (g / XSLOTS) & 1;
-        if (!slot_free_or_drain(g, xs, xph, pub)) { ok = false; break; }
-        const int tile = (int)(g / jobs_per_tile);
-        const int kc = (int)((g - (uint32_t)tile * jobs_per_tile) % (uint32_t)nkc);
+        if (!bwait(&bars[B_XEMPTY + xs], xph ^ 1, ctx, 301)) { ok = false; break; }
+        const int tile = (int)(g / (uint32_t)nkc);
+        const int kc = (int)(g - (uint32_t)tile * (uint32_t)nkc);
         const uint32_t dst0 = x_base + xs * XSLOT_BYTES;
         const __nv_bfloat16* src0 = p.feat + ((size_t)c_begin * S + (size_t)tile * TILE_M) * p.C + kc * 64 + sub * 8;
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const int row = xw * 32 + j * 4 + r4;
-          const bool valid = tile * TILE_M + row < ntok && !(dbg_skip & 2);
+          const bool valid = tile * TILE_M + row < ntok;
           cp_async_16(dst0 + off_kmajor_sw128(row, sub * 8), src0 + (size_t)(valid ? row : 0) * p.C, valid ? 16u : 0u);
         }
         cp_async_commit();
@@ -549,26 +448,20 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       };
       for (uint32_t g = 0; g < njobs; ++g) {
         const uint32_t xs = g % XSLOTS, xph = (g / XSLOTS) & 1;
-        if (!slot_free_or_drain(g, xs, xph, pub)) { ok = false; break; }
-        const int tile = (int)(g / jobs_per_tile);
-        const int kc = (int)((g - (uint32_t)tile * jobs_per_tile) % (uint32_t)nkc);
+        if (!bwait(&bars[B_XEMPTY + xs], xph ^ 1, ctx, 301)) { ok = false; break; }
+        const int tile = (int)(g / (uint32_t)nkc);
+        const int kc = (int)(g - (uint32_t)tile * (uint32_t)nkc);
         const int t = tile * TILE_M + 4 * lane;
-        const bool valid = t < ntok && !(dbg_skip & 2);
+        const bool valid = t < ntok;
         const int clipl = valid ? t / S : 0;
         const int s = valid ? t - clipl * S : 0;
         // virtual clip -> (real clip, voxel group): rows of the feature map keep the real pitch SR
         const int vc = c_begin + clipl, rc = vc / p.G, vg = vc - rc * p.G;
         const __nv_bfloat16* src = p.feat + ((size_t)rc * p.C + kc * 64 + xw * 16) * p.SR + (size_t)vg * S + s;
         const uint32_t dst0 = x_base + xs * XSLOT_BYTES;
-        if (l2_hints) {
 #pragma unroll
-          for (int j = 0; j < 16; ++j)
-            cp_async_8_hint(dst0 + off_mnmajor_sw128(4 * lane, xw * 16 + j, 8192), src + (size_t)j * p.SR, valid ? 8u : 0u, pol_first);
-        } else {
-#pragma unroll
-          for (int j = 0; j < 16; ++j)
-            cp_async_8(dst0 + off_mnmajor_sw128(4 * lane, xw * 16 + j, 8192), src + (size_t)j * p.SR, valid ? 8u : 0u);
-        }
+        for (int j = 0; j < 16; ++j)
+          cp_async_8_hint(dst0 + off_mnmajor_sw128(4 * lane, xw * 16 + j, 8192), src + (size_t)j * p.SR, valid ? 8u : 0u, pol_first);
         cp_async_commit();
         if (pub + (XDEPTH - 1) <= g) {
           cp_async_wait<XDEPTH - 1>();
@@ -586,8 +479,8 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       const uint32_t nunits = 2 * njobs;
       auto load32 = [&](uint32_t u, float4* q) {
         const uint32_t g = u >> 1, h = u & 1;
-        const int tile = (int)(g / jobs_per_tile);
-        const int kc = (int)((g - (uint32_t)tile * jobs_per_tile) % (uint32_t)nkc);
+        const int tile = (int)(g / (uint32_t)nkc);
+        const int kc = (int)(g - (uint32_t)tile * (uint32_t)nkc);
         const int t = tile * TILE_M + 4 * lane;
         const bool valid = t < ntok;
         const int clipl = valid ? t / S : 0;
@@ -687,15 +580,11 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         if (lane < p.P) p.osum[(size_t)(c_begin + first_clip) * p.P + lane] = acc0;
         if (lane + 32 < p.P) p.osum[(size_t)(c_begin + first_clip) * p.P + lane + 32] = acc1;
         acc0 = s0[1]; acc1 = s1[1];
-        __syncwarp();
-        if (PASN_K1_EXPERIMENTS && p.ready != nullptr && lane == 0) red_release_gpu_add(p.ready + c_begin + first_clip, 1);
       }
       if ((last_tok + 1) % S == 0) {
         if (lane < p.P) p.osum[(size_t)(c_begin + last_clip) * p.P + lane] = acc0;
         if (lane + 32 < p.P) p.osum[(size_t)(c_begin + last_clip) * p.P + lane + 32] = acc1;
         acc0 = acc1 = 0.f;
-        __syncwarp();
-        if (PASN_K1_EXPERIMENTS && p.ready != nullptr && lane == 0) red_release_gpu_add(p.ready + c_begin + last_clip, 1);
       }
     }
   } else if (warp >= W_EPI0) {
@@ -712,45 +601,6 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
     for (int i = 0; i < PP; ++i) facc[i] = 0.f;
     bool ok = true;
     const uint64_t pol_last = l2_policy_evict_last();
-
-    // acc_A^T half hh (128 voxel columns of this warp's 32 channel lanes) -> H1^T = relu(. + b1[d]) bf16, in place.
-    // hh = 0 packs upwards into [256,320), hh = 1 downwards into [448,512): every store lands on columns whose fp32
-    // content this warp has already loaded, and [320,448) is left free for FEpartial^T.
-    auto h1t_convert = [&](int tile) -> bool {
-      if (!bwait(&bars[B_ADONE], tile & 1, ctx, 507)) return false;
-      tc_fence_after();
-      if (tr) K1_TRACE(1, tile, 7);
-      uint32_t ra[32], rb[32], pk[16];
-      const int c0 = hh ? 3 : 0, dc = hh ? -1 : 1;
-      const uint32_t src = COL_AT + 128u * hh, dst = hh ? COL_H1T1 : COL_H1T0;
-      auto cvt = [&](const uint32_t (&r)[32]) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j)
-          pk[j] = pack_bf16x2_relu(__uint_as_float(r[2 * j]) + b1d, __uint_as_float(r[2 * j + 1]) + b1d);
-      };
-      tmem_ld_x32(tl + src + 32 * c0, ra);
-      tmem_ld_wait();
-      tmem_ld_x32(tl + src + 32 * (c0 + dc), rb);
-      cvt(ra);
-      tmem_st_x16(tl + dst + 16 * c0, pk);
-      tmem_ld_wait();
-      tmem_ld_x32(tl + src + 32 * (c0 + 2 * dc), ra);
-      cvt(rb);
-      tmem_st_x16(tl + dst + 16 * (c0 + dc), pk);
-      tmem_ld_wait();
-      tmem_ld_x32(tl + src + 32 * (c0 + 3 * dc), rb);
-      cvt(ra);
-      tmem_st_x16(tl + dst + 16 * (c0 + 2 * dc), pk);
-      tmem_ld_wait();
-      cvt(rb);
-      tmem_st_x16(tl + dst + 16 * (c0 + 3 * dc), pk);
-      tmem_st_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bars[B_H1TREADY]);
-      if (tr) K1_TRACE(1, tile, 8);
-      return true;
-    };
 
     for (int tile = 0; tile < ntiles && ok; ++tile) {
       const uint32_t tp = tile & 1;
@@ -793,8 +643,43 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       if (lane == 0) mbar_arrive(&bars[B_G1READY]);
       if (tr) K1_TRACE(1, tile, 2);
 
-      // single-phase order: acc_A^T is complete already, convert it while the G2 MMAs run
-      if (!two_phase && !(ok = h1t_convert(tile))) break;
+      // ---- E2: acc_A^T half hh (128 voxel columns of this warp's 32 channel lanes) -> H1^T = relu(. + b1[d]) bf16, in
+      //      place, while the G2 MMAs run.  hh = 0 packs upwards into [256,320), hh = 1 downwards into [448,512): every
+      //      store lands on columns whose fp32 content this warp has already loaded, and [320,448) is left free for FEpartial^T.
+      if (!(ok = bwait(&bars[B_ADONE], tp, ctx, 507))) break;
+      tc_fence_after();
+      if (tr) K1_TRACE(1, tile, 7);
+      {
+        uint32_t ra[32], rb[32], pk[16];
+        const int c0 = hh ? 3 : 0, dc = hh ? -1 : 1;
+        const uint32_t src = COL_AT + 128u * hh, dst = hh ? COL_H1T1 : COL_H1T0;
+        auto cvt = [&](const uint32_t (&r)[32]) {
+#pragma unroll
+          for (int j = 0; j < 16; ++j)
+            pk[j] = pack_bf16x2_relu(__uint_as_float(r[2 * j]) + b1d, __uint_as_float(r[2 * j + 1]) + b1d);
+        };
+        tmem_ld_x32(tl + src + 32 * c0, ra);
+        tmem_ld_wait();
+        tmem_ld_x32(tl + src + 32 * (c0 + dc), rb);
+        cvt(ra);
+        tmem_st_x16(tl + dst + 16 * c0, pk);
+        tmem_ld_wait();
+        tmem_ld_x32(tl + src + 32 * (c0 + 2 * dc), ra);
+        cvt(rb);
+        tmem_st_x16(tl + dst + 16 * (c0 + dc), pk);
+        tmem_ld_wait();
+        tmem_ld_x32(tl + src + 32 * (c0 + 3 * dc), rb);
+        cvt(ra);
+        tmem_st_x16(tl + dst + 16 * (c0 + 2 * dc), pk);
+        tmem_ld_wait();
+        cvt(rb);
+        tmem_st_x16(tl + dst + 16 * (c0 + 3 * dc), pk);
+      }
+      tmem_st_wait();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bars[B_H1TREADY]);
+      if (tr) K1_TRACE(1, tile, 8);
 
       // ---- E3: acc_G2 (cols [64,192)) -> G2 = relu(. + b4) bf16 in place at [64+64hh, +32)
       if (!(ok = bwait(&bars[B_G2DONE], tp, ctx, 503))) break;
@@ -852,9 +737,6 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
       if (lane == 0) mbar_arrive(&bars[B_OSREADY]);
       if (tr) K1_TRACE(1, tile, 6);
 
-      // two-phase order: the A phase ends after the O MMAs were issued
-      if (two_phase && !(ok = h1t_convert(tile))) break;
-
       // ---- E5: drain FEpartial^T of this warp's channel half (lane = d % 128) into per-clip register accumulators;
       //      finished clips leave as bf16 hi/lo rows of the K2 operand images
       if (!(ok = bwait(&bars[hh ? B_FEDONE1 : B_FEDONE0], tp, ctx, 506))) break;
@@ -865,7 +747,7 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
         const int last_clip = last_tok / S;
         const bool boundary = last_clip > first_clip;
         const bool ends = ((last_tok + 1) % S) == 0;
-        const uint32_t fe = tl + ((hh && !two_phase) ? 0u : COL_FE);   // serial order: half 1 sits in the G-branch columns
+        const uint32_t fe = tl + (hh ? 0u : COL_FE);   // half 1 sits in the G-branch columns
         uint32_t nb[PP];  // slot-1 partial = start of the next clip (only meaningful when `boundary`)
         {
           uint32_t a[PP];
@@ -879,71 +761,31 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
 #pragma unroll
           for (int j = 0; j < PP; ++j) facc[j] += __uint_as_float(a[j]);
         }
-        // FEpartial^T columns read: half 0 hands them to half 1's pooling MMAs, half 1 frees [256,512) for the next A phase
+        // FEpartial^T columns read: once both halves are, the next tile's layer-1 MMAs may overwrite them
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&bars[hh ? B_ABFREE : B_FEFREE0]);
+        if (lane == 0) mbar_arrive(&bars[B_ABFREE]);
         if (tr) K1_TRACE(1, tile, 10);
 #pragma unroll 1
         for (int rep = 0; rep < 2; ++rep) {
           const bool flush = rep == 0 ? boundary : ends;
           if (!flush) continue;
-          if (dbg_skip & 8) {   // timing experiment: no hi/lo split, no stores (results garbage)
-            if (PASN_K1_EXPERIMENTS && p.ready != nullptr && lane == 0) red_release_gpu_add(p.ready + c_begin + (rep == 0 ? first_clip : last_clip), 1);
-            if (rep == 0) {
-#pragma unroll
-              for (int j = 0; j < PP; ++j) facc[j] = __uint_as_float(nb[j]);
-            } else {
-#pragma unroll
-              for (int j = 0; j < PP; ++j) facc[j] = 0.f;
-            }
-            continue;
-          }
           const int clip = c_begin + (rep == 0 ? first_clip : last_clip);
           const int tile2 = clip / p.cpt;
           const int rowb = (clip - tile2 * p.cpt) * PP;
           uint8_t* img = p.feimg + (size_t)tile2 * FE_TILE_BYTES + (size_t)(d >> 6) * 16384;
-          if (flush_kmajor) {
-            // K2's A operand K-major (row = (clip,p), k = d contiguous): the 32 lanes of a warp hold 32 consecutive d of
-            // one row, i.e. 64 bytes inside one 128-byte swizzle row -> one line per warp store (hi at +0, lo at +64 KB)
+          // K2's A operand K-major (row = (clip,p), k = d contiguous): the 32 lanes of a warp hold 32 consecutive d of
+          // one row, i.e. 64 bytes inside one 128-byte swizzle row -> one line per warp store (hi at +0, lo at +64 KB);
+          // evict_last: K2 reads them right after this kernel
 #pragma unroll
-            for (int j = 0; j < PP; ++j) {
-              const float v = facc[j];
-              const __nv_bfloat16 h = __float2bfloat16_rn(v);
-              const __nv_bfloat16 l = __float2bfloat16_rn(v - __bfloat162float(h));
-              const uint32_t off = off_kmajor_sw128(rowb + j, d & 63);
-              if (l2_hints) {
-                st_global_u16_hint(img + off, __bfloat16_as_ushort(h), pol_last);
-                st_global_u16_hint(img + 65536 + off, __bfloat16_as_ushort(l), pol_last);
-              } else {
-                *reinterpret_cast<__nv_bfloat16*>(img + off) = h;
-                *reinterpret_cast<__nv_bfloat16*>(img + 65536 + off) = l;
-              }
-              // the burst of 2*PP stores per thread competes with the feature gather of the next tile's first chunks
-              // for the load/store path; these warps have nothing to do until that tile's layer 1 is done, so pace it
-              if (flush_sleep && (j & 3) == 3) __nanosleep(flush_sleep);
-            }
-          } else {
-            // K2's A operand MN-major (row = (clip,p) contiguous, k = d): this thread's PP values for its d are
-            // PP/8 16-byte chunks per image: rows [rowb, rowb+PP) of k-chunk image d/64, hi at +0 and lo at +64 KB
-#pragma unroll
-            for (int c = 0; c < PP / 8; ++c) {
-              uint32_t hi4[4], lo4[4];
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const float v0 = facc[8 * c + 2 * j], v1 = facc[8 * c + 2 * j + 1];
-                const float h0 = round_bf16(v0), h1 = round_bf16(v1);
-                hi4[j] = pack_bf16x2(h0, h1);
-                lo4[j] = pack_bf16x2(v0 - h0, v1 - h1);
-              }
-              const uint32_t off = off_mnmajor_sw128(rowb + 8 * c, d & 63, 8192);
-              *reinterpret_cast<uint4*>(img + off) = make_uint4(hi4[0], hi4[1], hi4[2], hi4[3]);
-              *reinterpret_cast<uint4*>(img + 65536 + off) = make_uint4(lo4[0], lo4[1], lo4[2], lo4[3]);
-            }
+          for (int j = 0; j < PP; ++j) {
+            const float v = facc[j];
+            const __nv_bfloat16 h = __float2bfloat16_rn(v);
+            const __nv_bfloat16 l = __float2bfloat16_rn(v - __bfloat162float(h));
+            const uint32_t off = off_kmajor_sw128(rowb + j, d & 63);
+            st_global_u16_hint(img + off, __bfloat16_as_ushort(h), pol_last);
+            st_global_u16_hint(img + 65536 + off, __bfloat16_as_ushort(l), pol_last);
           }
-          // hand the clip to the prototype kernel (it polls the counter; see proto_w2_kernel)
-          __syncwarp();
-          if (PASN_K1_EXPERIMENTS && p.ready != nullptr && lane == 0) red_release_gpu_add(p.ready + clip, 1);
           if (rep == 0) {
 #pragma unroll
             for (int j = 0; j < PP; ++j) facc[j] = __uint_as_float(nb[j]);
@@ -968,32 +810,30 @@ __global__ void __launch_bounds__(K1_THREADS, 1) head_tokens2_kernel(const K1Par
   }
 }
 
-template <int PP, bool TRACE, bool TWO_PHASE, int IN>
+template <int PP, bool TRACE, int IN>
 static int launch_inst(const K1Params& k1, int grid, cudaStream_t st) {
   static bool attr_done = false;
   if (!attr_done) {
-    if (cudaFuncSetAttribute(head_tokens2_kernel<PP, TRACE, TWO_PHASE, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM) != cudaSuccess)
+    if (cudaFuncSetAttribute(head_tokens2_kernel<PP, TRACE, IN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K1_SMEM) != cudaSuccess)
       return PASN_ERR_CUDA;
     attr_done = true;
   }
-  head_tokens2_kernel<PP, TRACE, TWO_PHASE, IN><<<grid, K1_THREADS, K1_SMEM, st>>>(k1);
+  head_tokens2_kernel<PP, TRACE, IN><<<grid, K1_THREADS, K1_SMEM, st>>>(k1);
   PASN_LAUNCH_CHECK();
   return PASN_OK;
 }
 template <int PP>
 static int launch_one(const K1Params& k1, int grid, cudaStream_t st) {
   // The instrumented instantiation (clock reads on the issue path) only runs while a trace buffer is installed.  The
-  // two-phase order (an A/B variant, slower) and the trace exist for bf16 maps; fp32 and fp16 maps always run the plain
-  // serial kernel.
+  // trace exists for bf16 maps; fp32 and fp16 maps always run the plain kernel.
   const bool tr = k1.trace != nullptr;
-  if (k1.f32_in) return launch_inst<PP, false, false, 2>(k1, grid, st);
-  if (k1.f16_in) return k1.nsc ? launch_inst<PP, false, false, 4>(k1, grid, st) : launch_inst<PP, false, false, 3>(k1, grid, st);
-  if (k1.nsc) return tr ? launch_inst<PP, true, false, 1>(k1, grid, st) : launch_inst<PP, false, false, 1>(k1, grid, st);
-  if (k1.phases != 1) return tr ? launch_inst<PP, true, true, 0>(k1, grid, st) : launch_inst<PP, false, true, 0>(k1, grid, st);
-  return tr ? launch_inst<PP, true, false, 0>(k1, grid, st) : launch_inst<PP, false, false, 0>(k1, grid, st);
+  if (k1.f32_in) return launch_inst<PP, false, 2>(k1, grid, st);
+  if (k1.f16_in) return k1.nsc ? launch_inst<PP, false, 4>(k1, grid, st) : launch_inst<PP, false, 3>(k1, grid, st);
+  if (k1.nsc) return tr ? launch_inst<PP, true, 1>(k1, grid, st) : launch_inst<PP, false, 1>(k1, grid, st);
+  return tr ? launch_inst<PP, true, 0>(k1, grid, st) : launch_inst<PP, false, 0>(k1, grid, st);
 }
 
-int launch_k1_two_phase(const K1Params& k1, int ppad, int grid, cudaStream_t st) {
+int launch_k1(const K1Params& k1, int ppad, int grid, cudaStream_t st) {
   if (ppad <= 16) return launch_one<16>(k1, grid, st);
   if (ppad <= 32) return launch_one<32>(k1, grid, st);
   if (ppad <= 40) return launch_one<40>(k1, grid, st);

@@ -1,5 +1,5 @@
-// Definitions shared by the single-CTA and CTA-pair variants of the fused token kernel (head_sm100.cu,
-// head_sm100_pair.cu): tile constants, packed-weight layout, kernel parameters, bounded waits, epilogue helpers.
+// Definitions shared by the fused head's token kernel (head_sm100_k1.cu) and its host side and prototype kernel
+// (head_sm100.cu): tile constants, packed-weight layout, kernel parameters, bounded waits, epilogue helpers.
 #pragma once
 #include "common.cuh"
 #include "sm100_prims.cuh"
@@ -12,7 +12,6 @@ constexpr int TILE_M = 128;
 constexpr int DD = 256;            // prototype depth D handled by this kernel
 constexpr int DH = DD / 2;         // occurrence hidden width
 constexpr int PP_MAX = 48;         // padded prototype count limit (multiple of 8)
-constexpr int K1_READY_TARGET = 9;  // 8 epilogue warps + the occurrence warp
 constexpr uint32_t FE_TILE_BYTES = 131072;  // K2 operand images of one 128-row tile: hi 64 KB | lo 64 KB
 
 // packed weight buffer (bf16 stage images + fp32 biases), see pack_weights_kernel
@@ -50,41 +49,20 @@ struct K1Params {
   int* err;
   int* fault;                  // host-mapped sticky fault word (or null)
   long long* trace;            // optional [3][16][16] clock64 stamps of CTA 0 (MMA thread, epilogue warp 4)
-  int phases;                  // two-phase kernel: 2 = G / A phases overlapped with the previous chain, 1 = serial order
-  int dbg_skip;                // timing experiments only: bit0 = do not copy weight stages, bit1 = do not gather X,
-                               // bit3 = do not flush finished clips (head_sm100_k1.cu only)
-  int flush_kmajor;            // 1: finished clips leave as 2-byte stores into K-major SWIZZLE_128B operand images (one 128-byte
-                               // line per warp store); 0: 16-byte chunks of MN-major images (32 lines per warp store)
-  int* ready;                  // [N] per-clip hand-off counter to the prototype kernel: +1 per epilogue warp that has stored
-                               // its part of the clip's pooled vectors, +1 for the clip's Osum row (K1_READY_TARGET in total)
-  int l2_hints;                // 1: pooled-vector images are stored evict_last, the feature map is read evict_first
-  int flush_sleep;             // ns slept after every fourth prototype row of a clip flush (0: none)
-  int x_drain;                 // 1: feature-gather warps publish everything in flight before they block on a full ring
-  int spin;                    // Ctx::spin
   int f16_in;                  // fp16 feature map (read as it is; layer-1 MMAs fp16 x fp16 with fp16 weight images), map in fp16
 };
-
-// 1: build the timing experiments of profiles/README.md into the fused kernels (PASN_DBG_SKIP, PASN_X_DRAIN, PASN_FLUSH_SLEEP,
-// PASN_FLUSH_KMAJOR, PASN_L2_HINTS, PASN_K2_EARLY); 0 (the product build): those switches are constants and their code is gone
-#ifndef PASN_K1_EXPERIMENTS
-#define PASN_K1_EXPERIMENTS 0
-#endif
 
 struct Ctx {
   int* err;
   volatile int* abort_s;
   int* fault;   // host-mapped sticky fault word (may be null)
-  int spin;     // bit per waiter class (wait code / 100: 1 issuers, 2-3 producers, 4 occurrence warp, 5 epilogue, 6 K2):
-                // poll with test_wait (never suspends) instead of try_wait (may suspend the thread for a while)
 };
 
 // bounded wait: returns false (and raises the CTA-wide abort flag) instead of hanging on a protocol bug.  The spin is
 // out of line so that the fast path at every call site is a single try_wait.
-static __device__ __noinline__ bool bwait_slow(uint64_t* bar, uint32_t parity, int* err, volatile int* abort_s, int* fault, int code,
-                                               int spin) {
+static __device__ __noinline__ bool bwait_slow(uint64_t* bar, uint32_t parity, int* err, volatile int* abort_s, int* fault, int code) {
   const long long t0 = clock64();
-  const bool poll = (spin >> (code / 100)) & 1;
-  while (!(poll ? mbar_test_wait(bar, parity) : mbar_try_wait(bar, parity))) {
+  while (!mbar_try_wait(bar, parity)) {
     if (*abort_s) return false;
     if (clock64() - t0 > 4000000000ll) {
       *abort_s = 1;
@@ -97,7 +75,7 @@ static __device__ __noinline__ bool bwait_slow(uint64_t* bar, uint32_t parity, i
 }
 __device__ __forceinline__ bool bwait(uint64_t* bar, uint32_t parity, const Ctx& c, int code) {
   if (mbar_try_wait(bar, parity)) return true;
-  return bwait_slow(bar, parity, c.err, c.abort_s, c.fault, code, c.spin);
+  return bwait_slow(bar, parity, c.err, c.abort_s, c.fault, code);
 }
 
 __device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
@@ -126,7 +104,7 @@ __device__ __forceinline__ void bias_relu_pack(const uint32_t (&r)[32], const fl
 
 }  // namespace k1
 
-// two-phase token kernel (head_sm100_k1.cu)
-int launch_k1_two_phase(const k1::K1Params& k1p, int ppad, int grid, cudaStream_t st);
+// token kernel (head_sm100_k1.cu)
+int launch_k1(const k1::K1Params& k1p, int ppad, int grid, cudaStream_t st);
 
 }  // namespace pasn

@@ -119,18 +119,6 @@ __device__ __forceinline__ void bulk_g2s_hint(uint32_t dst_smem, const void* src
                : "memory");
 }
 
-// gpu-scope release / acquire on a global counter (cross-kernel hand-off of finished work items)
-__device__ __forceinline__ void red_release_gpu_add(int* addr, int v) {
-  asm volatile("red.release.gpu.global.add.s32 [%0], %1;" ::"l"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ int ld_acquire_gpu(const int* addr) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(addr) : "memory");
-  return v;
-}
-// generic-proxy view of global memory (after an acquire) -> visible to subsequent async-proxy (bulk copy) reads
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 // arrive on `bar` (without bumping its pending count) once all cp.async issued so far by this thread have landed
 __device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* bar) {
   asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");

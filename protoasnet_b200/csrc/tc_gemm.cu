@@ -16,16 +16,8 @@
 // with remote arrivals.  Per flop a pair pulls 2/3 of the bytes from L2 that two independent CTAs would (the chain's big
 // GEMMs are bound by the ~6300 B/clk L2 -> SM fabric, not by the tensor pipe: profiles/README.md).
 //
-// MODE 2 ("quad") puts two such pairs in one 4-CTA cluster on M-adjacent 256-row tiles.  They need the same B tile, so each of
-// the four CTAs loads a quarter of it and the TMA unit multicasts it into the CTA of the other pair that holds the same
-// half: per 64-deep k-block a CTA then pulls 16 + 8 KB through the L2 -> SM fabric instead of 16 + 16 (the long-K GEMMs
-// run exactly at that fabric's limit).  A stage may only be refilled once BOTH pairs have consumed it: their commits
-// arrive on the "stage free" barriers of all four CTAs.  Opt-in (PASN_GEMM_QUAD=1): measured slower than plain pairs.
-//
 // Every mbarrier wait is bounded: a protocol fault becomes an error code in *err, not a hung GPU.
 #include <cuda.h>
-
-#include <cstdlib>
 
 #include "sm100_prims.cuh"
 #include "tc_gemm.cuh"
@@ -56,7 +48,6 @@ struct alignas(64) KParams {
   int out_tma[2];
   int tall;   // 1: a tile has two 128-row (per CTA) sub-tiles that share each B stage; they take the two accumulator buffers
   int tiles_m, tiles_n, nkb;
-  int warm;   // 1: the producer touches its first operand boxes before waiting for the grid in front (see the kernel)
   int* err;
   long long* trace;   // optional: 64 globaltimer stamps of CTA 0 (tools/trace_gemm.py)
 };
@@ -72,15 +63,6 @@ __device__ __forceinline__ void tma_load_3d_2sm(uint32_t dst, const CUtensorMap*
   asm volatile(
       "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(dst),
       "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar) & 0xFEFFFFFFu)
-      : "memory");
-}
-// ... and multicast: the box lands at the same shared-memory offset in every CTA of `mask`, the bytes are counted on the
-// barrier of each destination CTA's pair leader
-__device__ __forceinline__ void tma_load_3d_2sm_mc(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, uint64_t* bar,
-                                                   uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3, %4}], [%5], %6;" ::"r"(dst),
-      "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar) & 0xFEFFFFFFu), "h"(mask)
       : "memory");
 }
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2) {
@@ -140,9 +122,8 @@ enum {
   EPI_PSUM = E_BIT_OUT | E_BIT_PSUM,
   EPI_AUX = E_BIT_OUT | E_BIT_AUX,
 };
-template <int MODE, int EPI>   // MODE 0: one CTA per tile, 1: CTA pairs, 2: two pairs per cluster sharing the B tile by multicast
+template <bool PAIR, int EPI>   // PAIR: CTA pairs, else one CTA per tile
 __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_constant__ KParams kp) {
-  constexpr bool PAIR = MODE >= 1, QUAD = MODE == 2;
   constexpr bool E_AUX = (EPI & E_BIT_AUX) != 0, E_PSUM = (EPI & E_BIT_PSUM) != 0, E_STAT = (EPI & E_BIT_STAT) != 0,
                  E_DIRECT = (EPI & E_BIT_DIRECT) != 0, E_OUT = (EPI & E_BIT_OUT) != 0, E_ABSOUT = (EPI & E_BIT_ABSOUT) != 0,
                  E_SPLIT = E_DIRECT, E_F16 = (EPI & E_BIT_F16) != 0;
@@ -158,9 +139,8 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
   if (tid == 0) TCG_TRACE(0);
   const uint32_t crank = PAIR ? cluster_ctarank() : 0u;         // rank in the cluster
   const uint32_t rank = crank & 1u;                             // rank in the pair: 0 = leader
-  const uint32_t pq = crank >> 1;                               // pair inside a quad
   if (tid == 0) {
-    for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&bars[B_FULL + i], 1); mbar_init(&bars[B_EMPTY + i], QUAD ? 2 : 1); }
+    for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&bars[B_FULL + i], 1); mbar_init(&bars[B_EMPTY + i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&bars[B_ACCFULL + i], 1); mbar_init(&bars[B_ACCEMPTY + i], PAIR ? 2 * EPI_WARPS : EPI_WARPS); }
     mbar_init(&bars[B_WARM], 1);
     fence_mbar_init();
@@ -187,14 +167,13 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
   const int bnl = PAIR ? bn / 2 : bn;                           // rows of the B tile this CTA loads
   const int tiles_per_batch = kp.tiles_m * kp.tiles_n;
   const int ntiles = g.batch * tiles_per_batch;
-  constexpr int CL = QUAD ? 4 : (PAIR ? 2 : 1);                             // CTAs per cluster = per tile
-  const int tile0 = (int)(blockIdx.x / CL);                                 // persistent walk of this CTA / pair / quad
+  constexpr int CL = PAIR ? 2 : 1;                                          // CTAs per cluster = per tile
+  const int tile0 = (int)(blockIdx.x / CL);                                 // persistent walk of this CTA / pair
   const int tstep = (int)(gridDim.x / CL);
-  constexpr int BMP = PAIR ? 2 * BM : BM;                                   // rows of one MMA (a pair's share)
-  constexpr int BMC = CL * BM;                                              // rows of one sub-tile across the cluster
+  constexpr int BMC = CL * BM;                                              // rows of one sub-tile (one MMA) across the cluster
   const int nu = kp.tall ? 2 : 1;                                           // sub-tiles per tile (long-K GEMMs: see launch())
   const int BMT = BMC * nu;                                                 // rows of a (cluster) tile
-  const uint16_t pair_mask = (uint16_t)(3u << (2u * pq));                   // the two CTAs of this pair
+  const uint16_t pair_mask = (uint16_t)(3u << (crank & ~1u));               // the two CTAs of this pair
   const uint32_t a_stage = A_BYTES * (uint32_t)nu;                          // A boxes of a stage (one per sub-tile)
   const uint32_t stage_bytes = a_stage + (uint32_t)bnl * 128u;              // multiple of 1024: swizzle atoms stay aligned
   const uint32_t nst_fit = (STAGES * STAGE_BYTES) / stage_bytes;
@@ -210,12 +189,12 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
         if constexpr (PAIR) tma_load_3d_2sm(dst, map, c0, c1, c2, bar);
         else tma_load_3d(dst, map, c0, c1, c2, bar);
       };
-      if (kp.warm && tile0 < ntiles) {
+      if (tile0 < ntiles) {
         // The first load of a launch takes ~2.7 us (tensor-map fetch, translation, cold lines) against ~1 us later on: touch
         // the first boxes of both operands while the grid in front is still draining.  What lands may be stale (A is being
         // written by that grid) and is thrown away; the real loads below overwrite the stage.
         const int b = tile0 / tiles_per_batch, r = tile0 - b * tiles_per_batch;
-        const int m0 = (r / kp.tiles_n) * BMT + (int)pq * BMP + (int)rank * BM, n0 = (r % kp.tiles_n) * bn + (int)rank * bnl;
+        const int m0 = (r / kp.tiles_n) * BMT + (int)rank * BM, n0 = (r % kp.tiles_n) * bn + (int)rank * bnl;
         const bool split_k = g.k_rows_per_batch > 0;
         const int krow = split_k ? b * g.k_rows_per_batch : 0;
         const uint32_t a_tx = g.a_mn_major ? 8192u : A_BYTES, b_tx = g.b_mn_major ? 8192u : (uint32_t)bnl * 128u;
@@ -227,10 +206,10 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
       }
       griddep_wait();
       TCG_TRACE(2);   // the grid in front has completed
-      if (kp.warm && tile0 < ntiles) ok = bwait(&bars[B_WARM], 0, kp.err, 702);
+      if (tile0 < ntiles) ok = bwait(&bars[B_WARM], 0, kp.err, 702);
       for (int t = tile0; t < ntiles && ok; t += tstep) {
         const int b = t / tiles_per_batch, r = t - b * tiles_per_batch;
-        const int m0 = (r / kp.tiles_n) * BMT + (int)pq * BMP + (int)rank * BM, n0 = (r % kp.tiles_n) * bn + (int)rank * bnl;
+        const int m0 = (r / kp.tiles_n) * BMT + (int)rank * BM, n0 = (r % kp.tiles_n) * bn + (int)rank * bnl;
         const bool split_k = g.k_rows_per_batch > 0;
         const int krow0 = split_k ? b * g.k_rows_per_batch : 0;
         for (int pass = 0; pass < g.npass && ok; ++pass) {
@@ -254,17 +233,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
                            &bars[B_FULL + s]);
               }
             }
-            if constexpr (QUAD) {
-              // this CTA's half of the B tile (128 rows) is also the half of the CTA with the same pair rank in the other
-              // pair: each of the two loads 64 of its rows and multicasts them to both (bn = 256 only)
-              const uint16_t mc = (uint16_t)((1u << rank) | (1u << (rank + 2u)));
-              if (!g.b_mn_major)
-                tma_load_3d_2sm_mc(dst + a_stage + pq * 8192u, &kp.tmB, g.b_off[pass] + kb * BK, n0 + 64 * (int)pq, g.b_batched ? b : 0,
-                                   &bars[B_FULL + s], mc);
-              else
-                tma_load_3d_2sm_mc(dst + a_stage + pq * 8192u, &kp.tmB, g.b_off[pass] + n0 + 64 * (int)pq, krow,
-                                   (g.b_batched && !split_k) ? b : 0, &bars[B_FULL + s], mc);
-            } else if (!g.b_mn_major) {
+            if (!g.b_mn_major) {
               tma_load(dst + a_stage, &kp.tmB, g.b_off[pass] + kb * BK, n0, g.b_batched ? b : 0, &bars[B_FULL + s]);
             } else if (g.group > 1) {
               for (int j = 0; j < bnl / 64; ++j)
@@ -284,7 +253,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
     // ------------------------------------------------------------------ MMA issuer (leader CTA of a pair)
     if (elect_one()) {
       const uint32_t ab_bf16 = g.ab_f16 ? 0u : 1u;   // one element type for both operands (launch() checks npass == 1)
-      const uint32_t id = make_idesc_16(BMP, (uint32_t)bn, ab_bf16, ab_bf16, g.a_mn_major ? 1u : 0u, g.b_mn_major ? 1u : 0u);
+      const uint32_t id = make_idesc_16(BMC, (uint32_t)bn, ab_bf16, ab_bf16, g.a_mn_major ? 1u : 0u, g.b_mn_major ? 1u : 0u);
       auto mma = [&](uint32_t d, uint32_t alo, uint32_t ahi, uint32_t blo, uint32_t bhi, uint32_t acc) {
         if constexpr (PAIR) mma_ss2_x(d, alo, ahi, blo, bhi, id, acc);
         else mma_ss_x(d, alo, ahi, blo, bhi, id, acc);
@@ -292,10 +261,6 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
       auto commit = [&](uint32_t bar_saddr) {          // to this pair
         if constexpr (PAIR) mma_commit2_a(bar_saddr, pair_mask);
         else mma_commit_a(bar_saddr);
-      };
-      auto commit_stage = [&](uint32_t bar_saddr) {    // "stage free": in a quad, to all four CTAs (both pairs refill each other)
-        if constexpr (QUAD) mma_commit2_a(bar_saddr, (uint16_t)0xF);
-        else commit(bar_saddr);
       };
       const uint32_t a_lbo = g.a_mn_major ? 8192u : 16u, a_kstep = g.a_mn_major ? 128u : 2u;
       constexpr uint32_t HI = desc_hi(1024, SWZ_128B);
@@ -327,7 +292,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
               for (int k4 = 0; k4 < 4; ++k4)
                 mma(tbase + 256u, alo1 + k4 * a_kstep, HI, blo + k4 * b_kstep, HI, (pass | kb | k4) ? 1u : 0u);
             }
-            commit_stage(bar0 + 8u * (B_EMPTY + s));
+            commit(bar0 + 8u * (B_EMPTY + s));
             s = s + 1 == nst ? 0 : s + 1;
             ph ^= (s == 0) ? 1u : 0u;
           }
@@ -518,7 +483,7 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const __grid_consta
       if (t >= ntiles) break;
       const int b = t / tiles_per_batch, r = t - b * tiles_per_batch;
       const int tn = r % kp.tiles_n;
-      const int m0 = (r / kp.tiles_n) * BMT + (tv % nu) * BMC + (int)pq * BMP + (int)rank * BM, n0 = tn * bn;
+      const int m0 = (r / kp.tiles_n) * BMT + (tv % nu) * BMC + (int)rank * BM, n0 = tn * bn;
       const uint32_t buf = i & 1;
       const int row = m0 + q * 32 + lane;
       const bool row_ok = row < g.M && (g.stat_rows == 0 || (long long)b * g.M + row < g.stat_rows);
@@ -776,36 +741,27 @@ int launch(const Gemm& g, cudaStream_t st) {
   const bool f16_out = g.out[0].mode == OUT_F16 || g.out[1].mode == OUT_F16;
   static bool attr_done = false;
   if (!attr_done) {
-    const void* fns[] = {(const void*)tc_gemm_kernel<0, EPI_FULL>, (const void*)tc_gemm_kernel<1, EPI_FULL>, (const void*)tc_gemm_kernel<2, EPI_FULL>,
-                         (const void*)tc_gemm_kernel<0, EPI_F16>, (const void*)tc_gemm_kernel<1, EPI_F16>,
-                         (const void*)tc_gemm_kernel<0, EPI_LEAN>, (const void*)tc_gemm_kernel<1, EPI_LEAN>,
-                         (const void*)tc_gemm_kernel<0, EPI_STAT>, (const void*)tc_gemm_kernel<1, EPI_STAT>,
-                         (const void*)tc_gemm_kernel<0, EPI_DIRECT>, (const void*)tc_gemm_kernel<1, EPI_DIRECT>,
-                         (const void*)tc_gemm_kernel<0, EPI_PSUM>, (const void*)tc_gemm_kernel<1, EPI_PSUM>,
-                         (const void*)tc_gemm_kernel<0, EPI_AUX>, (const void*)tc_gemm_kernel<1, EPI_AUX>};
+    const void* fns[] = {(const void*)tc_gemm_kernel<false, EPI_FULL>, (const void*)tc_gemm_kernel<true, EPI_FULL>,
+                         (const void*)tc_gemm_kernel<false, EPI_F16>, (const void*)tc_gemm_kernel<true, EPI_F16>,
+                         (const void*)tc_gemm_kernel<false, EPI_LEAN>, (const void*)tc_gemm_kernel<true, EPI_LEAN>,
+                         (const void*)tc_gemm_kernel<false, EPI_STAT>, (const void*)tc_gemm_kernel<true, EPI_STAT>,
+                         (const void*)tc_gemm_kernel<false, EPI_DIRECT>, (const void*)tc_gemm_kernel<true, EPI_DIRECT>,
+                         (const void*)tc_gemm_kernel<false, EPI_PSUM>, (const void*)tc_gemm_kernel<true, EPI_PSUM>,
+                         (const void*)tc_gemm_kernel<false, EPI_AUX>, (const void*)tc_gemm_kernel<true, EPI_AUX>};
     for (const void* f : fns)
       if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES) != cudaSuccess) return PASN_ERR_CUDA;
     attr_done = true;
   }
-  static const int pair_env = [] { const char* e = getenv("PASN_GEMM_PAIR"); return e ? atoi(e) : -1; }();   // A/B switch
   // pairs pay off when the main loop is long (big K: +10 % on square GEMMs, tools/bench_gemm.py), from 8 k-block passes per
   // tile.  (With the generic epilogue the K = 512 GEMMs of the chain lost 4 us of 64 to pairs -- the partner CTA's last rows
   // left 1.5-1.9 us after the leader's, tools/trace_gemm.py; with the lean epilogues pairs win there too: config 2 at
   // N = 1024 0.194 -> 0.187 ms, config 5 at N = 32 0.822 -> 0.806 ms.)
-  static const int pair_min = [] { const char* e = getenv("PASN_GEMM_PAIR_MIN"); return e ? atoi(e) : 8; }();
-  const bool pair = (pair_env >= 0 ? pair_env != 0 : (g.pair != 0 && ceil_div(g.K, BK) * g.npass >= pair_min)) && g.bn >= 128 && g.M > BM;
-  // two pairs per cluster sharing the B tile by multicast (full-width tiles, at least two pair tiles along M).  Correct (unit
-  // tests with PASN_GEMM_PAIR=1 PASN_GEMM_QUAD=1) but measured SLOWER than plain pairs -- 8192^3: 694 vs 1264 TFLOP/s, layer-1
-  // shape 602 vs 1005: the stage hand-back needs both pairs' commits and the 4-deep ring cannot cover the extra cluster
-  // round trip -- so it is opt-in only.
-  static const int quad_env = [] { const char* e = getenv("PASN_GEMM_QUAD"); return e ? atoi(e) : 0; }();
-  const bool quad = pair && quad_env != 0 && g.bn == 256 && g.M > 2 * BM && !f16_out;
-  const int cl = quad ? 4 : (pair ? 2 : 1);
+  const int kpasses = ceil_div(g.K, BK) * g.npass;
+  const bool pair = g.pair != 0 && kpasses >= 8 && g.bn >= 128 && g.M > BM;
+  const int cl = pair ? 2 : 1;
   // tall tiles for long main loops: two sub-tiles per CTA share every B stage (and take both accumulator buffers, so the
   // epilogue no longer overlaps the MMAs -- negligible when K is long): a quarter less L2 -> SM traffic per flop
-  static const int tall_env = [] { const char* e = getenv("PASN_GEMM_TALL"); return e ? atoi(e) : -1; }();
-  const bool tall = pair && !quad && g.M > cl * BM &&
-                    (tall_env >= 0 ? tall_env != 0 : ceil_div(g.K, BK) * g.npass >= 40);   // (24 k-block passes: 285 vs 267 us, slower)
+  const bool tall = pair && g.M > cl * BM && kpasses >= 40;   // (24 k-block passes: 285 vs 267 us, slower)
   int* fault = fault_word();   // bounded waits report into the host-mapped sticky fault word
   if (fault == nullptr) return PASN_ERR_CUDA;
   KParams kp;
@@ -814,8 +770,6 @@ int launch(const Gemm& g, cudaStream_t st) {
   kp.trace = nullptr;
   if (g_trace != nullptr && g_trace_slot < 64) kp.trace = g_trace + 64 * g_trace_slot++;   // debug: a row of stamps per launch
   kp.tall = tall ? 1 : 0;
-  static const int warm_env = [] { const char* e = getenv("PASN_GEMM_WARM"); return e ? atoi(e) : 1; }();
-  kp.warm = (warm_env != 0 && !quad) ? 1 : 0;
 
   kp.tiles_m = ceil_div(g.M, cl * BM * (tall ? 2 : 1));
   kp.tiles_n = ceil_div(g.N, g.bn);
@@ -842,7 +796,7 @@ int launch(const Gemm& g, cudaStream_t st) {
   }
   if (!g.b_mn_major) {
     if (!make_map(&kp.tmB, ab_dt, 2, g.B, (unsigned long long)g.kb,
-                  (unsigned long long)(g.b_rows ? g.b_rows : g.N), g.b_batched ? g.batch : 1, (unsigned long long)g.ldb * 2, (unsigned long long)g.b_bs * 2, BK, (unsigned)(quad ? 64 : (pair ? g.bn / 2 : g.bn))))
+                  (unsigned long long)(g.b_rows ? g.b_rows : g.N), g.b_batched ? g.batch : 1, (unsigned long long)g.ldb * 2, (unsigned long long)g.b_bs * 2, BK, (unsigned)(pair ? g.bn / 2 : g.bn)))
       return PASN_ERR_ALIGN;
   } else {   // [batch][K rows][kb columns], n contiguous: boxes of 64 n x 64 k
     if (!make_map(&kp.tmB, ab_dt, 2, g.B, (unsigned long long)g.kb,
@@ -875,8 +829,7 @@ int launch(const Gemm& g, cudaStream_t st) {
   }();
   const long long ntiles = (long long)g.batch * kp.tiles_m * kp.tiles_n;
   {
-    static const int pdl_env = [] { const char* e = getenv("PASN_GEMM_PDL"); return e ? atoi(e) : 1; }();
-    const int ncl = (int)(ntiles < num_sms / cl ? ntiles : num_sms / cl);   // clusters of 1, 2 (pair) or 4 (quad) CTAs
+    const int ncl = (int)(ntiles < num_sms / cl ? ntiles : num_sms / cl);   // clusters of 1 or 2 (pair) CTAs
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(cl * ncl); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = SMEM_BYTES; cfg.stream = st;
     cudaLaunchAttribute at[2];
@@ -886,14 +839,11 @@ int launch(const Gemm& g, cudaStream_t st) {
       at[na].val.clusterDim.x = cl; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
       ++na;
     }
-    if (pdl_env) {
-      at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      at[na].val.programmaticStreamSerializationAllowed = 1;
-      ++na;
-    }
+    at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
     cfg.attrs = at; cfg.numAttrs = na;
     // the leanest epilogue that can do what this launch asks for
-    static const int epi_env = [] { const char* e = getenv("PASN_GEMM_EPI"); return e ? atoi(e) : 1; }();   // 0: always the generic one
     int need = 0;
     for (int mi = 0; mi < 2; ++mi) {
       if (g.out[mi].mode == OUT_NONE) continue;
@@ -906,16 +856,14 @@ int launch(const Gemm& g, cudaStream_t st) {
     if (g.psum) need |= E_BIT_PSUM;
     if (g.rowstat) need |= E_BIT_STAT;
     // (EPI_AUX: fwd+bwd of 256 clips 1.09-1.10 -> 1.06-1.07 ms; at 64 clips the step is launch-bound and moves with the box)
-    static const int aux_env = [] { const char* e = getenv("PASN_GEMM_EPI_AUX"); return e ? atoi(e) : 1; }();
     static const int variants[] = {EPI_LEAN, EPI_STAT, EPI_DIRECT, EPI_PSUM, EPI_AUX};
     int epi = f16_out ? EPI_F16 : EPI_FULL;   // (fp16 outputs: the fp16 chain's occurrence-map stores only)
-    if (epi_env && !quad && !f16_out)
+    if (!f16_out)
       for (int v : variants)
-        if ((v & need) == need && (v != EPI_AUX || aux_env)) { epi = v; break; }
+        if ((v & need) == need) { epi = v; break; }
     cudaError_t e;
-#define TCG_LAUNCH(EPI_) (pair ? cudaLaunchKernelEx(&cfg, tc_gemm_kernel<1, EPI_>, kp) : cudaLaunchKernelEx(&cfg, tc_gemm_kernel<0, EPI_>, kp))
-    if (quad) e = cudaLaunchKernelEx(&cfg, tc_gemm_kernel<2, EPI_FULL>, kp);
-    else if (epi == EPI_LEAN) e = TCG_LAUNCH(EPI_LEAN);
+#define TCG_LAUNCH(EPI_) (pair ? cudaLaunchKernelEx(&cfg, tc_gemm_kernel<true, EPI_>, kp) : cudaLaunchKernelEx(&cfg, tc_gemm_kernel<false, EPI_>, kp))
+    if (epi == EPI_LEAN) e = TCG_LAUNCH(EPI_LEAN);
     else if (epi == EPI_STAT) e = TCG_LAUNCH(EPI_STAT);
     else if (epi == EPI_DIRECT) e = TCG_LAUNCH(EPI_DIRECT);
     else if (epi == EPI_PSUM) e = TCG_LAUNCH(EPI_PSUM);

@@ -323,14 +323,11 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   float* FE = feats ? feats + (size_t)n0 * P * D : reinterpret_cast<float*>(ws + p.off_fe);
   // Plain forward (nobody asked for features_extracted, no push): the GEMM that would write the pooled features leaves the
   // two reductions the prototype stage needs (||f||^2, <f, v_p>) instead -- the features are neither stored nor read back.
-  static const int stats_env = [] { const char* e = getenv("PASN_TILED_STATS"); return e ? atoi(e) : 1; }();
-  // Used where it pays (1, default): many prototypes (config 5: 8 MB of features per clip), and the per-clip pooling GEMM of
-  // few prototypes straight into features (image head: the GEMM keeps the prototype slices in shared memory).  Elsewhere the
-  // statistics' vector reads (a row per lane) cost the epilogue more than the round trip.  2: always, 0: never.
-  // (Both are W2-before-pooling shapes: the statistics ride in the per-clip pooling GEMM.  The other order's last GEMM can
-  // leave them too -- PASN_TILED_STATS=2 -- but no named config takes that way, so it is not on by default.)
-  const bool fuse_stats = (stats_env == 2 || (stats_env == 1 && p.w2_first && (P >= 1024 || P <= 64))) && !occ_only &&
-                          feats == nullptr && push == nullptr;
+  // Used where it pays: many prototypes (config 5: 8 MB of features per clip), and the per-clip pooling GEMM of few
+  // prototypes straight into features (image head: the GEMM keeps the prototype slices in shared memory).  Elsewhere the
+  // statistics' vector reads (a row per lane) cost the epilogue more than the round trip.  (Both are W2-before-pooling
+  // shapes: the statistics ride in the per-clip pooling GEMM.)
+  const bool fuse_stats = p.w2_first && (P >= 1024 || P <= 64) && !occ_only && feats == nullptr && push == nullptr;
   float* STAT = reinterpret_cast<float*>(ws + p.off_stat);
   int stat_parts = 2 * ceil_div(D, D >= 256 ? 256 : 128);   // column half-tiles of the GEMM that leaves the statistics
   const __nv_bfloat16* W13 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w13);
@@ -378,8 +375,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   long long pool_lda = 0;
   // W2-after-pooling order: the row sums over s then come from a small column-sum kernel below.  (fp32 maps keep the
   // per-clip form there: their map leaves as 4-byte plain stores, which measured slower than the TMA rows -- 0.72 vs 0.64 ms)
-  static const int tokc_all = [] { const char* e = getenv("PASN_TOKC_ALL"); return e ? atoi(e) : 0; }();
-  const bool tok_c = p.tok_c && (occ_only || p.w2_first || ex == 1 || tokc_all);
+  const bool tok_c = p.tok_c && (occ_only || p.w2_first || ex == 1);
   if (tok_c) {
     // few prototypes: O^T = |G2 W5^T| over all tokens in one GEMM (rows = tokens, N = P).  The occurrence map leaves
     // channel-major per clip through plain stores that are coalesced along the voxels; the token-major copy
@@ -468,9 +464,8 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
         g.rowstat = STAT; g.dotvec = w.prototypes; g.dot_ld = D; g.dot_mod = P; g.dot_early = 1;   // (parameters: the chain does not write them)
         // few prototypes, few voxels (image head: 40 x 49): three clips share a 128-row tile, block-diagonally -- a clip alone
         // uses 40 of the tile's rows and two of the four epilogue row groups
-        static const int group_env = [] { const char* e = getenv("PASN_POOL_GROUP"); return e ? atoi(e) : 1; }();
         const int G = 128 / P < 4 ? 128 / P : 4;
-        if (group_env && tok_c && ex == 1 && S <= 64 && G >= 2 && nb >= 2 * G) {
+        if (tok_c && ex == 1 && S <= 64 && G >= 2 && nb >= 2 * G) {
           g.group = G; g.group_rows = P; g.group_items = nb;
           g.M = G * P; g.batch = ceil_div(nb, G); g.bn = 128;
           g.stat_rows = (long long)nb * P;
@@ -508,10 +503,6 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.rowparts = PSUM; g.nparts = tok_c ? 1 : 2 * p.tiles_n_c; g.colvec = b2;
     g.act = tcg::ACT_NONE;
     g.out[0] = {FE, tcg::OUT_F32, (long long)D, 0, 0};
-    if (fuse_stats) {
-      g.out[0].mode = tcg::OUT_NONE;
-      g.rowstat = STAT; g.dotvec = w.prototypes; g.dot_ld = D; g.dot_mod = P; g.dot_early = 1;   // (parameters: the chain does not write them)
-    }
     if ((rc = tcg::launch(g, st))) return rc;
   }
   }

@@ -1,4 +1,4 @@
-"""Time the fused head (K1 main-kernel events + whole step) at N=1024; PASN_DBG_SKIP experiments use garbage data."""
+"""Time the fused head (K1 main-kernel events + whole step) at N=1024."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -21,4 +21,4 @@ with torch.no_grad():
     ks = []
     for _ in range(10):
         m(x); ks.append(lib.pasn_debug_last_main_kernel_ms())
-print(f"skip={os.environ.get('PASN_DBG_SKIP','0')} {sys.argv[1:]} step {e0.elapsed_time(e1)/10*1e3:.1f} us, K1 {np.mean(ks)*1e3:.1f} us")
+print(f"{sys.argv[1:]} step {e0.elapsed_time(e1)/10*1e3:.1f} us, K1 {np.mean(ks)*1e3:.1f} us")

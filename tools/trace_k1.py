@@ -20,23 +20,13 @@ with torch.no_grad():
     lib.pasn_debug_set_trace(None)
 t = buf.cpu()[:768].view(3, 16, 16)
 t0 = int(t[0, 0, 0])
-if os.environ.get("PASN_K1_PHASES", "2") == "0":   # first-generation kernel
-    names_m = ["start", "tmemfree", "L1issued", "g1ready", "G2issued", "g2ready", "Oissued", "osready", "hs0", "hs1", "poolissued"]
-    names_e = ["E-start", "l1done", "E1done", "E2a done", "g2done", "E3done", "odone+osempty", "E4done", "E2b done", "fedone", "E5done"]
-else:                                              # two-phase kernel (head_sm100_k1.cu)
-    names_m = ["start", "gbfree", "Gissued", "abfree", "G2issued", "Oissued", "Aissued", "pool0", "pool1", "g1ready_seen", "w4a_seen"]
-    names_e = ["E-start", "gdone", "E1done", "g2done", "E3done", "odone", "E4done", "adone", "E2done", "fedone", "E5done"]
+names_m = ["start", "gbfree", "Gissued", "abfree", "G2issued", "Oissued", "Aissued", "pool0", "pool1", "g1ready_seen", "w4a_seen"]
+names_e = ["E-start", "gdone", "E1done", "g2done", "E3done", "odone", "E4done", "adone", "E2done", "fedone", "E5done"]
 for tile in range(12):
     if int(t[0, tile, 0]) == 0:
         break
     print(f"tile {tile}")
     print("  MMA: " + " ".join(f"{n}={int(t[0, tile, i]) - t0}" for i, n in enumerate(names_m)))
-    print(f"  MMA thread blocked on x_full {int(t[0, tile, 11])} cyc, w_full {int(t[0, tile, 12])} cyc (of which G phase: {int(t[0, tile, 13])}, {int(t[0, tile, 14])})")
-    print("  chunk durations G:", [int(v) for v in t[2, tile, :8]], " A:", [int(v) for v in t[2, tile, 8:16]])
+    print(f"  MMA thread blocked on x_full {int(t[0, tile, 11])} cyc, w_full {int(t[0, tile, 12])} cyc")
+    print("  chunk durations (G + A blocks):", [int(v) for v in t[2, tile, :8]])
     print("  EPI: " + " ".join(f"{n}={int(t[1, tile, i]) - t0}" for i, n in enumerate(names_e)))
-
-if os.environ.get("PASN_K1_PHASES", "2") != "0":
-    print("A phase of tile 3, per chunk: [chunk start, +wait_x, +wait_w and 8 MMAs issued and W commit, +X commit] relative to chunk 0 start")
-    b = int(t[2, 8, 0])
-    for kc in range(8):
-        print("  kc", kc, [int(t[2, 8 + kc, i]) - b for i in (0, 1, 3, 4)])

@@ -28,5 +28,4 @@ for it in range(20):
     b = g[16 + it * 8: 16 + it * 8 + 8]
     if not b[0]:
         break
-    print(f"  it {it} tile {t[200 + it]}: ready-wait passed {rel(b[7])}, stage full seen {[rel(v) for v in b[:4]]}, MMAs committed {rel(b[4])}, epilogue start {rel(b[5])}, end {rel(b[6])}")
-print("first queue grabs of CTA 0 (time ns, slot):", [(rel(t[240 + 2 * j]), t[240 + 2 * j + 1]) for j in range(4)])
+    print(f"  it {it} tile {t[200 + it]}: tile taken {rel(b[7])}, stage full seen {[rel(v) for v in b[:4]]}, MMAs committed {rel(b[4])}, epilogue start {rel(b[5])}, end {rel(b[6])}")
