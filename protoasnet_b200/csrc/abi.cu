@@ -116,7 +116,8 @@ extern "C" int pasn_occurrence_lnorm(const void* occ, int32_t dtype, int64_t row
 // fp16 feature maps: tensor-core backward only
 static bool backward_ok(const pasn_dims* d) { return dims_ok(d) && (d->dtype != PASN_F16 || tiled_backward_supported(*d)); }
 extern "C" size_t pasn_head_backward_workspace_bytes(const pasn_dims* dims) {
-  return backward_ok(dims) ? backward_workspace_bytes(*dims) : 0;
+  if (!backward_ok(dims)) return 0;
+  return tiled_backward_supported(*dims) ? tiled_backward_workspace_bytes(*dims) : generic_backward_workspace_bytes(*dims);
 }
 extern "C" int pasn_head_backward(const void* feat, const pasn_weights* w, const pasn_dims* dims, const float* grad_logits,
                                   const float* grad_similarity, const float* grad_occurrence, const pasn_grads* grads,
@@ -129,8 +130,9 @@ extern "C" int pasn_head_backward(const void* feat, const pasn_weights* w, const
   const float* const* gp = reinterpret_cast<const float* const*>(grads);
   for (int i = 0; i < 11; ++i)
     if (!gp[i]) return PASN_ERR_INVALID;
-  return head_backward(feat, *w, *dims, grad_logits, grad_similarity, grad_occurrence, *grads, grad_feat, workspace,
-                       workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  auto backward = tiled_backward_supported(*dims) ? tiled_head_backward : generic_head_backward;
+  return backward(feat, *w, *dims, grad_logits, grad_similarity, grad_occurrence, *grads, grad_feat, workspace,
+                  workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int pasn_debug_sm100_error(const void* workspace, const pasn_dims* dims, void* stream) {

@@ -95,14 +95,15 @@ int launch_sim_stats(const float* sim, const int64_t* labels, int N, int P, int 
                      int top_b, float* class_max, int32_t* class_arg, double* sums, unsigned long long* counts, double* simsum,
                      cudaStream_t st);
 int launch_occ_lnorm(const void* occ, int dtype, long long rows, int S, int p, double* sums, float* row_norm, cudaStream_t st);
-size_t backward_workspace_bytes(const pasn_dims& d);
-int head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
-                  const float* gOcc, const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
 int generic_head_forward(const void* feat, const pasn_weights& w, const pasn_dims& d, float* logits, float* sim,
                          void* occ, float* feats, float* dist, const pasn_push_args* push, void* ws, size_t ws_bytes,
                          cudaStream_t st);
 int generic_occurrence_only(const void* feat, const pasn_weights& w, const pasn_dims& d, void* occ, void* ws,
                             size_t ws_bytes, cudaStream_t st);
+// backward on the CUDA cores: fp32 / bf16 feature maps, any shape; the shapes tiled_backward_supported() rejects
+size_t generic_backward_workspace_bytes(const pasn_dims& d);
+int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
+                          const float* gOcc, const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // ---- prototype stage (proto_stage.cu): cosine -> (.+1)/2 -> logits -> 1-s -> running argmin keys ----
 int launch_proto_stage(const float* feats /*[N,P,D]*/, const float* protos, const float* last_layer, int N, int P,

@@ -40,6 +40,17 @@ struct Plan {
 
 inline int pick_bn(int n) { return n <= 64 ? 64 : (n <= 128 ? 128 : 256); }
 
+// clips per chunk of the forward / backward chain: as many as `budget` bytes of scratch hold at per_clip bytes each, at
+// least one, at most N.  PASN_TILED_CHUNK lowers the cap (tests force chunking with it).
+int clips_per_chunk(const pasn_dims& d, size_t budget, size_t per_clip) {
+  static const int chunk_env = [] { const char* e = getenv("PASN_TILED_CHUNK"); return e ? atoi(e) : 0; }();
+  long long nb = (long long)(budget / per_clip);
+  if (chunk_env > 0 && nb > chunk_env) nb = chunk_env;
+  if (nb < 1) nb = 1;
+  if (nb > d.N) nb = d.N > 0 ? d.N : 1;
+  return (int)nb;
+}
+
 Plan make_plan(const pasn_dims& d) {
   Plan p{};
   p.ex = d.dtype == PASN_F32 ? 2 : 1;
@@ -58,12 +69,7 @@ Plan make_plan(const pasn_dims& d) {
   const size_t per_clip = S * ex * d.C * 2 + S * ex * 2 * d.D * 2 + S * ex * p.D2 * 2 + occ_elems * ex * 2 +
                           (size_t)d.P * 2 * p.tiles_n_c * 4 + (size_t)d.P * 2 * d.D * 2 + S * ex * d.D * 2 +
                           (size_t)d.P * d.D * 4 + 2048;
-  long long nb = (long long)(((size_t)2 << 30) / per_clip);
-  static const int chunk_env = [] { const char* e = getenv("PASN_TILED_CHUNK"); return e ? atoi(e) : 0; }();   // tests: force chunking
-  if (chunk_env > 0 && nb > chunk_env) nb = chunk_env;
-  if (nb < 1) nb = 1;
-  if (nb > d.N) nb = d.N > 0 ? d.N : 1;
-  p.nb = (int)nb;
+  p.nb = clips_per_chunk(d, (size_t)2 << 30, per_clip);
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t r = o; o += align_up(bytes, 1024); return r; };
   p.off_xt = take((size_t)p.nb * S * ex * d.C * 2);
@@ -209,16 +215,66 @@ __global__ void __launch_bounds__(256) clip_colsum_kernel(const __nv_bfloat16* _
   }
 }
 
-// passes of a product of two operands that each come as planes (hi at column 0, lo at column *_lo)
-void set_passes(tcg::Gemm& g, int ex, int a_lo, int b_lo) {
+// passes of a product of two operands that each come as planes (hi at column 0, lo at column *_lo); an operand without a
+// lo plane (bf16 mode, or a bf16-exact feature map) drops its pass.  Both split: hi*hi, hi*lo, lo*hi.  The lo*lo term is
+// below the representation error of the split itself (each operand keeps 16 significant bits: |x - xh - xl| <= 2^-17 |x|,
+// and |xl wl| <= 2^-18 |x w|), so it is not computed.
+void set_passes(tcg::Gemm& g, int a_lo, int b_lo, bool a_has_lo = true, bool b_has_lo = true) {
   g.pair = 1;   // CTA pairs wherever the shape allows (tc_gemm.cu decides)
   for (int q = 0; q < 4; ++q) g.a_off[q] = g.b_off[q] = 0;
-  if (ex == 1) { g.npass = 1; return; }
-  // hi*hi, hi*lo, lo*hi.  The lo*lo term is below the representation error of the split itself (each operand keeps 16
-  // significant bits: |x - xh - xl| <= 2^-17 |x|, and |xl wl| <= 2^-18 |x w|), so it is not computed.
-  g.npass = 3;
-  g.b_off[1] = b_lo;
-  g.a_off[2] = a_lo;
+  int n = 1;
+  if (b_has_lo) { g.b_off[n] = b_lo; ++n; }
+  if (a_has_lo) { g.a_off[n] = a_lo; ++n; }
+  g.npass = n;
+}
+
+// The first layer's A operand for nb clips of the feature map at x: token-major planes XT[(n*S + s)][planes*C] in dst, either
+// bf16 hi | lo (hilo: fp32 and fp16 maps) or one plane in the map's own type (bf16 and fp16 maps) -- or, for one plane, the
+// map itself where it already is such an operand:
+//   channels_last: token-major as it lies;
+//   NCDHW with 16-byte aligned channel rows, when direct is non-null: [C][S] per clip IS the MN-major form of the operand
+//   (voxels contiguous), which the TMA unit tiles straight out of the caller's buffer (*direct = true: one GEMM per clip).
+int token_operand(const char* x, const pasn_dims& d, int nb, bool hilo, __nv_bfloat16* dst, const __nv_bfloat16** xt,
+                  bool* direct, cudaStream_t st) {
+  const int C = d.C, S = d.S;
+  const bool aligned = ((uintptr_t)x & 15) == 0;
+  if (direct) *direct = false;
+  *xt = reinterpret_cast<const __nv_bfloat16*>(x);
+  if (!hilo && d.layout == PASN_LAYOUT_NSC) return aligned ? PASN_OK : PASN_ERR_ALIGN;
+  if (!hilo && direct && (S * 2) % 16 == 0 && aligned) {
+    *direct = true;
+    return PASN_OK;
+  }
+  *xt = dst;
+  if (d.layout == PASN_LAYOUT_NSC) {
+    const long long T = (long long)nb * S;
+    if (d.dtype == PASN_F16) to_tokens_nsc_split_kernel<__half><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const __half*>(x), T, C, dst);
+    else to_tokens_nsc_split_kernel<float><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, dst);
+  } else {
+    const dim3 grid(ceil_div(S, 32), ceil_div(C, 64), nb);
+    const size_t clip_bytes = (size_t)C * S * 2;
+    if (!hilo && S < 128 && clip_bytes <= 96 * 1024 && clip_bytes % 16 == 0 && aligned) {
+      static bool attr_done = false;
+      if (!attr_done) {
+        if (cudaFuncSetAttribute(to_tokens_small_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024) != cudaSuccess)
+          return PASN_ERR_CUDA;
+        attr_done = true;
+      }
+      to_tokens_small_bf16_kernel<<<nb, 256, clip_bytes, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, dst);
+    } else if (hilo && d.dtype == PASN_F16) {
+      to_tokens_ncs_kernel<__half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 2, dst);
+    } else if (hilo) {
+      to_tokens_ncs_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(x), C, S, 2, dst);
+    } else if (d.dtype == PASN_F16) {
+      to_tokens_ncs_kernel<__half, __half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 1,
+                                                                 reinterpret_cast<__half*>(dst));
+    } else {
+      to_tokens_ncs_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, 1, dst);
+    }
+  }
+  PASN_LAUNCH_CHECK();
+  count_launch();
+  return PASN_OK;
 }
 
 }  // namespace
@@ -274,47 +330,14 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   const long long T = (long long)nb * S;
   const size_t elt = dtype_bytes(d.dtype);
   const bool f16 = d.dtype == PASN_F16;   // layer 1 fp16 x fp16, the map stored in fp16; everything else as bf16 mode
+  const bool hilo = ex == 2;
   int rc;
 
   // ---- tokens
   const __nv_bfloat16* xt;
+  bool x_direct;
   const char* x = reinterpret_cast<const char*>(feat) + (size_t)n0 * C * S * elt;
-  // bf16 / fp16 NCDHW feature maps with 16-byte aligned channel rows need no transposition: [C][S] per clip IS the MN-major form
-  // of the A operand (voxels contiguous), which the TMA unit tiles straight out of the caller's buffer
-  const bool x_direct = d.layout == PASN_LAYOUT_NCS && ex == 1 && (S * 2) % 16 == 0 && ((uintptr_t)x & 15) == 0;
-  if (d.layout == PASN_LAYOUT_NSC && ex == 1) {
-    xt = reinterpret_cast<const __nv_bfloat16*>(x);   // channels_last bf16 / fp16 feature map: already token-major
-    if (((uintptr_t)xt & 15) != 0) return PASN_ERR_ALIGN;
-  } else if (x_direct) {
-    xt = reinterpret_cast<const __nv_bfloat16*>(x);
-  } else {
-    __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(ws + p.off_xt);
-    if (d.layout == PASN_LAYOUT_NSC) {
-      to_tokens_nsc_split_kernel<float><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, dst);
-    } else {
-      dim3 grid(ceil_div(S, 32), ceil_div(C, 64), nb);
-      const size_t clip_bytes = (size_t)C * S * 2;
-      if (ex == 1 && S < 128 && clip_bytes <= 96 * 1024 && clip_bytes % 16 == 0 && ((uintptr_t)x & 15) == 0) {
-        static bool attr_done = false;
-        if (!attr_done) {
-          if (cudaFuncSetAttribute(to_tokens_small_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024) != cudaSuccess)
-            return PASN_ERR_CUDA;
-          attr_done = true;
-        }
-        to_tokens_small_bf16_kernel<<<nb, 256, clip_bytes, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, dst);
-      } else if (f16) {
-        to_tokens_ncs_kernel<__half, __half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 1,
-                                                                   reinterpret_cast<__half*>(dst));
-      } else if (ex == 1) {
-        to_tokens_ncs_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, ex, dst);
-      } else {
-        to_tokens_ncs_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(x), C, S, ex, dst);
-      }
-    }
-    PASN_LAUNCH_CHECK();
-    count_launch();
-    xt = dst;
-  }
+  if ((rc = token_operand(x, d, nb, hilo, reinterpret_cast<__nv_bfloat16*>(ws + p.off_xt), &xt, &x_direct, st))) return rc;
   __nv_bfloat16* Y = reinterpret_cast<__nv_bfloat16*>(ws + p.off_y);
   __nv_bfloat16* G2 = reinterpret_cast<__nv_bfloat16*>(ws + p.off_g2);
   __nv_bfloat16* OCC = reinterpret_cast<__nv_bfloat16*>(ws + p.off_occ);
@@ -345,7 +368,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.A = xt; g.lda = (long long)ex * C; g.a_bs = 0; g.a_batched = 0; g.ka = ex * C;
     g.B = occ_only ? W13 + (size_t)D * ex * C : W13; g.ldb = (long long)ex * C; g.b_bs = 0; g.b_batched = 0; g.kb = ex * C;
     g.M = (int)T; g.N = nA; g.K = C; g.batch = 1; g.bn = 256;
-    set_passes(g, ex, C, C);
+    set_passes(g, C, C, hilo, hilo);
     g.bias = occ_only ? b13 + D : b13; g.act = tcg::ACT_RELU;
     g.ab_f16 = f16 ? 1 : 0;   // X and [W1; W3] both fp16 (pack: tiled_pack_weights)
     g.out[0] = {Y, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * nA, 0, nA};
@@ -363,7 +386,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.A = Y + g1_off; g.lda = (long long)ex * nA; g.a_batched = 0; g.ka = ex * nA - g1_off;
     g.B = W4; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
     g.M = (int)T; g.N = D2; g.K = D; g.batch = 1; g.bn = pick_bn(D2);
-    set_passes(g, ex, nA, D);
+    set_passes(g, nA, D, hilo, hilo);
     g.bias = b4; g.act = tcg::ACT_RELU;
     g.out[0] = {G2, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * D2, 0, D2};
     if ((rc = tcg::launch(g, st))) return rc;
@@ -384,7 +407,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.A = G2; g.lda = (long long)ex * D2; g.a_batched = 0; g.ka = ex * D2;
     g.B = W5; g.ldb = (long long)ex * D2; g.b_batched = 0; g.kb = ex * D2;
     g.M = (int)T; g.N = P; g.K = D2; g.batch = 1; g.bn = 64;
-    set_passes(g, ex, D2, D2);
+    set_passes(g, D2, D2, hilo, hilo);
     g.act = tcg::ACT_ABS;
     int no = 0;
     if (occ_user != nullptr) {
@@ -410,7 +433,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.b_rows = S;   // tokens of this clip; the padded columns of the operand copy come out as exact zeros
     g.M = P; g.K = D2; g.batch = nb; g.bn = p.bn_c;
     g.N = ex == 2 ? p.Sp : S;
-    set_passes(g, ex, D2, D2);
+    set_passes(g, D2, D2, hilo, hilo);
     g.act = tcg::ACT_ABS;
     int no = 0;
     const bool need_copy = !occ_only && !(p.occ_direct && occ_user != nullptr);
@@ -440,7 +463,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
       g.A = Y; g.lda = (long long)ex * 2 * D; g.a_batched = 0; g.ka = ex * 2 * D;
       g.B = W2; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
       g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, ex, 2 * D, D);
+      set_passes(g, 2 * D, D, hilo, hilo);
       g.bias = b2; g.act = tcg::ACT_NONE;
       g.out[0] = {F, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * D, 0, D};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -452,10 +475,10 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
       g.B = F; g.ldb = (long long)ex * D; g.b_bs = (long long)S * ex * D; g.b_batched = 1; g.kb = ex * D;
       g.b_mn_major = 1; g.b_rows = S;
       g.M = P; g.N = D; g.K = ex == 2 ? p.Sp : S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, ex, p.Sp, D);
+      set_passes(g, p.Sp, D, hilo, hilo);
       if (tok_c) {   // occurrence values token-major: [S rows][P] per clip, prototypes contiguous (MN-major A)
         g.a_mn_major = 1; g.a_bs = (long long)S * pool_lda; g.ka = ex * p.Pp; g.a_rows = S; g.K = S;
-        set_passes(g, ex, p.Pp, D);
+        set_passes(g, p.Pp, D, hilo, hilo);
       }
       g.act = tcg::ACT_NONE;
       g.out[0] = {FE, tcg::OUT_F32, (long long)D, (long long)P * D, 0};
@@ -483,10 +506,10 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.B = Y; g.ldb = (long long)ex * 2 * D; g.b_bs = (long long)S * ex * 2 * D; g.b_batched = 1; g.kb = ex * 2 * D;
     g.b_mn_major = 1; g.b_rows = S;
     g.M = P; g.N = D; g.K = ex == 2 ? p.Sp : S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-    set_passes(g, ex, p.Sp, 2 * D);
+    set_passes(g, p.Sp, 2 * D, hilo, hilo);
     if (tok_c) {   // occurrence values token-major: [S rows][P] per clip (MN-major A)
       g.a_mn_major = 1; g.a_bs = (long long)S * pool_lda; g.ka = ex * p.Pp; g.a_rows = S; g.K = S;
-      set_passes(g, ex, p.Pp, 2 * D);
+      set_passes(g, p.Pp, 2 * D, hilo, hilo);
     }
     g.act = tcg::ACT_NONE;
     g.out[0] = {POOL, tcg::OUT_BF16_HILO, (long long)2 * D, (long long)P * 2 * D, D};
@@ -498,8 +521,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
     g.A = POOL; g.lda = 2 * D; g.a_batched = 0; g.ka = 2 * D;
     g.B = W2; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
     g.M = nb * P; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-    set_passes(g, ex, D, D);
-    if (ex == 1) { g.npass = 2; g.a_off[1] = D; }   // pooled = hi + lo planes, W2 bf16
+    set_passes(g, D, D, true, hilo);   // pooled = hi + lo planes in both modes
     g.rowparts = PSUM; g.nparts = tok_c ? 1 : 2 * p.tiles_n_c; g.colvec = b2;
     g.act = tcg::ACT_NONE;
     g.out[0] = {FE, tcg::OUT_F32, (long long)D, 0, 0};
@@ -555,7 +577,7 @@ int tiled_occurrence_only(const void* feat, const pasn_weights& w, const void* p
 // Backward of the head on the tensor cores (SURVEY.md section 8(f) row 2; reference: loss.backward() through
 // Video_XProtoNet.forward, src/agents/XProtoNet_Base.py:397, src/models/Video_XProtoNet.py:82-98).
 //
-// Every contraction of the fp32 gradient (backward.cu documents the math and the sub-gradient conventions) runs as a
+// Every contraction of the fp32 gradient (generic.cu documents the math and the sub-gradient conventions) runs as a
 // three-pass bf16 hi/lo GEMM of tc_gemm.cu over token-major planes, i.e. fp32-grade products with fp32 accumulation:
 //   recomputed forward   XT -> [H1|G1] -> G2 -> Opre (sign carrier + |.| planes) ; F = W2 H1 + b2 ; FE = O^T F
 //   prototype stage      gFE, gV, gWl                                     (two small CUDA-core kernels)
@@ -600,12 +622,7 @@ BPlan make_bplan(const pasn_dims& d) {
   // fp32 partials of the largest weight gradient at full machine width
   const size_t m13 = (size_t)2 * d.D * d.C, m2 = (size_t)d.D * d.D;
   b.part_bytes = align_up((m13 > m2 ? m13 : m2) * 4 * 80, 1024);
-  long long nb = (long long)(((size_t)1500 << 20) / per_clip);
-  static const int chunk_env = [] { const char* e = getenv("PASN_TILED_CHUNK"); return e ? atoi(e) : 0; }();
-  if (chunk_env > 0 && nb > chunk_env) nb = chunk_env;
-  if (nb < 1) nb = 1;
-  if (nb > d.N) nb = d.N > 0 ? d.N : 1;
-  b.nb = (int)nb;
+  b.nb = clips_per_chunk(d, (size_t)1500 << 20, per_clip);
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t r = o; o += align_up(bytes, 1024); return r; };
   const size_t T = (size_t)b.nb * S;
@@ -626,16 +643,6 @@ BPlan make_bplan(const pasn_dims& d) {
   b.off_part = take(b.part_bytes);
   b.total = o + 256;
   return b;
-}
-
-// three-pass product of two plane pairs; an operand without a lo plane (bf16-exact feature map) drops its pass
-void set_passes_b(tcg::Gemm& g, int a_lo, int b_lo, bool a_has_lo = true, bool b_has_lo = true) {
-  g.pair = 1;
-  for (int q = 0; q < 4; ++q) g.a_off[q] = g.b_off[q] = 0;
-  int n = 1;
-  if (b_has_lo) { g.b_off[n] = b_lo; ++n; }
-  if (a_has_lo) { g.a_off[n] = a_lo; ++n; }
-  g.npass = n;
 }
 
 // prototype stage backward, part 1: one warp per (clip, prototype) row.
@@ -833,7 +840,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     g.A = A; g.lda = lda; g.ka = (int)lda; g.a_mn_major = 1; g.a_rows = (int)T;
     g.B = B; g.ldb = ldb; g.kb = (int)ldb; g.b_mn_major = 1; g.b_rows = (int)T;
     g.M = M; g.N = N; g.K = kper; g.batch = parts; g.k_rows_per_batch = kper; g.bn = bn;
-    set_passes_b(g, a_lo, b_lo, true, b_has_lo);
+    set_passes(g, a_lo, b_lo, true, b_has_lo);
     g.out[0] = {PART, tcg::OUT_F32, (long long)N, (long long)M * N, 0, 0, 0, 0};
     int r = tcg::launch(g, st);
     if (r) return r;
@@ -856,22 +863,8 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     const long long T = (long long)nb * S;
     const char* x = reinterpret_cast<const char*>(feat) + (size_t)n0 * C * S * elt;
     // ---- token-major feature planes
-    const __nv_bfloat16* xt = XT;
-    if (d.layout == PASN_LAYOUT_NSC && xe == 1) {
-      xt = reinterpret_cast<const __nv_bfloat16*>(x);
-      if (((uintptr_t)xt & 15) != 0) return PASN_ERR_ALIGN;
-    } else if (d.layout == PASN_LAYOUT_NSC) {
-      if (d.dtype == PASN_F16) to_tokens_nsc_split_kernel<__half><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const __half*>(x), T, C, XT);
-      else to_tokens_nsc_split_kernel<float><<<148 * 8, 256, 0, st>>>(reinterpret_cast<const float*>(x), T, C, XT);
-      count_launch();
-    } else {
-      dim3 grid(ceil_div(S, 32), ceil_div(C, 64), nb);
-      if (xe == 1) to_tokens_ncs_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(x), C, S, 1, XT);
-      else if (d.dtype == PASN_F16) to_tokens_ncs_kernel<__half><<<grid, 256, 0, st>>>(reinterpret_cast<const __half*>(x), C, S, 2, XT);
-      else to_tokens_ncs_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(x), C, S, 2, XT);
-      count_launch();
-    }
-    PASN_LAUNCH_CHECK();
+    const __nv_bfloat16* xt;
+    if ((rc = token_operand(x, d, nb, x_lo, XT, &xt, nullptr, st))) return rc;
     const long long ldx = (long long)xe * C;
 
     // ================= forward, recomputed
@@ -880,7 +873,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = xt; g.lda = ldx; g.ka = (int)ldx;
       g.B = W13; g.ldb = 2 * C; g.kb = 2 * C;
       g.M = (int)T; g.N = 2 * D; g.K = C; g.batch = 1; g.bn = 256;
-      set_passes_b(g, C, C, x_lo, true);
+      set_passes(g, C, C, x_lo, true);
       g.bias = b13; g.act = tcg::ACT_RELU;
       g.out[0] = {Y, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, 0, 0, 0};
       if (occ_only) {   // G1 alone, into its usual columns [D, 2D) of the planes
@@ -894,7 +887,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = Y + D; g.lda = 4 * D; g.ka = 4 * D - D;
       g.B = W4; g.ldb = 2 * D; g.kb = 2 * D;
       g.M = (int)T; g.N = D2; g.K = D; g.batch = 1; g.bn = pick_bn(D2);
-      set_passes_b(g, 2 * D, D);
+      set_passes(g, 2 * D, D);
       g.bias = b4; g.act = tcg::ACT_RELU;
       g.out[0] = {G2, tcg::OUT_BF16_HILO, (long long)2 * D2, 0, D2, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -904,7 +897,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = G2; g.lda = 2 * D2; g.ka = 2 * D2;
       g.B = W5; g.ldb = 2 * D2; g.kb = 2 * D2;
       g.M = (int)T; g.N = P; g.K = D2; g.batch = 1; g.bn = pick_bn(P);
-      set_passes_b(g, D2, D2);
+      set_passes(g, D2, D2);
       g.act = tcg::ACT_NONE;
       g.out[0] = {OS, tcg::OUT_BF16, (long long)Pp, 0, 0, Pp, 0, 0};
       if (!occ_only) g.out[1] = {OA, tcg::OUT_BF16_HILO, (long long)2 * Pp, 0, Pp, Pp, 1, 0};
@@ -921,7 +914,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = Y; g.lda = 4 * D; g.ka = 4 * D;
       g.B = W2; g.ldb = 2 * D; g.kb = 2 * D;
       g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes_b(g, 2 * D, D);
+      set_passes(g, 2 * D, D);
       g.bias = b2;
       g.out[0] = {F, tcg::OUT_BF16_HILO, (long long)2 * D, 0, D, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -931,7 +924,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = OA; g.lda = 2 * Pp; g.a_bs = (long long)S * 2 * Pp; g.a_batched = 1; g.ka = 2 * Pp; g.a_mn_major = 1; g.a_rows = S;
       g.B = F; g.ldb = 2 * D; g.b_bs = (long long)S * 2 * D; g.b_batched = 1; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = S;
       g.M = P; g.N = D; g.K = S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes_b(g, Pp, D);
+      set_passes(g, Pp, D);
       g.out[0] = {FE, tcg::OUT_F32, (long long)D, (long long)P * D, 0, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
     }
@@ -955,7 +948,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = F; g.lda = 2 * D; g.a_bs = (long long)S * 2 * D; g.a_batched = 1; g.ka = 2 * D;
       g.B = GFE; g.ldb = 2 * D; g.b_bs = (long long)P * 2 * D; g.b_batched = 1; g.kb = 2 * D;
       g.M = S; g.N = P; g.K = D; g.batch = nb; g.bn = pick_bn(P);
-      set_passes_b(g, D, D);
+      set_passes(g, D, D);
       if (gOcc) g.addin = {gOcc + (size_t)n0 * P * S, 1, (long long)P * S, (long long)S};
       g.signin = {OS, (long long)Pp, (long long)S * Pp, 0};
       g.out[0] = {GO, tcg::OUT_BF16_HILO, (long long)2 * Pp, (long long)S * 2 * Pp, Pp, Pp, 0, 0};
@@ -966,7 +959,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = OA; g.lda = 2 * Pp; g.a_bs = (long long)S * 2 * Pp; g.a_batched = 1; g.ka = 2 * Pp;
       g.B = GFE; g.ldb = 2 * D; g.b_bs = (long long)P * 2 * D; g.b_batched = 1; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = P;
       g.M = S; g.N = D; g.K = P; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes_b(g, Pp, D);
+      set_passes(g, Pp, D);
       g.out[0] = {GF, tcg::OUT_BF16_HILO, (long long)2 * D, (long long)S * 2 * D, D, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
     }
@@ -978,7 +971,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = GF; g.lda = 2 * D; g.ka = 2 * D;
       g.B = W2; g.ldb = 2 * D; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = D;
       g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes_b(g, D, D);
+      set_passes(g, D, D);
       g.mask = {Y, (long long)4 * D, 0, 0};
       g.out[0] = {GY, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -991,7 +984,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = GO; g.lda = 2 * Pp; g.ka = 2 * Pp;
       g.B = W5; g.ldb = 2 * D2; g.kb = 2 * D2; g.b_mn_major = 1; g.b_rows = P;
       g.M = (int)T; g.N = D2; g.K = P; g.batch = 1; g.bn = pick_bn(D2);
-      set_passes_b(g, Pp, D2);
+      set_passes(g, Pp, D2);
       g.mask = {G2, (long long)2 * D2, 0, 0};
       g.out[0] = {GG2, tcg::OUT_BF16_HILO, (long long)2 * D2, 0, D2, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -1003,7 +996,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = GG2; g.lda = 2 * D2; g.ka = 2 * D2;
       g.B = W4; g.ldb = 2 * D; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = D2;
       g.M = (int)T; g.N = D; g.K = D2; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes_b(g, D2, D);
+      set_passes(g, D2, D);
       g.mask = {Y + D, (long long)4 * D, 0, 0};
       g.out[0] = {GY + D, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, D, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
@@ -1021,7 +1014,7 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       g.A = GY; g.lda = 4 * D; g.ka = 4 * D;
       g.B = W13; g.ldb = 2 * C; g.kb = 2 * C; g.b_mn_major = 1; g.b_rows = 2 * D;
       g.M = (int)T; g.N = C; g.K = 2 * D; g.batch = 1; g.bn = C >= 256 ? 256 : (C >= 128 ? 128 : 64);
-      set_passes_b(g, 2 * D, C);
+      set_passes(g, 2 * D, C);
       if (occ_only) {   // the G1 half alone: gG1 [W3]
         g.A = GY + D; g.ka = 4 * D - D; g.B = W13 + (size_t)D * 2 * C; g.b_rows = D; g.K = D;
       }

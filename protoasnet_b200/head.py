@@ -38,6 +38,16 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def _head_params(m) -> list:
+    """The eleven head tensors of ``m`` in ``pasn_weights`` / ``pasn_grads`` order."""
+    a, o = m.add_on_layers, m.occurrence_module
+    return [a[0].weight, a[0].bias, a[2].weight, a[2].bias, o[0].weight, o[0].bias, o[2].weight, o[2].bias,
+            o[4].weight, m.prototype_vectors, m.last_layer.weight]
+
+
+_OCC_PARAMS = slice(4, 9)   # occurrence_module's five tensors within that order
+
+
 class _HeadRuntime:
     """Per-module launcher: owns the scratch buffer and the derived bf16 weight cache (never saved)."""
 
@@ -47,9 +57,7 @@ class _HeadRuntime:
         self._packed: Dict = {}
 
     def _weights_struct(self, m) -> Tuple[PasnWeights, list]:
-        a, o = m.add_on_layers, m.occurrence_module
-        tensors = [a[0].weight, a[0].bias, a[2].weight, a[2].bias, o[0].weight, o[0].bias, o[2].weight, o[2].bias,
-                   o[4].weight, m.prototype_vectors, m.last_layer.weight]
+        tensors = _head_params(m)
         for t in tensors:
             if t.dtype != torch.float32 or not t.is_contiguous():
                 raise _lib.PasnError("head parameters must be contiguous fp32 (the state_dict layout of the reference)")
@@ -167,10 +175,9 @@ class _HeadRuntime:
         return occ
 
 
-def _library_backward(ctx_rt, x, g_logits, g_sim, g_occ, want_gx):
+def _library_backward(rt, x, g_logits, g_sim, g_occ, want_gx):
     """pasn_head_backward on (x, head parameters): returns (grad_x or None, [11 parameter gradients]).  With g_logits and
     g_sim both None only the occurrence branch is differentiated (compute_occurence_map)."""
-    rt = ctx_rt
     lib = _lib.load()
     m = rt.owner
     dims, xc, spatial = rt.make_dims(x, m.kernel_path)   # GENERIC keeps the CUDA-core backward, anything else lets the
@@ -203,6 +210,10 @@ def _library_backward(ctx_rt, x, g_logits, g_sim, g_occ, want_gx):
     return gx, grads
 
 
+def _param_grads(grads, params, needed) -> tuple:
+    return tuple(g.reshape(p.shape) if need else None for g, p, need in zip(grads, params, needed))
+
+
 class _OccFunction(torch.autograd.Function):
     """(features, occurrence_module parameters) -> occurrence_map with gradients: compute_occurence_map under grad, which
     the reference's TransformLoss calls once more per training step (src/loss/loss.py:302).  Forward = the library's
@@ -220,10 +231,7 @@ class _OccFunction(torch.autograd.Function):
     def backward(ctx, g_occ):
         x, *params = ctx.saved_tensors
         gx, grads = _library_backward(ctx.rt, x, None, None, g_occ, ctx.needs_input_grad[1])
-        out = [None, gx]
-        for i in range(5):   # occ_w1, occ_b1, occ_w2, occ_b2, occ_w3 = entries 4..8 of the weight struct
-            out.append(grads[4 + i].reshape(params[i].shape) if ctx.needs_input_grad[2 + i] else None)
-        return tuple(out)
+        return (None, gx) + _param_grads(grads[_OCC_PARAMS], params, ctx.needs_input_grad[2:])
 
 
 class _HeadFunction(torch.autograd.Function):
@@ -242,11 +250,7 @@ class _HeadFunction(torch.autograd.Function):
     def backward(ctx, g_logits, g_sim, g_occ):
         x, *params = ctx.saved_tensors
         gx, grads = _library_backward(ctx.rt, x, g_logits, g_sim, g_occ, ctx.needs_input_grad[1])
-        tensors = grads
-        out = [None, gx]
-        for i, t in enumerate(tensors):
-            out.append(grads[i].reshape(params[i].shape) if ctx.needs_input_grad[2 + i] else None)
-        return tuple(out)
+        return (None, gx) + _param_grads(grads, params, ctx.needs_input_grad[2:])
 
 
 class HostPipeline:
@@ -440,10 +444,7 @@ class PrototypeHeadMixin:
 
     def _kernel_autograd(self, x):
         """(logits, similarity, occurrence_map) with gradients flowing through pasn_head_backward."""
-        a, o = self.add_on_layers, self.occurrence_module
-        params = (a[0].weight, a[0].bias, a[2].weight, a[2].bias, o[0].weight, o[0].bias, o[2].weight, o[2].bias,
-                  o[4].weight, self.prototype_vectors, self.last_layer.weight)
-        return _HeadFunction.apply(self._rt, x, *params)
+        return _HeadFunction.apply(self._rt, x, *_head_params(self))
 
     # ---- reference API ----
     def forward(self, x):
@@ -462,8 +463,7 @@ class PrototypeHeadMixin:
         x = self.cnn_backbone(x)
         if self._grad_guard(x):
             if self.autograd_mode == "kernel":
-                o = self.occurrence_module
-                return _OccFunction.apply(self._rt, x, o[0].weight, o[0].bias, o[2].weight, o[2].bias, o[4].weight)
+                return _OccFunction.apply(self._rt, x, *_head_params(self)[_OCC_PARAMS])
             return torch.abs(self.occurrence_module(x)).unsqueeze(2)
         return self._rt.occurrence_only(x)
 
