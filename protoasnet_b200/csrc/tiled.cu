@@ -215,17 +215,74 @@ __global__ void __launch_bounds__(256) clip_colsum_kernel(const __nv_bfloat16* _
   }
 }
 
-// passes of a product of two operands that each come as planes (hi at column 0, lo at column *_lo); an operand without a
-// lo plane (bf16 mode, or a bf16-exact feature map) drops its pass.  Both split: hi*hi, hi*lo, lo*hi.  The lo*lo term is
-// below the representation error of the split itself (each operand keeps 16 significant bits: |x - xh - xl| <= 2^-17 |x|,
-// and |xl wl| <= 2^-18 |x w|), so it is not computed.
-void set_passes(tcg::Gemm& g, int a_lo, int b_lo, bool a_has_lo = true, bool b_has_lo = true) {
+// A bf16 activation or weight in the plane format of the chain: row r (of batch item b) starts at ptr + b*bs + r*ld, the hi
+// plane at column 0 and, when split, the lo plane at column lo (x ~ hi + lo: fp32 mode, and every backward operand).
+struct Planes {
+  const __nv_bfloat16* ptr;
+  long long ld;
+  int lo;             // width of a plane: the lo plane's column (an unsplit output keeps it as its lo_off)
+  bool split;
+  int cols = 0;       // columns an operand load covers from ptr, the tensor map's width (0: ld)
+  long long bs = 0;   // batch stride (0: one matrix for all batch items)
+  int rows = 0;       // rows per batch item that hold values, the rest read as zeros (0: all)
+  bool mn = false;    // read MN-major: rows are the k index (token-major operands of the pooling and weight gradients)
+  int width() const { return cols ? cols : (int)ld; }
+  Planes at(int c) const { Planes v = *this; v.ptr += c; v.cols = width() - c; return v; }   // columns from c on
+  Planes row(long long r) const { Planes v = *this; v.ptr += r * ld; return v; }
+  Planes with(long long bs_, int rows_, bool mn_) const { Planes v = *this; v.bs = bs_; v.rows = rows_; v.mn = mn_; return v; }
+};
+// a buffer of rows of w hi columns, followed by w lo columns when split
+Planes planes(const void* p, int w, bool split) {
+  return {reinterpret_cast<const __nv_bfloat16*>(p), (split ? 2 : 1) * (long long)w, w, split};
+}
+// the output that writes v (ncols: columns stored per plane, 0: N); every output view is of the chain's own workspace
+tcg::Output store(const Planes& v, int ncols = 0) {
+  return {const_cast<__nv_bfloat16*>(v.ptr), v.split ? tcg::OUT_BF16_HILO : tcg::OUT_BF16, v.ld, v.bs, v.lo, ncols, 0, 0};
+}
+// a GEMM of the chain over A = a, B = b.  Passes: hi*hi, then B's lo plane, then A's (this order fixes the fp32
+// accumulation order); an operand without a lo plane (bf16 mode, or a bf16-exact feature map) drops its pass.  The lo*lo
+// term is below the representation error of the split itself (each operand keeps 16 significant bits:
+// |x - xh - xl| <= 2^-17 |x|, and |xl wl| <= 2^-18 |x w|), so it is not computed.
+tcg::Gemm gemm(const Planes& a, const Planes& b, int M, int N, int K, int batch, int bn) {
+  tcg::Gemm g{};
+  g.A = a.ptr; g.lda = a.ld; g.a_bs = a.bs; g.a_batched = a.bs != 0; g.ka = a.width(); g.a_mn_major = a.mn; g.a_rows = a.rows;
+  g.B = b.ptr; g.ldb = b.ld; g.b_bs = b.bs; g.b_batched = b.bs != 0; g.kb = b.width(); g.b_mn_major = b.mn; g.b_rows = b.rows;
+  g.M = M; g.N = N; g.K = K; g.batch = batch; g.bn = bn;
+  g.npass = 1;
+  if (b.split) g.b_off[g.npass++] = b.lo;
+  if (a.split) g.a_off[g.npass++] = a.lo;
   g.pair = 1;   // CTA pairs wherever the shape allows (tc_gemm.cu decides)
-  for (int q = 0; q < 4; ++q) g.a_off[q] = g.b_off[q] = 0;
-  int n = 1;
-  if (b_has_lo) { g.b_off[n] = b_lo; ++n; }
-  if (a_has_lo) { g.a_off[n] = a_lo; ++n; }
-  g.npass = n;
+  return g;
+}
+
+// Layers shared by the forward chain and the backward's recompute.
+// [H1 | G1] = relu(X [W1; W3]^T + [b1; b3]), or G1 alone with w13 and b13 from row D on
+int first_layer(const Planes& x, const Planes& w13, const float* b13, int M, int N, int C, int batch, int bn,
+                const tcg::Output& y, bool f16, cudaStream_t st) {
+  tcg::Gemm g = gemm(x, w13, M, N, C, batch, bn);
+  g.bias = b13; g.act = tcg::ACT_RELU;
+  g.ab_f16 = f16;   // X and [W1; W3] both fp16 (pack: tiled_pack_weights)
+  g.out[0] = y;
+  return tcg::launch(g, st);
+}
+// G2 = relu(G1 W4^T + b4)
+int g1_layer(const Planes& g1, const Planes& w4, const float* b4, long long T, int D, const Planes& g2, cudaStream_t st) {
+  tcg::Gemm g = gemm(g1, w4, (int)T, D / 2, D, 1, pick_bn(D / 2));
+  g.bias = b4; g.act = tcg::ACT_RELU;
+  g.out[0] = store(g2);
+  return tcg::launch(g, st);
+}
+// F = H1 W2^T + b2 over all tokens
+int w2_layer(const Planes& h1, const Planes& w2, const float* b2, long long T, int D, const Planes& f, cudaStream_t st) {
+  tcg::Gemm g = gemm(h1, w2, (int)T, D, D, 1, D >= 256 ? 256 : 128);
+  g.bias = b2;
+  g.out[0] = store(f);
+  return tcg::launch(g, st);
+}
+// per-clip pooling out[n] = O[n] V[n] over the clip's S tokens: o = the occurrence values (per clip [P][S], or token-major
+// [S][P] read MN-major), K of them per plane; v = token-major values of all tokens (H1 or F), the MN-major B operand
+tcg::Gemm pooling(const Planes& o, int K, const Planes& v, int P, int D, int S, int nb) {
+  return gemm(o, v.with((long long)S * v.ld, S, true), P, D, K, nb, D >= 256 ? 256 : 128);
 }
 
 // The first layer's A operand for nb clips of the feature map at x: token-major planes XT[(n*S + s)][planes*C] in dst, either
@@ -338,11 +395,7 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   bool x_direct;
   const char* x = reinterpret_cast<const char*>(feat) + (size_t)n0 * C * S * elt;
   if ((rc = token_operand(x, d, nb, hilo, reinterpret_cast<__nv_bfloat16*>(ws + p.off_xt), &xt, &x_direct, st))) return rc;
-  __nv_bfloat16* Y = reinterpret_cast<__nv_bfloat16*>(ws + p.off_y);
-  __nv_bfloat16* G2 = reinterpret_cast<__nv_bfloat16*>(ws + p.off_g2);
-  __nv_bfloat16* OCC = reinterpret_cast<__nv_bfloat16*>(ws + p.off_occ);
   float* PSUM = reinterpret_cast<float*>(ws + p.off_psum);
-  __nv_bfloat16* POOL = reinterpret_cast<__nv_bfloat16*>(ws + p.off_pool);
   float* FE = feats ? feats + (size_t)n0 * P * D : reinterpret_cast<float*>(ws + p.off_fe);
   // Plain forward (nobody asked for features_extracted, no push): the GEMM that would write the pooled features leaves the
   // two reductions the prototype stage needs (||f||^2, <f, v_p>) instead -- the features are neither stored nor read back.
@@ -353,102 +406,68 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   const bool fuse_stats = p.w2_first && (P >= 1024 || P <= 64) && !occ_only && feats == nullptr && push == nullptr;
   float* STAT = reinterpret_cast<float*>(ws + p.off_stat);
   int stat_parts = 2 * ceil_div(D, D >= 256 ? 256 : 128);   // column half-tiles of the GEMM that leaves the statistics
-  const __nv_bfloat16* W13 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w13);
-  const __nv_bfloat16* W4 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w4);
-  const __nv_bfloat16* W5 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w5);
-  const __nv_bfloat16* W2 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w2);
+  const Planes w13 = planes(pk + L.off_w13, C, hilo), w4 = planes(pk + L.off_w4, D, hilo),
+               w5 = planes(pk + L.off_w5, D2, hilo), w2 = planes(pk + L.off_w2, D, hilo);
   const float* b13 = reinterpret_cast<const float*>(pk + L.off_b13);
   const float* b4 = reinterpret_cast<const float*>(pk + L.off_b4);
   const float* b2 = reinterpret_cast<const float*>(pk + L.off_b2);
 
   // ---- (A) [H1 | G1] = relu(X [W1; W3]^T + [b1; b3])        (occurrence only: G1 alone)
   const int nA = occ_only ? D : 2 * D;          // output columns per plane
-  {
-    tcg::Gemm g{};
-    g.A = xt; g.lda = (long long)ex * C; g.a_bs = 0; g.a_batched = 0; g.ka = ex * C;
-    g.B = occ_only ? W13 + (size_t)D * ex * C : W13; g.ldb = (long long)ex * C; g.b_bs = 0; g.b_batched = 0; g.kb = ex * C;
-    g.M = (int)T; g.N = nA; g.K = C; g.batch = 1; g.bn = 256;
-    set_passes(g, C, C, hilo, hilo);
-    g.bias = occ_only ? b13 + D : b13; g.act = tcg::ACT_RELU;
-    g.ab_f16 = f16 ? 1 : 0;   // X and [W1; W3] both fp16 (pack: tiled_pack_weights)
-    g.out[0] = {Y, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * nA, 0, nA};
-    if (x_direct) {   // one GEMM per clip: rows = its S voxels, operand [C rows][S] as it lies in the feature map
-      g.a_mn_major = 1; g.lda = S; g.a_bs = (long long)C * S; g.a_batched = 1; g.ka = S; g.a_rows = C;
-      g.M = S; g.batch = nb;
-      g.out[0].bs = (long long)S * ex * nA;
-    }
-    if ((rc = tcg::launch(g, st))) return rc;
+  const Planes y = planes(ws + p.off_y, nA, hilo), g2 = planes(ws + p.off_g2, D2, hilo);
+  if (x_direct) {   // one GEMM per clip: rows = its S voxels, operand [C rows][S] as it lies in the feature map
+    rc = first_layer(Planes{xt, S, 0, false}.with((long long)C * S, C, true), occ_only ? w13.row(D) : w13, occ_only ? b13 + D : b13,
+                     S, nA, C, nb, 256, store(y.with((long long)S * y.ld, 0, false)), f16, st);
+  } else {
+    rc = first_layer(planes(xt, C, hilo), occ_only ? w13.row(D) : w13, occ_only ? b13 + D : b13, (int)T, nA, C, 1, 256, store(y),
+                     f16, st);
   }
+  if (rc) return rc;
   // ---- (B) G2 = relu(G1 W4^T + b4)
-  const int g1_off = occ_only ? 0 : D;          // column of G1 inside a plane of Y
-  {
-    tcg::Gemm g{};
-    g.A = Y + g1_off; g.lda = (long long)ex * nA; g.a_batched = 0; g.ka = ex * nA - g1_off;
-    g.B = W4; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
-    g.M = (int)T; g.N = D2; g.K = D; g.batch = 1; g.bn = pick_bn(D2);
-    set_passes(g, nA, D, hilo, hilo);
-    g.bias = b4; g.act = tcg::ACT_RELU;
-    g.out[0] = {G2, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * D2, 0, D2};
-    if ((rc = tcg::launch(g, st))) return rc;
-  }
+  if ((rc = g1_layer(y.at(occ_only ? 0 : D), w4, b4, T, D, g2, st))) return rc;
   // ---- (C) O[n] = |W5 G2[n]^T|  -> occurrence_map [n][P][S] (+ the pooling operand copy when the map cannot serve as one)
   void* occ_user = occ ? reinterpret_cast<char*>(occ) + (size_t)n0 * P * S * elt : nullptr;
   const int occ_mode = ex == 2 ? tcg::OUT_F32 : (f16 ? tcg::OUT_F16 : tcg::OUT_BF16);   // the map in the feature map's type
-  const __nv_bfloat16* pool_a = nullptr;     // pooling A operand
-  long long pool_lda = 0;
+  Planes pool{};   // the pooling's A operand: the occurrence values, pool_k of them per plane and clip
+  int pool_k = S;
   // W2-after-pooling order: the row sums over s then come from a small column-sum kernel below.  (fp32 maps keep the
   // per-clip form there: their map leaves as 4-byte plain stores, which measured slower than the TMA rows -- 0.72 vs 0.64 ms)
   const bool tok_c = p.tok_c && (occ_only || p.w2_first || ex == 1);
   if (tok_c) {
     // few prototypes: O^T = |G2 W5^T| over all tokens in one GEMM (rows = tokens, N = P).  The occurrence map leaves
     // channel-major per clip through plain stores that are coalesced along the voxels; the token-major copy
-    // [T][ex*Pp] is the pooling's MN-major A operand.
-    tcg::Gemm g{};
-    g.A = G2; g.lda = (long long)ex * D2; g.a_batched = 0; g.ka = ex * D2;
-    g.B = W5; g.ldb = (long long)ex * D2; g.b_batched = 0; g.kb = ex * D2;
-    g.M = (int)T; g.N = P; g.K = D2; g.batch = 1; g.bn = 64;
-    set_passes(g, D2, D2, hilo, hilo);
+    // [T][ex*Pp] is the pooling's MN-major A operand ([S rows][P] per clip, prototypes contiguous).
+    tcg::Gemm g = gemm(g2, w5, (int)T, P, D2, 1, 64);
     g.act = tcg::ACT_ABS;
     int no = 0;
-    if (occ_user != nullptr) {
-      g.out[no] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0, P, 0, S};
-      ++no;
-    }
+    if (occ_user != nullptr) g.out[no++] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0, P, 0, S};
+    const Planes o = planes(ws + p.off_occ, p.Pp, hilo);
     if (!occ_only) {
-      g.out[no] = {OCC, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * p.Pp, 0, p.Pp, P, 0, 0};
-      ++no;
-      pool_a = OCC; pool_lda = (long long)ex * p.Pp;
+      g.out[no++] = store(o, P);
+      pool = o.with((long long)S * o.ld, S, true);
     }
     if ((rc = tcg::launch(g, st))) return rc;
     if (!occ_only && !p.w2_first) {   // Osum[n][p] = sum_s O[n,s,p] (of the stored values: what the pooling will read)
       dim3 grid(ceil_div(P, 32), nb);
-      clip_colsum_kernel<<<grid, 256, 0, st>>>(OCC, S, P, ex * p.Pp, ex == 2 ? p.Pp : 0, PSUM);
+      clip_colsum_kernel<<<grid, 256, 0, st>>>(o.ptr, S, P, o.ld, o.split ? o.lo : 0, PSUM);
       PASN_LAUNCH_CHECK();
       count_launch();
     }
   } else {
-    tcg::Gemm g{};
-    g.A = W5; g.lda = (long long)ex * D2; g.a_batched = 0; g.ka = ex * D2;
-    g.B = G2; g.ldb = (long long)ex * D2; g.b_bs = (long long)S * ex * D2; g.b_batched = 1; g.kb = ex * D2;
-    g.b_rows = S;   // tokens of this clip; the padded columns of the operand copy come out as exact zeros
-    g.M = P; g.K = D2; g.batch = nb; g.bn = p.bn_c;
-    g.N = ex == 2 ? p.Sp : S;
-    set_passes(g, D2, D2, hilo, hilo);
+    pool_k = ex == 2 ? p.Sp : S;
+    // b_rows = S: tokens of this clip; the padded columns of the operand copy come out as exact zeros
+    tcg::Gemm g = gemm(w5, g2.with((long long)S * g2.ld, S, false), P, pool_k, D2, nb, p.bn_c);
     g.act = tcg::ACT_ABS;
     int no = 0;
     const bool need_copy = !occ_only && !(p.occ_direct && occ_user != nullptr);
-    if (occ_user != nullptr) {
-      g.out[no] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0};
-      g.out[no].ncols = S;
-      ++no;
-    }
+    if (occ_user != nullptr) g.out[no++] = {occ_user, occ_mode, (long long)S, (long long)P * S, 0, S, 0, 0};
     if (need_copy) {
-      g.out[no] = {OCC, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * p.Sp, (long long)P * ex * p.Sp, p.Sp};
-      g.out[no].ncols = ex == 2 ? p.Sp : S;
-      ++no;
-      pool_a = OCC; pool_lda = (long long)ex * p.Sp;
+      pool = planes(ws + p.off_occ, p.Sp, hilo);
+      pool = pool.with((long long)P * pool.ld, 0, false);
+      pool.cols = hilo ? 0 : S;   // one plane: its columns from S on are not stored
+      g.out[no++] = store(pool, pool_k);
     } else if (!occ_only) {
-      pool_a = reinterpret_cast<const __nv_bfloat16*>(occ_user); pool_lda = S;
+      pool = Planes{reinterpret_cast<const __nv_bfloat16*>(occ_user), S, 0, false}.with((long long)P * S, 0, false);
     }
     g.psum = (occ_only || p.w2_first) ? nullptr : PSUM;
     g.psum_rounded = ex == 1;
@@ -457,76 +476,35 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
   if (occ_only) return PASN_OK;
   if (p.w2_first) {
     // ---- (D') F = H1 W2^T + b2 over all tokens, then FE[n] = O[n] F[n] (K = S) straight into fp32
-    __nv_bfloat16* F = reinterpret_cast<__nv_bfloat16*>(ws + p.off_f);
-    {
-      tcg::Gemm g{};
-      g.A = Y; g.lda = (long long)ex * 2 * D; g.a_batched = 0; g.ka = ex * 2 * D;
-      g.B = W2; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
-      g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, 2 * D, D, hilo, hilo);
-      g.bias = b2; g.act = tcg::ACT_NONE;
-      g.out[0] = {F, ex == 1 ? tcg::OUT_BF16 : tcg::OUT_BF16_HILO, (long long)ex * D, 0, D};
-      if ((rc = tcg::launch(g, st))) return rc;
-    }
-    {
-      tcg::Gemm g{};
-      g.A = pool_a; g.lda = pool_lda; g.a_bs = (long long)P * pool_lda; g.a_batched = 1;
-      g.ka = ex == 2 ? 2 * p.Sp : S;
-      g.B = F; g.ldb = (long long)ex * D; g.b_bs = (long long)S * ex * D; g.b_batched = 1; g.kb = ex * D;
-      g.b_mn_major = 1; g.b_rows = S;
-      g.M = P; g.N = D; g.K = ex == 2 ? p.Sp : S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, p.Sp, D, hilo, hilo);
-      if (tok_c) {   // occurrence values token-major: [S rows][P] per clip, prototypes contiguous (MN-major A)
-        g.a_mn_major = 1; g.a_bs = (long long)S * pool_lda; g.ka = ex * p.Pp; g.a_rows = S; g.K = S;
-        set_passes(g, p.Pp, D, hilo, hilo);
+    const Planes f = planes(ws + p.off_f, D, hilo);
+    if ((rc = w2_layer(y, w2, b2, T, D, f, st))) return rc;
+    tcg::Gemm g = pooling(pool, pool_k, f, P, D, S, nb);
+    g.out[0] = {FE, tcg::OUT_F32, (long long)D, (long long)P * D, 0};
+    if (fuse_stats) {
+      g.out[0].mode = tcg::OUT_NONE;
+      g.rowstat = STAT; g.dotvec = w.prototypes; g.dot_ld = D; g.dot_mod = P; g.dot_early = 1;   // (parameters: the chain does not write them)
+      // few prototypes, few voxels (image head: 40 x 49): three clips share a 128-row tile, block-diagonally -- a clip alone
+      // uses 40 of the tile's rows and two of the four epilogue row groups
+      const int G = 128 / P < 4 ? 128 / P : 4;
+      if (tok_c && ex == 1 && S <= 64 && G >= 2 && nb >= 2 * G) {
+        g.group = G; g.group_rows = P; g.group_items = nb;
+        g.M = G * P; g.batch = ceil_div(nb, G); g.bn = 128;
+        g.stat_rows = (long long)nb * P;
+        stat_parts = 2 * ceil_div(D, 128);
       }
-      g.act = tcg::ACT_NONE;
-      g.out[0] = {FE, tcg::OUT_F32, (long long)D, (long long)P * D, 0};
-      if (fuse_stats) {
-        g.out[0].mode = tcg::OUT_NONE;
-        g.rowstat = STAT; g.dotvec = w.prototypes; g.dot_ld = D; g.dot_mod = P; g.dot_early = 1;   // (parameters: the chain does not write them)
-        // few prototypes, few voxels (image head: 40 x 49): three clips share a 128-row tile, block-diagonally -- a clip alone
-        // uses 40 of the tile's rows and two of the four epilogue row groups
-        const int G = 128 / P < 4 ? 128 / P : 4;
-        if (tok_c && ex == 1 && S <= 64 && G >= 2 && nb >= 2 * G) {
-          g.group = G; g.group_rows = P; g.group_items = nb;
-          g.M = G * P; g.batch = ceil_div(nb, G); g.bn = 128;
-          g.stat_rows = (long long)nb * P;
-          stat_parts = 2 * ceil_div(D, 128);
-        }
-      }
-      if ((rc = tcg::launch(g, st))) return rc;
     }
-  } else {
-  // ---- (D) pooled[n] = O[n] H1[n]   (K = S; H1 token-major = MN-major B operand) -> bf16 hi | lo planes
-  {
-    tcg::Gemm g{};
-    g.A = pool_a; g.lda = pool_lda; g.a_bs = (long long)P * pool_lda; g.a_batched = 1;
-    g.ka = ex == 2 ? 2 * p.Sp : S;
-    g.B = Y; g.ldb = (long long)ex * 2 * D; g.b_bs = (long long)S * ex * 2 * D; g.b_batched = 1; g.kb = ex * 2 * D;
-    g.b_mn_major = 1; g.b_rows = S;
-    g.M = P; g.N = D; g.K = ex == 2 ? p.Sp : S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-    set_passes(g, p.Sp, 2 * D, hilo, hilo);
-    if (tok_c) {   // occurrence values token-major: [S rows][P] per clip (MN-major A)
-      g.a_mn_major = 1; g.a_bs = (long long)S * pool_lda; g.ka = ex * p.Pp; g.a_rows = S; g.K = S;
-      set_passes(g, p.Pp, 2 * D, hilo, hilo);
-    }
-    g.act = tcg::ACT_NONE;
-    g.out[0] = {POOL, tcg::OUT_BF16_HILO, (long long)2 * D, (long long)P * 2 * D, D};
     if ((rc = tcg::launch(g, st))) return rc;
-  }
-  // ---- (E) FE = pooled W2^T + (sum_s O) b2^T   (pooled = hi + lo; fp32 mode: W2 = hi + lo as well)
-  {
-    tcg::Gemm g{};
-    g.A = POOL; g.lda = 2 * D; g.a_batched = 0; g.ka = 2 * D;
-    g.B = W2; g.ldb = (long long)ex * D; g.b_batched = 0; g.kb = ex * D;
-    g.M = nb * P; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-    set_passes(g, D, D, true, hilo);   // pooled = hi + lo planes in both modes
+  } else {
+    // ---- (D) pooled[n] = O[n] H1[n]   (K = S; H1 token-major = MN-major B operand) -> bf16 hi | lo planes in both modes
+    const Planes pooled = planes(ws + p.off_pool, D, true);
+    tcg::Gemm g = pooling(pool, pool_k, y, P, D, S, nb);
+    g.out[0] = store(pooled.with((long long)P * pooled.ld, 0, false));
+    if ((rc = tcg::launch(g, st))) return rc;
+    // ---- (E) FE = pooled W2^T + (sum_s O) b2^T   (fp32 mode: W2 = hi + lo as well)
+    g = gemm(pooled, w2, nb * P, D, D, 1, D >= 256 ? 256 : 128);
     g.rowparts = PSUM; g.nparts = tok_c ? 1 : 2 * p.tiles_n_c; g.colvec = b2;
-    g.act = tcg::ACT_NONE;
     g.out[0] = {FE, tcg::OUT_F32, (long long)D, 0, 0};
     if ((rc = tcg::launch(g, st))) return rc;
-  }
   }
   // ---- cosine / similarity / logits / distance / push keys (+ winner capture)
   if (fuse_stats)
@@ -539,37 +517,34 @@ static int tiled_chunk(const void* feat, const pasn_weights& w, const void* pack
                             dist ? dist + (size_t)n0 * P : nullptr, pp, st);
 }
 
-int tiled_head_forward(const void* feat, const pasn_weights& w, const void* packed, const pasn_dims& d, float* logits,
-                       float* sim, void* occ, float* feats, float* dist, const pasn_push_args* push, void* ws,
-                       size_t ws_bytes, cudaStream_t st) {
+// the chain over all clips, chunk by chunk
+static int tiled_chunks(const void* feat, const pasn_weights& w, const void* packed, const pasn_dims& d, float* logits,
+                        float* sim, void* occ, float* feats, float* dist, const pasn_push_args* push, void* ws, size_t ws_bytes,
+                        bool occ_only, cudaStream_t st) {
   if (!tiled_supported(d) || packed == nullptr) return PASN_ERR_UNSUPPORTED;
   const Plan p = make_plan(d);
   if (ws_bytes < p.total) return PASN_ERR_WORKSPACE;
   if (((uintptr_t)ws & 255) != 0 || ((uintptr_t)feat & 15) != 0) return PASN_ERR_ALIGN;
-  main_kernel_begin(st);   // tiled path: the "dominant kernel" is the GEMM chain
+  if (!occ_only) main_kernel_begin(st);   // tiled path: the "dominant kernel" is the GEMM chain
   for (int n0 = 0; n0 < d.N; n0 += p.nb) {
     const int nb = d.N - n0 < p.nb ? d.N - n0 : p.nb;
     const int rc = tiled_chunk(feat, w, packed, d, p, n0, nb, logits, sim, occ, feats, dist, push, reinterpret_cast<char*>(ws),
-                               false, st);
+                               occ_only, st);
     if (rc) return rc;
   }
-  main_kernel_end(st);
+  if (!occ_only) main_kernel_end(st);
   return PASN_OK;
+}
+
+int tiled_head_forward(const void* feat, const pasn_weights& w, const void* packed, const pasn_dims& d, float* logits,
+                       float* sim, void* occ, float* feats, float* dist, const pasn_push_args* push, void* ws,
+                       size_t ws_bytes, cudaStream_t st) {
+  return tiled_chunks(feat, w, packed, d, logits, sim, occ, feats, dist, push, ws, ws_bytes, false, st);
 }
 
 int tiled_occurrence_only(const void* feat, const pasn_weights& w, const void* packed, const pasn_dims& d, void* occ, void* ws,
                           size_t ws_bytes, cudaStream_t st) {
-  if (!tiled_supported(d) || packed == nullptr) return PASN_ERR_UNSUPPORTED;
-  const Plan p = make_plan(d);
-  if (ws_bytes < p.total) return PASN_ERR_WORKSPACE;
-  if (((uintptr_t)ws & 255) != 0 || ((uintptr_t)feat & 15) != 0) return PASN_ERR_ALIGN;
-  for (int n0 = 0; n0 < d.N; n0 += p.nb) {
-    const int nb = d.N - n0 < p.nb ? d.N - n0 : p.nb;
-    const int rc = tiled_chunk(feat, w, packed, d, p, n0, nb, nullptr, nullptr, occ, nullptr, nullptr, nullptr,
-                               reinterpret_cast<char*>(ws), true, st);
-    if (rc) return rc;
-  }
-  return PASN_OK;
+  return tiled_chunks(feat, w, packed, d, nullptr, nullptr, occ, nullptr, nullptr, nullptr, ws, ws_bytes, true, st);
 }
 
 
@@ -805,16 +780,17 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
   const PackLayout L = pack_layout(d2);
   if ((rc = tiled_pack_weights(w, d2, ws + b.off_pk, st))) return rc;
   const char* pk = ws + b.off_pk;
-  const __nv_bfloat16* W13 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w13);   // [2D][2C]
-  const __nv_bfloat16* W4 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w4);     // [D2][2D]
-  const __nv_bfloat16* W5 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w5);     // [P][2 D2]
-  const __nv_bfloat16* W2 = reinterpret_cast<const __nv_bfloat16*>(pk + L.off_w2);     // [D][2D]
+  const Planes w13 = planes(pk + L.off_w13, C, true), w4 = planes(pk + L.off_w4, D, true),
+               w5 = planes(pk + L.off_w5, D2, true), w2 = planes(pk + L.off_w2, D, true);
   const float* b13 = reinterpret_cast<const float*>(pk + L.off_b13);
   const float* b4 = reinterpret_cast<const float*>(pk + L.off_b4);
   const float* b2 = reinterpret_cast<const float*>(pk + L.off_b2);
   auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(ws + off); };
-  __nv_bfloat16 *XT = bf(b.off_xt), *Y = bf(b.off_y), *G2 = bf(b.off_g2), *OS = bf(b.off_os), *OA = bf(b.off_oa), *F = bf(b.off_f),
-                *GFE = bf(b.off_gfe), *GO = bf(b.off_go), *GF = bf(b.off_gf), *GY = bf(b.off_gy), *GG2 = bf(b.off_gg2);
+  __nv_bfloat16 *XT = bf(b.off_xt), *OS = bf(b.off_os), *GFE = bf(b.off_gfe), *GO = bf(b.off_go);
+  // activations and their gradients: hi | lo planes (the recomputed forward's Y keeps 2D columns per plane)
+  const Planes y = planes(bf(b.off_y), 2 * D, true), g2 = planes(bf(b.off_g2), D2, true), oa = planes(bf(b.off_oa), Pp, true),
+               f = planes(bf(b.off_f), D, true), gfe = planes(GFE, D, true), go = planes(GO, Pp, true),
+               gf = planes(bf(b.off_gf), D, true), gy = planes(bf(b.off_gy), 2 * D, true), gg2 = planes(bf(b.off_gg2), D2, true);
   float* FE = reinterpret_cast<float*>(ws + b.off_fe);
   float4* RS = reinterpret_cast<float4*>(ws + b.off_rs);
   float* PART = reinterpret_cast<float*>(ws + b.off_part);
@@ -828,19 +804,16 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     return PASN_OK;
   }
 
-  // gW[m][n] (+)= sum_t A[t][m] B[t][n] over the tokens of the chunk (hi|lo planes, lo at column a_lo / b_lo)
-  auto wgrad = [&](const __nv_bfloat16* A, long long lda, int a_lo, int M, const __nv_bfloat16* B, long long ldb, int b_lo,
-                   bool b_has_lo, int N, long long T, float* dst0, int rows0, float* dst1) -> int {
+  // gW[m][n] (+)= sum_t a[t][m] b[t][n] over the T tokens of the chunk
+  auto wgrad = [&](const Planes& a, int M, const Planes& bv, int N, long long T, float* dst0, int rows0, float* dst1) -> int {
     const int bn = N >= 256 ? 256 : (N >= 128 ? 128 : 64);
     const int tiles = ceil_div(M, 256) * ceil_div(N, bn) * 2;
     int kper;
     int parts = split_parts(T, tiles > 148 ? 148 : tiles, &kper);
     while ((size_t)parts * M * N * 4 > b.part_bytes && parts > 1) { kper *= 2; parts = (int)((T + kper - 1) / kper); }
-    tcg::Gemm g{};
-    g.A = A; g.lda = lda; g.ka = (int)lda; g.a_mn_major = 1; g.a_rows = (int)T;
-    g.B = B; g.ldb = ldb; g.kb = (int)ldb; g.b_mn_major = 1; g.b_rows = (int)T;
-    g.M = M; g.N = N; g.K = kper; g.batch = parts; g.k_rows_per_batch = kper; g.bn = bn;
-    set_passes(g, a_lo, b_lo, true, b_has_lo);
+    tcg::Gemm g = gemm(a.with(0, (int)T, true), bv.with(0, (int)T, true), M, N, kper, parts, bn);
+    g.ka = (int)a.ld; g.kb = (int)bv.ld;   // the maps span ld columns from where the views start
+    g.k_rows_per_batch = kper;
     g.out[0] = {PART, tcg::OUT_F32, (long long)N, (long long)M * N, 0, 0, 0, 0};
     int r = tcg::launch(g, st);
     if (r) return r;
@@ -850,9 +823,10 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     count_launch();
     return PASN_OK;
   };
-  auto colsum = [&](const __nv_bfloat16* X, long long T, long long ld, int lo_off, int ncols, float* g0, int cols0, float* g1) -> int {
+  // g0[c] (+)= sum over the T rows of v's hi + lo planes, columns c >= cols0 into g1
+  auto colsum = [&](const Planes& v, long long T, int ncols, float* g0, int cols0, float* g1) -> int {
     dim3 grid(ceil_div(ncols, 64), (unsigned)((T + 511) / 512));   // ncols is even on every caller (channel counts)
-    colsum_planes_kernel<<<grid, 256, 0, st>>>(X, T, ld, lo_off, ncols, g0, cols0, g1 ? g1 : g0);
+    colsum_planes_kernel<<<grid, 256, 0, st>>>(v.ptr, T, v.ld, v.lo, ncols, g0, cols0, g1 ? g1 : g0);
     if (cudaGetLastError() != cudaSuccess) return PASN_ERR_CUDA;
     count_launch();
     return PASN_OK;
@@ -865,42 +839,23 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     // ---- token-major feature planes
     const __nv_bfloat16* xt;
     if ((rc = token_operand(x, d, nb, x_lo, XT, &xt, nullptr, st))) return rc;
-    const long long ldx = (long long)xe * C;
+    const Planes xv = planes(xt, C, x_lo);
 
-    // ================= forward, recomputed
-    {  // [H1 | G1] = relu(X [W1; W3]^T + b)
-      tcg::Gemm g{};
-      g.A = xt; g.lda = ldx; g.ka = (int)ldx;
-      g.B = W13; g.ldb = 2 * C; g.kb = 2 * C;
-      g.M = (int)T; g.N = 2 * D; g.K = C; g.batch = 1; g.bn = 256;
-      set_passes(g, C, C, x_lo, true);
-      g.bias = b13; g.act = tcg::ACT_RELU;
-      g.out[0] = {Y, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, 0, 0, 0};
-      if (occ_only) {   // G1 alone, into its usual columns [D, 2D) of the planes
-        g.B = W13 + (size_t)D * 2 * C; g.N = D; g.bias = b13 + D; g.bn = D >= 256 ? 256 : 128;
-        g.out[0] = {Y + D, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, D, 0, 0};
-      }
-      if ((rc = tcg::launch(g, st))) return rc;
+    // ================= forward, recomputed: the forward's layers in fp32 mode
+    if (occ_only) {   // G1 alone, into its usual columns [D, 2D) of the planes
+      rc = first_layer(xv, w13.row(D), b13 + D, (int)T, D, C, 1, D >= 256 ? 256 : 128, store(y.at(D), D), false, st);
+    } else {
+      rc = first_layer(xv, w13, b13, (int)T, 2 * D, C, 1, 256, store(y), false, st);
     }
-    {  // G2 = relu(G1 W4^T + b4)
-      tcg::Gemm g{};
-      g.A = Y + D; g.lda = 4 * D; g.ka = 4 * D - D;
-      g.B = W4; g.ldb = 2 * D; g.kb = 2 * D;
-      g.M = (int)T; g.N = D2; g.K = D; g.batch = 1; g.bn = pick_bn(D2);
-      set_passes(g, 2 * D, D);
-      g.bias = b4; g.act = tcg::ACT_RELU;
-      g.out[0] = {G2, tcg::OUT_BF16_HILO, (long long)2 * D2, 0, D2, 0, 0, 0};
-      if ((rc = tcg::launch(g, st))) return rc;
-    }
+    if (rc) return rc;
+    if ((rc = g1_layer(y.at(D), w4, b4, T, D, g2, st))) return rc;
     {  // Opre = G2 W5^T over all tokens: signed bf16 copy (sign carrier) and |.| as hi|lo planes; pad columns come out as zeros
-      tcg::Gemm g{};
-      g.A = G2; g.lda = 2 * D2; g.ka = 2 * D2;
-      g.B = W5; g.ldb = 2 * D2; g.kb = 2 * D2;
-      g.M = (int)T; g.N = P; g.K = D2; g.batch = 1; g.bn = pick_bn(P);
-      set_passes(g, D2, D2);
-      g.act = tcg::ACT_NONE;
-      g.out[0] = {OS, tcg::OUT_BF16, (long long)Pp, 0, 0, Pp, 0, 0};
-      if (!occ_only) g.out[1] = {OA, tcg::OUT_BF16_HILO, (long long)2 * Pp, 0, Pp, Pp, 1, 0};
+      tcg::Gemm g = gemm(g2, w5, (int)T, P, D2, 1, pick_bn(P));
+      g.out[0] = store(Planes{OS, Pp, 0, false}, Pp);
+      if (!occ_only) {
+        g.out[1] = store(oa, Pp);
+        g.out[1].absval = 1;
+      }
       if ((rc = tcg::launch(g, st))) return rc;
     }
     if (occ_only) {
@@ -909,22 +864,9 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       PASN_LAUNCH_CHECK();
       count_launch();
     } else {
-    {  // F = H1 W2^T + b2
-      tcg::Gemm g{};
-      g.A = Y; g.lda = 4 * D; g.ka = 4 * D;
-      g.B = W2; g.ldb = 2 * D; g.kb = 2 * D;
-      g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, 2 * D, D);
-      g.bias = b2;
-      g.out[0] = {F, tcg::OUT_BF16_HILO, (long long)2 * D, 0, D, 0, 0, 0};
-      if ((rc = tcg::launch(g, st))) return rc;
-    }
+    if ((rc = w2_layer(y, w2, b2, T, D, f, st))) return rc;
     {  // FE[n] = O[n]^T F[n]   (K = S; both operands token-major)
-      tcg::Gemm g{};
-      g.A = OA; g.lda = 2 * Pp; g.a_bs = (long long)S * 2 * Pp; g.a_batched = 1; g.ka = 2 * Pp; g.a_mn_major = 1; g.a_rows = S;
-      g.B = F; g.ldb = 2 * D; g.b_bs = (long long)S * 2 * D; g.b_batched = 1; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = S;
-      g.M = P; g.N = D; g.K = S; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, Pp, D);
+      tcg::Gemm g = pooling(oa.with((long long)S * oa.ld, S, true), S, f, P, D, S, nb);
       g.out[0] = {FE, tcg::OUT_F32, (long long)D, (long long)P * D, 0, 0, 0, 0};
       if ((rc = tcg::launch(g, st))) return rc;
     }
@@ -944,80 +886,56 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     }
     // ================= pooling backward
     {  // gOpre[n][s][p] = ((F[n] gFE[n]^T)[s][p] + gOcc[n][p][s]) * sign(Opre[n][s][p])
-      tcg::Gemm g{};
-      g.A = F; g.lda = 2 * D; g.a_bs = (long long)S * 2 * D; g.a_batched = 1; g.ka = 2 * D;
-      g.B = GFE; g.ldb = 2 * D; g.b_bs = (long long)P * 2 * D; g.b_batched = 1; g.kb = 2 * D;
-      g.M = S; g.N = P; g.K = D; g.batch = nb; g.bn = pick_bn(P);
-      set_passes(g, D, D);
+      tcg::Gemm g = gemm(f.with((long long)S * f.ld, 0, false), gfe.with((long long)P * gfe.ld, 0, false), S, P, D, nb, pick_bn(P));
       if (gOcc) g.addin = {gOcc + (size_t)n0 * P * S, 1, (long long)P * S, (long long)S};
       g.signin = {OS, (long long)Pp, (long long)S * Pp, 0};
-      g.out[0] = {GO, tcg::OUT_BF16_HILO, (long long)2 * Pp, (long long)S * 2 * Pp, Pp, Pp, 0, 0};
+      g.out[0] = store(go.with((long long)S * go.ld, 0, false), Pp);
       if ((rc = tcg::launch(g, st))) return rc;
     }
     {  // gF[n][s][d] = sum_p O[n][s][p] gFE[n][p][d]
-      tcg::Gemm g{};
-      g.A = OA; g.lda = 2 * Pp; g.a_bs = (long long)S * 2 * Pp; g.a_batched = 1; g.ka = 2 * Pp;
-      g.B = GFE; g.ldb = 2 * D; g.b_bs = (long long)P * 2 * D; g.b_batched = 1; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = P;
-      g.M = S; g.N = D; g.K = P; g.batch = nb; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, Pp, D);
-      g.out[0] = {GF, tcg::OUT_BF16_HILO, (long long)2 * D, (long long)S * 2 * D, D, 0, 0, 0};
+      tcg::Gemm g = gemm(oa.with((long long)S * oa.ld, 0, false), gfe.with((long long)P * gfe.ld, P, true), S, D, P, nb,
+                         D >= 256 ? 256 : 128);
+      g.out[0] = store(gf.with((long long)S * gf.ld, 0, false));
       if ((rc = tcg::launch(g, st))) return rc;
     }
     // ================= add-on branch
-    if ((rc = wgrad(GF, 2 * D, D, D, Y, 4 * D, 2 * D, true, D, T, gr.addon_w2, D, nullptr))) return rc;     // gW2 += gF^T H1
-    if ((rc = colsum(GF, T, 2 * D, D, D, gr.addon_b2, D, nullptr))) return rc;
+    if ((rc = wgrad(gf, D, y, D, T, gr.addon_w2, D, nullptr))) return rc;     // gW2 += gF^T H1
+    if ((rc = colsum(gf, T, D, gr.addon_b2, D, nullptr))) return rc;
     {  // gH1 = (gF W2) masked by H1 > 0   -> columns [0, D) of the [gH1 | gG1] planes
-      tcg::Gemm g{};
-      g.A = GF; g.lda = 2 * D; g.ka = 2 * D;
-      g.B = W2; g.ldb = 2 * D; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = D;
-      g.M = (int)T; g.N = D; g.K = D; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, D, D);
-      g.mask = {Y, (long long)4 * D, 0, 0};
-      g.out[0] = {GY, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, 0, 0, 0};
+      tcg::Gemm g = gemm(gf, w2.with(0, D, true), (int)T, D, D, 1, D >= 256 ? 256 : 128);
+      g.mask = {y.ptr, y.ld, 0, 0};
+      g.out[0] = store(gy);
       if ((rc = tcg::launch(g, st))) return rc;
     }
     }   // !occ_only
     // ================= occurrence branch
-    if ((rc = wgrad(GO, 2 * Pp, Pp, P, G2, 2 * D2, D2, true, D2, T, gr.occ_w3, P, nullptr))) return rc;      // gW5 += gOpre^T G2
+    if ((rc = wgrad(go, P, g2, D2, T, gr.occ_w3, P, nullptr))) return rc;      // gW5 += gOpre^T G2
     {  // gG2 = (gOpre W5) masked by G2 > 0
-      tcg::Gemm g{};
-      g.A = GO; g.lda = 2 * Pp; g.ka = 2 * Pp;
-      g.B = W5; g.ldb = 2 * D2; g.kb = 2 * D2; g.b_mn_major = 1; g.b_rows = P;
-      g.M = (int)T; g.N = D2; g.K = P; g.batch = 1; g.bn = pick_bn(D2);
-      set_passes(g, Pp, D2);
-      g.mask = {G2, (long long)2 * D2, 0, 0};
-      g.out[0] = {GG2, tcg::OUT_BF16_HILO, (long long)2 * D2, 0, D2, 0, 0, 0};
+      tcg::Gemm g = gemm(go, w5.with(0, P, true), (int)T, D2, P, 1, pick_bn(D2));
+      g.mask = {g2.ptr, g2.ld, 0, 0};
+      g.out[0] = store(gg2);
       if ((rc = tcg::launch(g, st))) return rc;
     }
-    if ((rc = wgrad(GG2, 2 * D2, D2, D2, Y + D, 4 * D, 2 * D, true, D, T, gr.occ_w2, D2, nullptr))) return rc;   // gW4 += gG2^T G1
-    if ((rc = colsum(GG2, T, 2 * D2, D2, D2, gr.occ_b2, D2, nullptr))) return rc;
+    if ((rc = wgrad(gg2, D2, y.at(D), D, T, gr.occ_w2, D2, nullptr))) return rc;   // gW4 += gG2^T G1
+    if ((rc = colsum(gg2, T, D2, gr.occ_b2, D2, nullptr))) return rc;
     {  // gG1 = (gG2 W4) masked by G1 > 0   -> columns [D, 2D) of the [gH1 | gG1] planes
-      tcg::Gemm g{};
-      g.A = GG2; g.lda = 2 * D2; g.ka = 2 * D2;
-      g.B = W4; g.ldb = 2 * D; g.kb = 2 * D; g.b_mn_major = 1; g.b_rows = D2;
-      g.M = (int)T; g.N = D; g.K = D2; g.batch = 1; g.bn = D >= 256 ? 256 : 128;
-      set_passes(g, D2, D);
-      g.mask = {Y + D, (long long)4 * D, 0, 0};
-      g.out[0] = {GY + D, tcg::OUT_BF16_HILO, (long long)4 * D, 0, 2 * D, D, 0, 0};
+      tcg::Gemm g = gemm(gg2, w4.with(0, D2, true), (int)T, D, D2, 1, D >= 256 ? 256 : 128);
+      g.mask = {y.at(D).ptr, y.ld, 0, 0};
+      g.out[0] = store(gy.at(D), D);
       if ((rc = tcg::launch(g, st))) return rc;
     }
     // ================= first layer: g[W1; W3] += [gH1 | gG1]^T X, biases, feature-map gradient
     if (occ_only) {
-      if ((rc = wgrad(GY + D, 4 * D, 2 * D, D, xt, ldx, C, x_lo, C, T, gr.occ_w1, D, nullptr))) return rc;
-      if ((rc = colsum(GY + D, T, 4 * D, 2 * D, D, gr.occ_b1, D, nullptr))) return rc;
+      if ((rc = wgrad(gy.at(D), D, xv, C, T, gr.occ_w1, D, nullptr))) return rc;
+      if ((rc = colsum(gy.at(D), T, D, gr.occ_b1, D, nullptr))) return rc;
     } else {
-      if ((rc = wgrad(GY, 4 * D, 2 * D, 2 * D, xt, ldx, C, x_lo, C, T, gr.addon_w1, D, gr.occ_w1))) return rc;
-      if ((rc = colsum(GY, T, 4 * D, 2 * D, 2 * D, gr.addon_b1, D, gr.occ_b1))) return rc;
+      if ((rc = wgrad(gy, 2 * D, xv, C, T, gr.addon_w1, D, gr.occ_w1))) return rc;
+      if ((rc = colsum(gy, T, 2 * D, gr.addon_b1, D, gr.occ_b1))) return rc;
     }
-    if (gX) {   // gX[n][c][s] = sum_o [gH1|gG1][n,s][o] [W1;W3][o][c]
-      tcg::Gemm g{};
-      g.A = GY; g.lda = 4 * D; g.ka = 4 * D;
-      g.B = W13; g.ldb = 2 * C; g.kb = 2 * C; g.b_mn_major = 1; g.b_rows = 2 * D;
-      g.M = (int)T; g.N = C; g.K = 2 * D; g.batch = 1; g.bn = C >= 256 ? 256 : (C >= 128 ? 128 : 64);
-      set_passes(g, 2 * D, C);
-      if (occ_only) {   // the G1 half alone: gG1 [W3]
-        g.A = GY + D; g.ka = 4 * D - D; g.B = W13 + (size_t)D * 2 * C; g.b_rows = D; g.K = D;
-      }
+    if (gX) {   // gX[n][c][s] = sum_o [gH1|gG1][n,s][o] [W1;W3][o][c]   (occurrence only: the G1 half alone, gG1 [W3])
+      const int bn = C >= 256 ? 256 : (C >= 128 ? 128 : 64);
+      tcg::Gemm g = occ_only ? gemm(gy.at(D), w13.row(D).with(0, D, true), (int)T, C, D, 1, bn)
+                             : gemm(gy, w13.with(0, 2 * D, true), (int)T, C, 2 * D, 1, bn);
       g.out[0] = {gX + (size_t)n0 * C * S, tcg::OUT_F32, (long long)S, (long long)C * S, 0, 0, 0, S};
       if ((rc = tcg::launch(g, st))) return rc;
     }
