@@ -16,6 +16,8 @@ namespace pasn {
 
 __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+// most clips one chunk of the generic or tiled path takes: kernels of both put the clip index in gridDim.y / z
+constexpr int kMaxChunkClips = 65535;
 
 // bytes per element of a feature / occurrence map of this pasn_dtype (the one place that knows the element sizes)
 __host__ __device__ inline size_t dtype_bytes(int dtype) { return dtype == PASN_F32 ? 4 : 2; }

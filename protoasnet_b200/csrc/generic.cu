@@ -183,9 +183,11 @@ int pool(const float* O, const float* F, float* FE, const pasn_dims& d, int nb, 
   return launch_gemm(g, false, st);
 }
 
-// clips per chunk when a clip needs per_clip bytes of scratch and the chunk may take cap bytes
+// clips per chunk when a clip needs per_clip bytes of scratch and the chunk may take cap bytes (at most kMaxChunkClips:
+// launch_gemm puts the clip index in gridDim.z)
 int chunk_clips(const pasn_dims& d, size_t per_clip, size_t cap) {
   long long c = (long long)(cap / (per_clip ? per_clip : 1));
+  if (c > kMaxChunkClips) c = kMaxChunkClips;
   if (c < 1) c = 1;
   if (c > d.N) c = d.N > 0 ? d.N : 1;
   return (int)c;
@@ -335,7 +337,6 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
   const float vnorm = sqrtf(bc[0]);
   const float nv = fmaxf(vnorm, eps);
   const bool v_clamped = !(vnorm > eps);
-  float gwl = 0.f;   // thread k < K accumulates gWl[k, p]
   for (int n = 0; n < nb; ++n) {
     const float* f = FE + ((size_t)n * P + p) * D;
     float ff = 0.f, dot = 0.f;
@@ -353,7 +354,9 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
     if (gLogits)
       for (int k = 0; k < K; ++k) gs = fmaf(gLogits[(size_t)n * K + k], last_layer[(size_t)k * P + p], gs);
     const float gcos = 0.5f * gs;
-    if (gLogits && tid < K) gwl = fmaf(gLogits[(size_t)n * K + tid], sim, gwl);
+    // the block owns column p of gWl: no other block writes it, so each clip adds its terms in place (any K)
+    if (gLogits)
+      for (int k = tid; k < K; k += 256) gWl[(size_t)k * P + p] += gLogits[(size_t)n * K + k] * sim;
     // cos = <f, v> / (nf nv); nf, nv constants when clamped
     const float inv = 1.0f / (nf * nv);
     const float cf = f_clamped ? 0.f : cosv / (nf * nf);
@@ -363,7 +366,6 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
       gV[(size_t)p * D + d] += gcos * (f[d] * inv - cv * v[d]);
     }
   }
-  if (gLogits && tid < K) gWl[(size_t)tid * P + p] += gwl;
 }
 
 // per-clip workspace of the backward (fp32); chunks bounded to ~384 MB

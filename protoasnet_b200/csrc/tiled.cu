@@ -41,10 +41,12 @@ struct Plan {
 inline int pick_bn(int n) { return n <= 64 ? 64 : (n <= 128 ? 128 : 256); }
 
 // clips per chunk of the forward / backward chain: as many as `budget` bytes of scratch hold at per_clip bytes each, at
-// least one, at most N.  PASN_TILED_CHUNK lowers the cap (tests force chunking with it).
+// least one, at most N, and at most kMaxChunkClips (several kernels put the clip index in gridDim.y / z).
+// PASN_TILED_CHUNK lowers the cap (tests force chunking with it).
 int clips_per_chunk(const pasn_dims& d, size_t budget, size_t per_clip) {
   static const int chunk_env = [] { const char* e = getenv("PASN_TILED_CHUNK"); return e ? atoi(e) : 0; }();
   long long nb = (long long)(budget / per_clip);
+  if (nb > kMaxChunkClips) nb = kMaxChunkClips;
   if (chunk_env > 0 && nb > chunk_env) nb = chunk_env;
   if (nb < 1) nb = 1;
   if (nb > d.N) nb = d.N > 0 ? d.N : 1;
@@ -685,11 +687,12 @@ __global__ void __launch_bounds__(256) proto_bwd_reduce_kernel(const float* __re
     for (int n = n_begin; n < n_end; ++n) acc = fmaf(rs[(size_t)n * P + p].x, FE[((size_t)n * P + p) * D + d], acc);
     atomicAdd(gV + (size_t)p * D + d, acc - sb * protos[(size_t)p * D + d]);
   }
-  if (gLogits && tid < K) {
-    float acc = 0.f;
-    for (int n = n_begin; n < n_end; ++n) acc = fmaf(gLogits[(size_t)n * K + tid], rs[(size_t)n * P + p].z, acc);
-    atomicAdd(gWl + (size_t)tid * P + p, acc);
-  }
+  if (gLogits)
+    for (int k = tid; k < K; k += 256) {
+      float acc = 0.f;
+      for (int n = n_begin; n < n_end; ++n) acc = fmaf(gLogits[(size_t)n * K + k], rs[(size_t)n * P + p].z, acc);
+      atomicAdd(gWl + (size_t)k * P + p, acc);
+    }
 }
 
 // dst[m][n] += sum_parts part[q][m][n]; rows >= rows0 continue in dst1 (stacked [W1; W3] gradient)

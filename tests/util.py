@@ -30,6 +30,12 @@ EMU_COSINE_PUSH = 2e-6        # float64 cosine chain on the kernel's own feature
                               # distance absolute, logits as a fraction of their scale                    (4.7e-7)
 EMU_COSINE_FWD = 2e-6         # ... vs forward() (which may take its cosine from row statistics of the pooling GEMM) (4.7e-7)
 
+# pasn_head_backward against float64 autograd on conditioned inputs (tests/test_backward_parity_gpu.py): max |got - ref|
+# over max |ref| of the feature-map gradient and of each of the eleven parameter gradients, per backward family.  Comments:
+# the worst value over the sweep at two seeds on one B200 at a 1000 W power limit (tools/bwd_parity_report.py).
+BWD_TILED_MAX = 1e-4          # tiled tensor-core chain (three-pass bf16 hi|lo GEMMs, fp32 accumulation)        (3.5e-5)
+BWD_GENERIC_MAX = 5e-5        # generic CUDA-core FFMA kernels: prototype / last-layer gradients summed in fp32
+                              # over 70 000 clips (2.1e-5); every shape with fewer than 100 clips stays at 1e-6  (9.7e-7)
 
 def occ_agreement(got, ref):
     """(fraction of entries bit-equal, worst entry in units of its allowance) of an occurrence map against the emulated
