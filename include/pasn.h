@@ -179,6 +179,25 @@ int pasn_head_backward(const void* feat, const pasn_weights* w, const pasn_dims*
                        const float* grad_similarity, const float* grad_occurrence, const pasn_grads* grads,
                        float* grad_feat, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Upstream gradients of every output of pasn_head_forward, each fp32 and optional (NULL: no gradient arrives through it). */
+typedef struct {
+  const float* grad_logits;     /* [N,K]                                                     */
+  const float* grad_similarity; /* [N,P]                                                     */
+  const float* grad_distance;   /* [N,P]   distance = 1 - similarity                         */
+  const float* grad_occurrence; /* [N,P,S]                                                   */
+  const float* grad_features;   /* [N,P,D] features_extracted                                */
+} pasn_upstream;
+/* Backward of Video_XProtoNet.push_forward (src/models/Video_XProtoNet.py:111-130; XProtoNet.py:87-106) and of forward:
+ * pasn_head_backward with every upstream gradient of the head (`up` non-NULL).  Same workspace
+ * (pasn_head_backward_workspace_bytes), kernel family, add-into-`grads` rule and channel-major fp32 grad_feat.  The
+ * distance gradient enters as minus a similarity gradient, the feature gradient is added to d(features_extracted) where
+ * the cosine's gradient forms it.  Occurrence-only mode (only the occurrence branch recomputed and differentiated, the
+ * other parameter gradients left untouched) is taken when grad_logits, grad_similarity, grad_distance and grad_features
+ * are all NULL.  pasn_head_backward(..., gl, gs, go, ...) is this call with {gl, gs, NULL, go, NULL}. */
+int pasn_head_backward_ex(const void* feat, const pasn_weights* w, const pasn_dims* dims, const pasn_upstream* up,
+                          const pasn_grads* grads, float* grad_feat, void* workspace, size_t workspace_bytes,
+                          void* stream);
+
 /* Loss / metric consumers of the head outputs, on the device (no per-step host round trip):
  *   class_max[n,k] / class_arg[n,k]  max (and global prototype index of the first maximum) of similarity over the
  *                                    prototypes of class k (P/K consecutive prototypes per class)

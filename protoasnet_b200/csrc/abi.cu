@@ -122,7 +122,13 @@ extern "C" size_t pasn_head_backward_workspace_bytes(const pasn_dims* dims) {
 extern "C" int pasn_head_backward(const void* feat, const pasn_weights* w, const pasn_dims* dims, const float* grad_logits,
                                   const float* grad_similarity, const float* grad_occurrence, const pasn_grads* grads,
                                   float* grad_feat, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!dims_ok(dims) || !w || !grads) return PASN_ERR_INVALID;
+  const pasn_upstream up{grad_logits, grad_similarity, nullptr, grad_occurrence, nullptr};
+  return pasn_head_backward_ex(feat, w, dims, &up, grads, grad_feat, workspace, workspace_bytes, stream);
+}
+extern "C" int pasn_head_backward_ex(const void* feat, const pasn_weights* w, const pasn_dims* dims, const pasn_upstream* up,
+                                     const pasn_grads* grads, float* grad_feat, void* workspace, size_t workspace_bytes,
+                                     void* stream) {
+  if (!dims_ok(dims) || !w || !up || !grads) return PASN_ERR_INVALID;
   if (!backward_ok(dims)) return PASN_ERR_UNSUPPORTED;
   if (faulted()) return PASN_ERR_FAULT;
   if (dims->N == 0) return PASN_OK;
@@ -131,8 +137,7 @@ extern "C" int pasn_head_backward(const void* feat, const pasn_weights* w, const
   for (int i = 0; i < 11; ++i)
     if (!gp[i]) return PASN_ERR_INVALID;
   auto backward = tiled_backward_supported(*dims) ? tiled_head_backward : generic_head_backward;
-  return backward(feat, *w, *dims, grad_logits, grad_similarity, grad_occurrence, *grads, grad_feat, workspace,
-                  workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  return backward(feat, *w, *dims, *up, *grads, grad_feat, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int pasn_debug_sm100_error(const void* workspace, const pasn_dims* dims, void* stream) {

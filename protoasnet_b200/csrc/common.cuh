@@ -104,8 +104,8 @@ int generic_occurrence_only(const void* feat, const pasn_weights& w, const pasn_
                             size_t ws_bytes, cudaStream_t st);
 // backward on the CUDA cores: fp32 / bf16 feature maps, any shape; the shapes tiled_backward_supported() rejects
 size_t generic_backward_workspace_bytes(const pasn_dims& d);
-int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
-                          const float* gOcc, const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
+int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const pasn_upstream& up,
+                          const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // ---- prototype stage (proto_stage.cu): cosine -> (.+1)/2 -> logits -> 1-s -> running argmin keys ----
 int launch_proto_stage(const float* feats /*[N,P,D]*/, const float* protos, const float* last_layer, int N, int P,
@@ -132,8 +132,8 @@ int tiled_occurrence_only(const void* feat, const pasn_weights& w, const void* p
 // dims.path asks for the generic CUDA-core kernels
 bool tiled_backward_supported(const pasn_dims& d);
 size_t tiled_backward_workspace_bytes(const pasn_dims& d);
-int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
-                        const float* gOcc, const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
+int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const pasn_upstream& up,
+                        const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // ---- fused tcgen05 path (head_sm100.cu) -----------------------------------------------------
 bool sm100_supported(const pasn_dims& d);

@@ -17,6 +17,7 @@
 // d|x|/dx at 0 = 0, CosineSimilarity clamps each norm at eps = 1e-8 (a clamped norm is a constant).
 //   H1 = relu(W1 x + b1), F = W2 H1 + b2, G1 = relu(W3 x + b3), G2 = relu(W4 G1 + b4), Opre = W5 G2, O = |Opre|
 //   FE[p,:] = sum_s O[p,s] F[:,s];  cos = <FE/nf, v/nv>;  sim = (cos+1)/2;  logits = sim Wl^T
+// push_forward's extra outputs, features_extracted = FE and distance = 1 - sim, pass their gradients in at gFE and gsim.
 // bf16 feature maps are read exactly (converted to fp32); weights are used unrounded: this is the gradient of the fp32
 // formulation, which is also what the reference's autograd computes.
 #include "common.cuh"
@@ -308,11 +309,12 @@ __global__ void sign_kernel(float* __restrict__ gO, const float* __restrict__ gO
 }
 
 // Cosine / similarity / logits backward.  One block per prototype p, looping over the clips of the chunk:
-//   gsim = gSim[n,p] + sum_k gLogits[n,k] Wl[k,p];  gcos = gsim / 2
-//   gFE[n,p,:], gV[p,:] += ..., gWl[k,p] += gLogits[n,k] * sim[n,p]
+//   gsim = gSim[n,p] - gDist[n,p] + sum_k gLogits[n,k] Wl[k,p];  gcos = gsim / 2
+//   gFE[n,p,:] = (cosine's gradient) + gFEin[n,p,:], gV[p,:] += ..., gWl[k,p] += gLogits[n,k] * sim[n,p]
 __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict__ FE, const float* __restrict__ protos,
                                                         const float* __restrict__ last_layer, const float* __restrict__ gLogits,
-                                                        const float* __restrict__ gSim, int nb, int P, int D, int K,
+                                                        const float* __restrict__ gSim, const float* __restrict__ gDist,
+                                                        const float* __restrict__ gFEin, int nb, int P, int D, int K,
                                                         float* __restrict__ gFE, float* __restrict__ gV, float* __restrict__ gWl) {
   __shared__ float red[3][8];
   __shared__ float bc[3];
@@ -351,6 +353,7 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
     const float cosv = bc[1] / (nf * nv);
     const float sim = (cosv + 1.0f) * 0.5f;
     float gs = gSim ? gSim[(size_t)n * P + p] : 0.f;
+    if (gDist) gs -= gDist[(size_t)n * P + p];
     if (gLogits)
       for (int k = 0; k < K; ++k) gs = fmaf(gLogits[(size_t)n * K + k], last_layer[(size_t)k * P + p], gs);
     const float gcos = 0.5f * gs;
@@ -361,8 +364,11 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
     const float inv = 1.0f / (nf * nv);
     const float cf = f_clamped ? 0.f : cosv / (nf * nf);
     const float cv = v_clamped ? 0.f : cosv / (nv * nv);
+    const size_t row = ((size_t)n * P + p) * D;
     for (int d = tid; d < D; d += 256) {
-      gFE[((size_t)n * P + p) * D + d] = gcos * (v[d] * inv - cf * f[d]);
+      float gf = gcos * (v[d] * inv - cf * f[d]);
+      if (gFEin) gf += gFEin[row + d];
+      gFE[row + d] = gf;
       gV[(size_t)p * D + d] += gcos * (f[d] * inv - cv * v[d]);
     }
   }
@@ -379,9 +385,11 @@ int bwd_chunk(const pasn_dims& d) { return chunk_clips(d, bwd_per_clip(d), (size
 
 size_t generic_backward_workspace_bytes(const pasn_dims& d) { return align_up(bwd_per_clip(d) * bwd_chunk(d), 256) + 256; }
 
-int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
-                          const float* gOcc, const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st) {
+int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const pasn_upstream& up,
+                          const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (ws_bytes < generic_backward_workspace_bytes(d)) return PASN_ERR_WORKSPACE;
+  const float *gLogits = up.grad_logits, *gSim = up.grad_similarity, *gDist = up.grad_distance, *gOcc = up.grad_occurrence,
+              *gFEin = up.grad_features;
   const int nbm = bwd_chunk(d);
   const int D = d.D, D2 = d.D / 2, S = d.S, P = d.P, C = d.C, K = d.K;
   const size_t DS = (size_t)D * S, D2S = (size_t)D2 * S, PS = (size_t)P * S, PD = (size_t)P * D;
@@ -436,7 +444,8 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
     if ((rc = pool(O, F, FE, d, nb, st))) return rc;
     // ---- prototype stage backward
     proto_bwd_kernel<<<P, 256, 0, st>>>(FE, w.prototypes, w.last_layer, gLogits ? gLogits + (size_t)n0 * K : nullptr,
-                                        gSim ? gSim + (size_t)n0 * P : nullptr, nb, P, D, K, gFE, g.prototypes, g.last_layer);
+                                        gSim ? gSim + (size_t)n0 * P : nullptr, gDist ? gDist + (size_t)n0 * P : nullptr,
+                                        gFEin ? gFEin + (size_t)n0 * PD : nullptr, nb, P, D, K, gFE, g.prototypes, g.last_layer);
     PASN_LAUNCH_CHECK();
     count_launch();
     {  // gO[b][p][s] = sum_d gFE[b][p][d] F[b][d][s]

@@ -623,12 +623,14 @@ BPlan make_bplan(const pasn_dims& d) {
 }
 
 // prototype stage backward, part 1: one warp per (clip, prototype) row.
-//   gs = gSim + sum_k gLogits[n,k] Wl[k,p];  gcos = gs / 2;  cos = <f,v> / (nf nv) with each norm clamped at eps (a clamped
-//   norm is a constant);  gFE = gcos (v / (nf nv) - cos f / nf^2)  -> bf16 hi|lo planes (operand of the next GEMMs);
+//   gs = gSim - gDist + sum_k gLogits[n,k] Wl[k,p];  gcos = gs / 2;  cos = <f,v> / (nf nv) with each norm clamped at eps (a
+//   clamped norm is a constant);  gFE = gcos (v / (nf nv) - cos f / nf^2) + gFEin (the upstream d(features_extracted)), in
+//   fp32, -> bf16 hi|lo planes (operand of the next GEMMs);
 //   row scalars for part 2: a = gcos / (nf nv), b = gcos cos / nv^2 (0 when nv is clamped), sim
 __global__ void __launch_bounds__(256) proto_bwd_rows_kernel(const float* __restrict__ FE, const float* __restrict__ protos,
                                                              const float* __restrict__ last_layer, const float* __restrict__ gLogits,
-                                                             const float* __restrict__ gSim, long long rows, int P, int D, int K,
+                                                             const float* __restrict__ gSim, const float* __restrict__ gDist,
+                                                             const float* __restrict__ gFEin, long long rows, int P, int D, int K,
                                                              __nv_bfloat16* __restrict__ gfe, float4* __restrict__ rs) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr float eps = 1e-8f;
@@ -648,14 +650,17 @@ __global__ void __launch_bounds__(256) proto_bwd_rows_kernel(const float* __rest
     const float inv = 1.0f / (nf * nv);
     const float cosv = dot * inv;
     float gs = gSim ? gSim[r] : 0.f;
+    if (gDist) gs -= gDist[r];
     if (gLogits)
       for (int k = 0; k < K; ++k) gs = fmaf(gLogits[(size_t)n * K + k], last_layer[(size_t)k * P + p], gs);
     const float gcos = 0.5f * gs;
     const float cf = (fnorm > eps) ? cosv / (nf * nf) : 0.f;
     const float cv = (vnorm > eps) ? cosv / (nv * nv) : 0.f;
     __nv_bfloat16* grow = gfe + (size_t)r * 2 * D;
+    const float* gin = gFEin ? gFEin + (size_t)r * D : nullptr;
     for (int d = lane; d < D; d += 32) {
-      const float gv = gcos * (v[d] * inv - cf * f[d]);
+      float gv = gcos * (v[d] * inv - cf * f[d]);
+      if (gin) gv += gin[d];
       const __nv_bfloat16 hi = __float2bfloat16_rn(gv);
       grow[d] = hi;
       grow[D + d] = __float2bfloat16_rn(gv - __bfloat162float(hi));
@@ -769,8 +774,10 @@ __global__ void __launch_bounds__(256) gopre_from_gocc_kernel(const float* __res
 bool tiled_backward_supported(const pasn_dims& d) { return tiled_supported(d) && d.path != PASN_PATH_GENERIC; }
 size_t tiled_backward_workspace_bytes(const pasn_dims& d) { return make_bplan(d).total; }
 
-int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const float* gLogits, const float* gSim,
-                        const float* gOcc, const pasn_grads& gr, float* gX, void* ws_, size_t ws_bytes, cudaStream_t st) {
+int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const pasn_upstream& up,
+                        const pasn_grads& gr, float* gX, void* ws_, size_t ws_bytes, cudaStream_t st) {
+  const float *gLogits = up.grad_logits, *gSim = up.grad_similarity, *gDist = up.grad_distance, *gOcc = up.grad_occurrence,
+              *gFEin = up.grad_features;
   const BPlan b = make_bplan(d);
   if (ws_bytes < b.total) return PASN_ERR_WORKSPACE;
   if (((uintptr_t)ws_ & 255) != 0) return PASN_ERR_ALIGN;
@@ -799,9 +806,9 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
   float* PART = reinterpret_cast<float*>(ws + b.off_part);
   const size_t elt = dtype_bytes(d.dtype);
   const bool x_lo = xe == 2;
-  // No gradient arrives through logits / similarity: backward of compute_occurence_map alone (TransformLoss re-entry,
-  // src/loss/loss.py:302) -- only the occurrence branch is recomputed and differentiated.
-  const bool occ_only = gLogits == nullptr && gSim == nullptr;
+  // No gradient arrives through logits, similarity, distance or the pooled features: backward of compute_occurence_map
+  // alone (TransformLoss re-entry, src/loss/loss.py:302) -- only the occurrence branch is recomputed and differentiated.
+  const bool occ_only = gLogits == nullptr && gSim == nullptr && gDist == nullptr && gFEin == nullptr;
   if (occ_only && gOcc == nullptr) {
     if (gX) cudaMemsetAsync(gX, 0, (size_t)d.N * C * S * 4, st);
     return PASN_OK;
@@ -879,7 +886,8 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
       long long blocks = (rows + 7) / 8;
       if (blocks > 148 * 16) blocks = 148 * 16;
       proto_bwd_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(FE, w.prototypes, w.last_layer, gLogits ? gLogits + (size_t)n0 * d.K : nullptr,
-                                                              gSim ? gSim + (size_t)n0 * P : nullptr, rows, P, D, d.K, GFE, RS);
+                                                              gSim ? gSim + (size_t)n0 * P : nullptr, gDist ? gDist + (size_t)n0 * P : nullptr,
+                                                              gFEin ? gFEin + (size_t)n0 * P * D : nullptr, rows, P, D, d.K, GFE, RS);
       PASN_LAUNCH_CHECK();
       count_launch();
       proto_bwd_reduce_kernel<<<dim3(P, nb >= 64 ? 16 : 1), 256, 0, st>>>(FE, w.prototypes, gLogits ? gLogits + (size_t)n0 * d.K : nullptr, RS, nb, P, D, d.K,

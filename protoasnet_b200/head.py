@@ -10,10 +10,11 @@ Reference interface being mirrored (paths relative to the reference checkout):
 
 The backbone stays PyTorch (north_star); everything from its feature map to the logits runs in the CUDA
 library.  There is NO PyTorch/CPU fallback for inference: a CPU tensor, or a missing library, raises.
-Training through the head (SURVEY.md section 8f row 2): ``autograd_mode='kernel'`` runs ``requires_grad`` calls
-through the library as well (forward as usual, backward = ``pasn_head_backward``, fp32 CUDA-core kernels that
-recompute the forward intermediates); ``'composite'`` opts in to a differentiable PyTorch composite of the same maths
-on the GPU; the default ``'error'`` refuses instead of silently switching.
+Training through the head (SURVEY.md section 8f row 2): ``autograd_mode='kernel'`` runs ``requires_grad`` calls of
+forward(), push_forward(), compute_occurence_map() and get_occurence_map_absolute_val() through the library as well
+(forward as usual, backward = ``pasn_head_backward_ex``, kernels that recompute the forward intermediates);
+``'composite'`` opts in to a differentiable PyTorch composite of the same maths on the GPU; the default ``'error'``
+refuses instead of silently switching.
 """
 from __future__ import annotations
 
@@ -26,7 +27,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib
-from ._lib import PasnDims, PasnGrads, PasnPushArgs, PasnWeights
+from ._lib import PasnDims, PasnGrads, PasnPushArgs, PasnUpstream, PasnWeights
 
 
 import os as _os
@@ -175,9 +176,17 @@ class _HeadRuntime:
         return occ
 
 
-def _library_backward(rt, x, g_logits, g_sim, g_occ, want_gx):
-    """pasn_head_backward on (x, head parameters): returns (grad_x or None, [11 parameter gradients]).  With g_logits and
-    g_sim both None only the occurrence branch is differentiated (compute_occurence_map)."""
+# the outputs of the head's forward whose gradients pasn_upstream carries, and its field for each
+_UPSTREAM = {"logits": "grad_logits", "similarity": "grad_similarity", "distance": "grad_distance",
+             "occurrence_map": "grad_occurrence", "features_extracted": "grad_features"}
+_FORWARD_OUTPUTS = ("logits", "similarity", "occurrence_map")                           # forward()
+_PUSH_OUTPUTS = ("features_extracted", "distance", "occurrence_map", "logits")          # push_forward()
+
+
+def _library_backward(rt, x, upstream: Dict[str, Optional[torch.Tensor]], want_gx):
+    """pasn_head_backward_ex on (x, head parameters): returns (grad_x or None, [11 parameter gradients]).  ``upstream``
+    maps output names (the keys of _UPSTREAM) to their gradients; a missing or None entry contributes nothing.  When the
+    occurrence map's is the only one, only the occurrence branch is differentiated (compute_occurence_map)."""
     lib = _lib.load()
     m = rt.owner
     dims, xc, spatial = rt.make_dims(x, m.kernel_path)   # GENERIC keeps the CUDA-core backward, anything else lets the
@@ -194,15 +203,17 @@ def _library_backward(rt, x, g_logits, g_sim, g_occ, want_gx):
                 return None
             return g.to(torch.float32).reshape(shape).contiguous()
 
-        gl = prep(g_logits, (dims.N, dims.K))
-        gs = prep(g_sim, (dims.N, dims.P))
-        go = prep(g_occ, (dims.N, dims.P, dims.S))
+        N, P = dims.N, dims.P
+        shapes = {"logits": (N, dims.K), "similarity": (N, P), "distance": (N, P), "occurrence_map": (N, P, dims.S),
+                  "features_extracted": (N, P, dims.D)}
+        gup = {k: prep(upstream.get(k), shapes[k]) for k in _UPSTREAM}
+        up = PasnUpstream(**{_UPSTREAM[k]: _ptr(t) for k, t in gup.items()})
         if dims.N > 0:
             need = int(lib.pasn_head_backward_workspace_bytes(C.byref(dims)))
             ws = torch.empty(max(need, 256), dtype=torch.uint8, device=dev)
-            st = lib.pasn_head_backward(xc.data_ptr(), C.byref(w), C.byref(dims), _ptr(gl), _ptr(gs), _ptr(go),
-                                        C.byref(gw), _ptr(gx), ws.data_ptr(), ws.numel(), stream)
-            _lib.check(st, "pasn_head_backward")
+            st = lib.pasn_head_backward_ex(xc.data_ptr(), C.byref(w), C.byref(dims), C.byref(up), C.byref(gw), _ptr(gx),
+                                           ws.data_ptr(), ws.numel(), stream)
+            _lib.check(st, "pasn_head_backward_ex")
         elif gx is not None:
             gx.zero_()
     if gx is not None:
@@ -217,7 +228,8 @@ def _param_grads(grads, params, needed) -> tuple:
 class _OccFunction(torch.autograd.Function):
     """(features, occurrence_module parameters) -> occurrence_map with gradients: compute_occurence_map under grad, which
     the reference's TransformLoss calls once more per training step (src/loss/loss.py:302).  Forward = the library's
-    occurrence-only path, backward = pasn_head_backward with no logits / similarity gradient (occurrence branch only)."""
+    occurrence-only path, backward = pasn_head_backward_ex with the occurrence map's gradient alone (occurrence branch
+    only)."""
 
     @staticmethod
     def forward(ctx, rt, x, *params):
@@ -230,27 +242,28 @@ class _OccFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_occ):
         x, *params = ctx.saved_tensors
-        gx, grads = _library_backward(ctx.rt, x, None, None, g_occ, ctx.needs_input_grad[1])
+        gx, grads = _library_backward(ctx.rt, x, {"occurrence_map": g_occ}, ctx.needs_input_grad[1])
         return (None, gx) + _param_grads(grads[_OCC_PARAMS], params, ctx.needs_input_grad[2:])
 
 
 class _HeadFunction(torch.autograd.Function):
-    """(features, 11 head parameters) -> (logits, similarity, occurrence_map): forward through the library's usual path,
-    backward through ``pasn_head_backward`` (fp32 CUDA-core kernels, forward intermediates recomputed)."""
+    """(features, 11 head parameters) -> the head outputs named by ``outputs`` (_FORWARD_OUTPUTS: forward()'s, or
+    _PUSH_OUTPUTS: push_forward()'s): forward through the library's usual path, backward through
+    ``pasn_head_backward_ex`` with the gradient of every returned output (forward intermediates recomputed)."""
 
     @staticmethod
-    def forward(ctx, rt, x, *params):
+    def forward(ctx, rt, outputs, x, *params):
         with torch.no_grad():
-            r = rt.run(x, want_occ=True)
-        ctx.rt = rt
+            r = rt.run(x, want_occ=True, want_feats="features_extracted" in outputs, want_dist="distance" in outputs)
+        ctx.rt, ctx.outputs = rt, outputs
         ctx.save_for_backward(x, *params)
-        return r["logits"], r["similarity"], r["occurrence_map"]
+        return tuple(r[k] for k in outputs)
 
     @staticmethod
-    def backward(ctx, g_logits, g_sim, g_occ):
+    def backward(ctx, *grads):
         x, *params = ctx.saved_tensors
-        gx, grads = _library_backward(ctx.rt, x, g_logits, g_sim, g_occ, ctx.needs_input_grad[1])
-        return (None, gx) + _param_grads(grads, params, ctx.needs_input_grad[2:])
+        gx, g = _library_backward(ctx.rt, x, dict(zip(ctx.outputs, grads)), ctx.needs_input_grad[2])
+        return (None, None, gx) + _param_grads(g, params, ctx.needs_input_grad[3:])
 
 
 class HostPipeline:
@@ -442,9 +455,9 @@ class PrototypeHeadMixin:
                 "composite of the head) to train.")
         return False
 
-    def _kernel_autograd(self, x):
-        """(logits, similarity, occurrence_map) with gradients flowing through pasn_head_backward."""
-        return _HeadFunction.apply(self._rt, x, *_head_params(self))
+    def _kernel_autograd(self, x, outputs=_FORWARD_OUTPUTS):
+        """The head outputs named by ``outputs`` with gradients flowing through pasn_head_backward_ex."""
+        return _HeadFunction.apply(self._rt, outputs, x, *_head_params(self))
 
     # ---- reference API ----
     def forward(self, x):
@@ -460,15 +473,13 @@ class PrototypeHeadMixin:
 
     def compute_occurence_map(self, x):
         """-> occurrence_map [N,P,1,(T),H,W].  Video_XProtoNet.py:100-109."""
-        x = self.cnn_backbone(x)
+        return self.get_occurence_map_absolute_val(self.cnn_backbone(x))
+
+    def get_occurence_map_absolute_val(self, x):
+        """compute_occurence_map on a backbone feature map.  Video_XProtoNet.py:106-109."""
         if self._grad_guard(x):
             if self.autograd_mode == "kernel":
                 return _OccFunction.apply(self._rt, x, *_head_params(self)[_OCC_PARAMS])
-            return torch.abs(self.occurrence_module(x)).unsqueeze(2)
-        return self._rt.occurrence_only(x)
-
-    def get_occurence_map_absolute_val(self, x):
-        if self._grad_guard(x):
             return torch.abs(self.occurrence_module(x)).unsqueeze(2)
         return self._rt.occurrence_only(x)
 
@@ -476,6 +487,8 @@ class PrototypeHeadMixin:
         """-> (features_extracted [N,P,D], 1 - similarity [N,P], occurrence_map, logits).  Video_XProtoNet.py:111-130."""
         x = self.cnn_backbone(x)
         if self._grad_guard(x):
+            if self.autograd_mode == "kernel":
+                return self._kernel_autograd(x, _PUSH_OUTPUTS)
             feats, sim, occ, logits = self._composite(x)
             return feats, 1 - sim, occ, logits
         r = self._rt.run(x, want_occ=True, want_feats=True, want_dist=True)

@@ -1,23 +1,75 @@
-"""Forward + backward of the head through the library at the cfg-3 shape (autograd_mode='kernel')."""
-import os, sys
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+"""Forward + backward of the head at the cfg-3 shape (fp32 feature map), through the library (autograd_mode='kernel')
+against the PyTorch composite, for forward() and push_forward(); the two modes alternate within one process.  Prints
+the card and its power limit first, then per (N, method, mode) the median step time over the repetitions.
+
+    python tools/time_backward.py [--n 64 256] [--reps 5] [--iters 20]
+"""
+import argparse
+import os
+import subprocess
+import sys
+
 import torch
-from protoasnet_b200 import synth
-from tests.util import build_model
-dims = synth.CONFIGS["cfg3_video_b1024"]
-sd = synth.make_head_params(dims, seed=200, bias_scale=0.02, bf16_round=True)
-for n in (64, 256):
-    for mode in ("kernel", "composite"):
-        m = build_model(dims, sd); m.autograd_mode = mode
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from protoasnet_b200 import synth  # noqa: E402
+from tests.util import build_model  # noqa: E402
+
+
+def _time(fn, iters):
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+    ev[0].record()
+    for _ in range(iters):
+        fn()
+    ev[1].record()
+    torch.cuda.synchronize()
+    return ev[0].elapsed_time(ev[1]) / iters
+
+
+def _loss(method, m, x):
+    """A loss on every output the method returns."""
+    if method == "forward":
+        logits, sim, occ = m(x)
+        return logits.sum() + sim.sum() + occ.float().abs().sum() * 1e-4
+    feats, dist, occ, logits = m.push_forward(x)
+    return feats.sum() * 1e-4 + dist.sum() + occ.float().abs().sum() * 1e-4 + logits.sum()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--n", type=int, nargs="+", default=[64, 256])
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--iters", type=int, default=20)
+    a = ap.parse_args()
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True).stdout.strip()
+    print(f"card: {q or torch.cuda.get_device_name()}")
+    dims = synth.CONFIGS["cfg3_video_b1024"]
+    sd = synth.make_head_params(dims, seed=200, bias_scale=0.02, bf16_round=True)
+    models = {mode: build_model(dims, sd) for mode in ("kernel", "composite")}
+    for mode, m in models.items():
+        m.autograd_mode = mode
+    for n in a.n:
         x = torch.relu(torch.randn((n, dims.C) + dims.spatial, device="cuda"))
-        def step():
-            for p in m.parameters(): p.grad = None
-            logits, sim, occ = m(x)
-            (logits.sum() + sim.sum() + occ.float().abs().sum() * 1e-4).backward()
-        for _ in range(2): step()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(5): step()
-        e1.record(); torch.cuda.synchronize()
-        print(f"N={n} {mode}: fwd+bwd {e0.elapsed_time(e1)/5:.2f} ms")
+        for method in ("forward", "push_forward"):
+            def step(m):
+                for p in m.parameters():
+                    p.grad = None
+                _loss(method, m, x).backward()
+
+            for m in models.values():   # warm-up (weight packing, module loads, cuDNN algorithm choice)
+                for _ in range(3):
+                    step(m)
+            torch.cuda.synchronize()
+            res = {mode: [] for mode in models}
+            for _ in range(a.reps):
+                for mode, m in models.items():
+                    res[mode].append(_time(lambda: step(m), a.iters))
+            med = {mode: sorted(r)[len(r) // 2] for mode, r in res.items()}
+            print(f"N={n} {method}: fwd+bwd " + ", ".join(
+                f"{mode} {med[mode]:.3f} ms (min {min(res[mode]):.3f}, max {max(res[mode]):.3f})" for mode in models) +
+                f" | kernel/composite {med['kernel'] / med['composite']:.3f}", flush=True)
+
+
+if __name__ == "__main__":
+    main()
