@@ -167,8 +167,12 @@ int pasn_occurrence_only(const void* feat, const pasn_weights* w, const void* pa
  * workspace size of 0 otherwise).  grad_logits = grad_similarity = NULL: only the occurrence branch is recomputed
  * and differentiated (backward of pasn_occurrence_only); the other parameter gradients are left untouched.
  *   grad_logits      [N,K] fp32 or NULL     grad_similarity [N,P] fp32 or NULL     grad_occurrence [N,P,S] fp32 or NULL
- *   grads            every pointer non-NULL, same shapes as pasn_weights; gradients are ADDED to the buffers
- *   grad_feat        [N,C,S] fp32 (always channel-major, whatever dims.layout says about feat), or NULL           */
+ *   grads            required; same shapes as pasn_weights; gradients are ADDED to the buffers.  A NULL member is not
+ *                    wanted: it is neither computed nor written, and work that serves only unwanted gradients is
+ *                    skipped (e.g. prototypes / last_layer alone: the forward recompute and the prototype stage, no
+ *                    pooling or branch backward).  A wanted gradient is computed the same way whatever else is wanted.
+ *                    Every member NULL and grad_feat NULL: PASN_OK, nothing launched.
+ *   grad_feat        [N,C,S] fp32 (always channel-major, whatever dims.layout says about feat), or NULL (not wanted) */
 typedef struct {
   float* addon_w1; float* addon_b1; float* addon_w2; float* addon_b2;
   float* occ_w1; float* occ_b1; float* occ_w2; float* occ_b2; float* occ_w3;
@@ -197,6 +201,13 @@ typedef struct {
 int pasn_head_backward_ex(const void* feat, const pasn_weights* w, const pasn_dims* dims, const pasn_upstream* up,
                           const pasn_grads* grads, float* grad_feat, void* workspace, size_t workspace_bytes,
                           void* stream);
+/* Backward of the last layer alone (a training stage with every other head parameter and the feature map frozen):
+ *   grad_last_layer[k][p] += sum_n grad_logits[n][k] * similarity[n][p]
+ * grad_logits [N,K] fp32, similarity [N,P] fp32 as pasn_head_forward returned it (no recompute, no workspace), grad_last_layer
+ * [K,P] fp32.  One CUDA-core FFMA GEMM whose output tiles are each summed by one block over all N: bit-identical from call
+ * to call.  N = 0: no-op. */
+int pasn_last_layer_backward(const float* grad_logits, const float* similarity, int32_t N, int32_t P, int32_t K,
+                             float* grad_last_layer, void* stream);
 
 /* Loss / metric consumers of the head outputs, on the device (no per-step host round trip):
  *   class_max[n,k] / class_arg[n,k]  max (and global prototype index of the first maximum) of similarity over the

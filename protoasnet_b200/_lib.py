@@ -27,7 +27,8 @@ SYMBOLS = [
     "pasn_push_merge_peers", "pasn_push_capture",
     "pasn_debug_launch_count", "pasn_debug_time_main_kernel", "pasn_debug_last_main_kernel_ms",
     "pasn_debug_sm100_error", "pasn_debug_set_trace", "pasn_debug_fault", "pasn_debug_set_fault",
-    "pasn_head_backward_workspace_bytes", "pasn_head_backward", "pasn_head_backward_ex", "pasn_similarity_stats",
+    "pasn_head_backward_workspace_bytes", "pasn_head_backward", "pasn_head_backward_ex", "pasn_last_layer_backward",
+    "pasn_similarity_stats",
     "pasn_occurrence_lnorm",
     "pasn_debug_tc_gemm_desc_bytes", "pasn_debug_tc_gemm", "pasn_debug_set_gemm_trace",
 ]
@@ -132,6 +133,8 @@ def load() -> C.CDLL:
     lib.pasn_head_backward_ex.restype = C.c_int
     lib.pasn_head_backward_ex.argtypes = [vp, C.POINTER(PasnWeights), C.POINTER(PasnDims), C.POINTER(PasnUpstream),
                                           C.POINTER(PasnGrads), vp, vp, C.c_size_t, vp]
+    lib.pasn_last_layer_backward.restype = C.c_int
+    lib.pasn_last_layer_backward.argtypes = [vp, vp, i32, i32, i32, vp, vp]
     lib.pasn_similarity_stats.restype = C.c_int
     lib.pasn_similarity_stats.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                           vp, vp, vp, vp, vp, vp]

@@ -132,12 +132,19 @@ extern "C" int pasn_head_backward_ex(const void* feat, const pasn_weights* w, co
   if (!backward_ok(dims)) return PASN_ERR_UNSUPPORTED;
   if (faulted()) return PASN_ERR_FAULT;
   if (dims->N == 0) return PASN_OK;
+  if (!bwd_needs(*grads, grad_feat).proto) return PASN_OK;   // no gradient wanted: no work
   if (!feat || !workspace) return PASN_ERR_INVALID;
-  const float* const* gp = reinterpret_cast<const float* const*>(grads);
-  for (int i = 0; i < 11; ++i)
-    if (!gp[i]) return PASN_ERR_INVALID;
   auto backward = tiled_backward_supported(*dims) ? tiled_head_backward : generic_head_backward;
   return backward(feat, *w, *dims, *up, *grads, grad_feat, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int pasn_last_layer_backward(const float* grad_logits, const float* similarity, int32_t N, int32_t P, int32_t K,
+                                        float* grad_last_layer, void* stream) {
+  if (N < 0 || P <= 0 || K <= 0) return PASN_ERR_INVALID;
+  if (faulted()) return PASN_ERR_FAULT;
+  if (N == 0) return PASN_OK;
+  if (!grad_logits || !similarity || !grad_last_layer) return PASN_ERR_INVALID;
+  return generic_last_layer_backward(grad_logits, similarity, N, P, K, grad_last_layer, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int pasn_debug_sm100_error(const void* workspace, const pasn_dims* dims, void* stream) {

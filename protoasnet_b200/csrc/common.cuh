@@ -106,6 +106,25 @@ int generic_occurrence_only(const void* feat, const pasn_weights& w, const pasn_
 size_t generic_backward_workspace_bytes(const pasn_dims& d);
 int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_dims& d, const pasn_upstream& up,
                           const pasn_grads& g, float* gX, void* ws, size_t ws_bytes, cudaStream_t st);
+// gWl[k][p] += sum_n gL[n][k] sim[n][p] (one FFMA GEMM, each output tile summed by one block: deterministic)
+int generic_last_layer_backward(const float* gL, const float* sim, int N, int P, int K, float* gWl, cudaStream_t st);
+
+// Which intermediate gradients of the head's backward some wanted output depends on.  A NULL member of pasn_grads (or a
+// NULL grad_feat) is not wanted, and work that serves only unwanted outputs is skipped; both backward families prune by
+// this table.  Every wanted output depends on the prototype stage, so `proto` is false exactly when nothing is wanted.
+struct BwdNeeds {
+  bool gH1, gF, gG1, gG2, gOpre, proto;
+};
+inline BwdNeeds bwd_needs(const pasn_grads& g, const float* gX) {
+  BwdNeeds n;
+  n.gH1 = g.addon_w1 || g.addon_b1 || gX;
+  n.gF = g.addon_w2 || g.addon_b2 || n.gH1;
+  n.gG1 = g.occ_w1 || g.occ_b1 || gX;
+  n.gG2 = g.occ_w2 || g.occ_b2 || n.gG1;
+  n.gOpre = g.occ_w3 || n.gG2;
+  n.proto = g.prototypes || g.last_layer || n.gF || n.gOpre;
+  return n;
+}
 
 // ---- prototype stage (proto_stage.cu): cosine -> (.+1)/2 -> logits -> 1-s -> running argmin keys ----
 int launch_proto_stage(const float* feats /*[N,P,D]*/, const float* protos, const float* last_layer, int N, int P,

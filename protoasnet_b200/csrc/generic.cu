@@ -310,7 +310,8 @@ __global__ void sign_kernel(float* __restrict__ gO, const float* __restrict__ gO
 
 // Cosine / similarity / logits backward.  One block per prototype p, looping over the clips of the chunk:
 //   gsim = gSim[n,p] - gDist[n,p] + sum_k gLogits[n,k] Wl[k,p];  gcos = gsim / 2
-//   gFE[n,p,:] = (cosine's gradient) + gFEin[n,p,:], gV[p,:] += ..., gWl[k,p] += gLogits[n,k] * sim[n,p]
+//   gFE[n,p,:] = (cosine's gradient) + gFEin[n,p,:], gV[p,:] += ..., gWl[k,p] += gLogits[n,k] * sim[n,p]  (gV, gWl may be
+//   NULL: not wanted)
 __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict__ FE, const float* __restrict__ protos,
                                                         const float* __restrict__ last_layer, const float* __restrict__ gLogits,
                                                         const float* __restrict__ gSim, const float* __restrict__ gDist,
@@ -358,18 +359,20 @@ __global__ void __launch_bounds__(256) proto_bwd_kernel(const float* __restrict_
       for (int k = 0; k < K; ++k) gs = fmaf(gLogits[(size_t)n * K + k], last_layer[(size_t)k * P + p], gs);
     const float gcos = 0.5f * gs;
     // the block owns column p of gWl: no other block writes it, so each clip adds its terms in place (any K)
-    if (gLogits)
-      for (int k = tid; k < K; k += 256) gWl[(size_t)k * P + p] += gLogits[(size_t)n * K + k] * sim;
+    if (gLogits && gWl)
+      for (int k = tid; k < K; k += 256) gWl[(size_t)k * P + p] = fmaf(gLogits[(size_t)n * K + k], sim, gWl[(size_t)k * P + p]);
     // cos = <f, v> / (nf nv); nf, nv constants when clamped
     const float inv = 1.0f / (nf * nv);
     const float cf = f_clamped ? 0.f : cosv / (nf * nf);
     const float cv = v_clamped ? 0.f : cosv / (nv * nv);
     const size_t row = ((size_t)n * P + p) * D;
+    // roundings spelled out: the compiler keeps a loop copy per `gV` case and would contract each its own way, so gFE
+    // would depend on whether gV is wanted
     for (int d = tid; d < D; d += 256) {
-      float gf = gcos * (v[d] * inv - cf * f[d]);
-      if (gFEin) gf += gFEin[row + d];
+      float gf = __fmul_rn(gcos, fmaf(v[d], inv, -__fmul_rn(cf, f[d])));
+      if (gFEin) gf = __fadd_rn(gf, gFEin[row + d]);
       gFE[row + d] = gf;
-      gV[(size_t)p * D + d] += gcos * (f[d] * inv - cv * v[d]);
+      if (gV) gV[(size_t)p * D + d] = fmaf(gcos, fmaf(f[d], inv, -__fmul_rn(cv, v[d])), gV[(size_t)p * D + d]);
     }
   }
 }
@@ -402,8 +405,10 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
   // strides of the feature map seen as B[k = channel][n = voxel] per clip
   const long long x_sk = d.layout == PASN_LAYOUT_NSC ? 1 : S, x_sn = d.layout == PASN_LAYOUT_NSC ? C : 1;
 
-  // gW[o][c] += sum_b sum_s gY[b][o][s] * X[b][c][s]
+  const BwdNeeds need = bwd_needs(g, gX);
+  // gW[o][c] += sum_b sum_s gY[b][o][s] * X[b][c][s]  (gW NULL: not wanted)
   auto wgrad = [&](const float* gY, int O_, const void* X, bool x_is_input, int Cin, float* gW, int nb) -> int {
+    if (!gW) return PASN_OK;
     GemmArgs a{};
     a.A = gY; a.B = X; a.C = gW; a.accumulate = 1; a.reduce_batch = 1; a.nbatch = nb;
     a.M = O_; a.N = Cin; a.K = S;
@@ -448,7 +453,7 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
                                         gFEin ? gFEin + (size_t)n0 * PD : nullptr, nb, P, D, K, gFE, g.prototypes, g.last_layer);
     PASN_LAUNCH_CHECK();
     count_launch();
-    {  // gO[b][p][s] = sum_d gFE[b][p][d] F[b][d][s]
+    if (need.gOpre) {  // gO[b][p][s] = sum_d gFE[b][p][d] F[b][d][s]
       GemmArgs a{};
       a.A = gFE; a.B = F; a.C = gO; a.nbatch = nb;
       a.M = P; a.N = S; a.K = D;
@@ -457,7 +462,7 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
       a.c_sb = (long long)PS; a.c_sm = S; a.c_sn = 1;
       if ((rc = launch_gemm(a, false, st))) return rc;
     }
-    {  // gF[b][d][s] = sum_p gFE[b][p][d] O[b][p][s]
+    if (need.gF) {  // gF[b][d][s] = sum_p gFE[b][p][d] O[b][p][s]
       GemmArgs a{};
       a.A = gFE; a.B = O; a.C = gF; a.nbatch = nb;
       a.M = D; a.N = S; a.K = P;
@@ -466,7 +471,7 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
       a.c_sb = (long long)DS; a.c_sm = S; a.c_sn = 1;
       if ((rc = launch_gemm(a, false, st))) return rc;
     }
-    {
+    if (need.gOpre) {
       const long long n = (long long)nb * PS;
       sign_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(gO, gOcc ? gOcc + (size_t)n0 * PS : nullptr, Opre, n);
       PASN_LAUNCH_CHECK();
@@ -475,15 +480,15 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
     // ---- add-on branch: F = W2 H1 + b2, H1 = relu(W1 x + b1)
     if ((rc = wgrad(gF, D, H1, false, D, g.addon_w2, nb))) return rc;
     if ((rc = rowsum(gF, g.addon_b2, D, nb))) return rc;
-    if ((rc = dgrad(w.addon_w2, D, D, gF, gH1, H1, 0, nb))) return rc;
+    if (need.gH1 && (rc = dgrad(w.addon_w2, D, D, gF, gH1, H1, 0, nb))) return rc;
     if ((rc = wgrad(gH1, D, x, true, C, g.addon_w1, nb))) return rc;
     if ((rc = rowsum(gH1, g.addon_b1, D, nb))) return rc;
     // ---- occurrence branch: Opre = W5 G2, G2 = relu(W4 G1 + b4), G1 = relu(W3 x + b3)
     if ((rc = wgrad(gO, P, G2, false, D2, g.occ_w3, nb))) return rc;
-    if ((rc = dgrad(w.occ_w3, P, D2, gO, gG2, G2, 0, nb))) return rc;
+    if (need.gG2 && (rc = dgrad(w.occ_w3, P, D2, gO, gG2, G2, 0, nb))) return rc;
     if ((rc = wgrad(gG2, D2, G1, false, D, g.occ_w2, nb))) return rc;
     if ((rc = rowsum(gG2, g.occ_b2, D2, nb))) return rc;
-    if ((rc = dgrad(w.occ_w2, D2, D, gG2, gG1, G1, 0, nb))) return rc;
+    if (need.gG1 && (rc = dgrad(w.occ_w2, D2, D, gG2, gG1, G1, 0, nb))) return rc;
     if ((rc = wgrad(gG1, D, x, true, C, g.occ_w1, nb))) return rc;
     if ((rc = rowsum(gG1, g.occ_b1, D, nb))) return rc;
     // ---- feature-map gradient (fp32, [N][C][S])
@@ -494,6 +499,16 @@ int generic_head_backward(const void* feat, const pasn_weights& w, const pasn_di
     }
   }
   return PASN_OK;
+}
+
+int generic_last_layer_backward(const float* gL, const float* sim, int N, int P, int K, float* gWl, cudaStream_t st) {
+  GemmArgs a{};
+  a.A = gL; a.B = sim; a.C = gWl; a.accumulate = 1; a.nbatch = 1;
+  a.M = K; a.N = P; a.K = N;
+  a.a_sm = 1; a.a_sk = K;   // A[m = k][kk = n] = gL[n][k]
+  a.b_sk = P; a.b_sn = 1;
+  a.c_sm = P; a.c_sn = 1;
+  return launch_gemm(a, false, st);
 }
 
 }  // namespace pasn

@@ -668,8 +668,8 @@ __global__ void __launch_bounds__(256) proto_bwd_rows_kernel(const float* __rest
     if (lane == 0) rs[r] = make_float4(gcos * inv, gcos * cv, (cosv + 1.0f) * 0.5f, 0.f);
   }
 }
-// part 2: gV[p,:] += sum_n a[n,p] FE[n,p,:] - (sum_n b[n,p]) v[p,:];  gWl[k,p] += sum_n gLogits[n,k] sim[n,p].
-// grid (P, slices of the clip range); every slice adds its share with atomics
+// part 2: gV[p,:] += sum_n a[n,p] FE[n,p,:] - (sum_n b[n,p]) v[p,:];  gWl[k,p] += sum_n gLogits[n,k] sim[n,p] (either
+// output may be NULL: not wanted).  grid (P, slices of the clip range); every slice adds its share with atomics
 __global__ void __launch_bounds__(256) proto_bwd_reduce_kernel(const float* __restrict__ FE, const float* __restrict__ protos,
                                                                const float* __restrict__ gLogits, const float4* __restrict__ rs,
                                                                int nb, int P, int D, int K, float* __restrict__ gV,
@@ -678,21 +678,23 @@ __global__ void __launch_bounds__(256) proto_bwd_reduce_kernel(const float* __re
   const int per = (nb + gridDim.y - 1) / gridDim.y;
   const int n_begin = blockIdx.y * per, n_end = min(nb, n_begin + per);
   if (n_begin >= n_end) return;
-  __shared__ float red[8];
-  float bsum = 0.f;
-  for (int n = n_begin + tid; n < n_end; n += 256) bsum += rs[(size_t)n * P + p].y;
-  bsum = warp_sum(bsum);
-  if ((tid & 31) == 0) red[tid >> 5] = bsum;
-  __syncthreads();
-  float sb = 0.f;
-  for (int i = 0; i < 8; ++i) sb += red[i];
-  for (int d = tid; d < D; d += 256) {
-    float acc = 0.f;
+  if (gV) {
+    __shared__ float red[8];
+    float bsum = 0.f;
+    for (int n = n_begin + tid; n < n_end; n += 256) bsum += rs[(size_t)n * P + p].y;
+    bsum = warp_sum(bsum);
+    if ((tid & 31) == 0) red[tid >> 5] = bsum;
+    __syncthreads();
+    float sb = 0.f;
+    for (int i = 0; i < 8; ++i) sb += red[i];
+    for (int d = tid; d < D; d += 256) {
+      float acc = 0.f;
 #pragma unroll 4
-    for (int n = n_begin; n < n_end; ++n) acc = fmaf(rs[(size_t)n * P + p].x, FE[((size_t)n * P + p) * D + d], acc);
-    atomicAdd(gV + (size_t)p * D + d, acc - sb * protos[(size_t)p * D + d]);
+      for (int n = n_begin; n < n_end; ++n) acc = fmaf(rs[(size_t)n * P + p].x, FE[((size_t)n * P + p) * D + d], acc);
+      atomicAdd(gV + (size_t)p * D + d, acc - sb * protos[(size_t)p * D + d]);
+    }
   }
-  if (gLogits)
+  if (gLogits && gWl)
     for (int k = tid; k < K; k += 256) {
       float acc = 0.f;
       for (int n = n_begin; n < n_end; ++n) acc = fmaf(gLogits[(size_t)n * K + k], rs[(size_t)n * P + p].z, acc);
@@ -813,14 +815,19 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     if (gX) cudaMemsetAsync(gX, 0, (size_t)d.N * C * S * 4, st);
     return PASN_OK;
   }
+  const BwdNeeds need = bwd_needs(gr, gX);
+  if (occ_only && !need.gOpre) return PASN_OK;   // nothing wanted from the occurrence branch
+  const bool want_w1 = gr.addon_w1 != nullptr, want_w3 = gr.occ_w1 != nullptr;
 
-  // gW[m][n] (+)= sum_t a[t][m] b[t][n] over the T tokens of the chunk
-  auto wgrad = [&](const Planes& a, int M, const Planes& bv, int N, long long T, float* dst0, int rows0, float* dst1) -> int {
+  // gW[m][n] (+)= sum_t a[t][m] b[t][n] over the T tokens of the chunk.  The token range is split as for an M_split-row
+  // output: one half of the stacked [W1; W3] gradient alone keeps the stacked call's split, and so its sums.
+  auto wgrad = [&](const Planes& a, int M, int M_split, const Planes& bv, int N, long long T, float* dst0, int rows0,
+                   float* dst1) -> int {
     const int bn = N >= 256 ? 256 : (N >= 128 ? 128 : 64);
-    const int tiles = ceil_div(M, 256) * ceil_div(N, bn) * 2;
+    const int tiles = ceil_div(M_split, 256) * ceil_div(N, bn) * 2;
     int kper;
     int parts = split_parts(T, tiles > 148 ? 148 : tiles, &kper);
-    while ((size_t)parts * M * N * 4 > b.part_bytes && parts > 1) { kper *= 2; parts = (int)((T + kper - 1) / kper); }
+    while ((size_t)parts * M_split * N * 4 > b.part_bytes && parts > 1) { kper *= 2; parts = (int)((T + kper - 1) / kper); }
     tcg::Gemm g = gemm(a.with(0, (int)T, true), bv.with(0, (int)T, true), M, N, kper, parts, bn);
     g.ka = (int)a.ld; g.kb = (int)bv.ld;   // the maps span ld columns from where the views start
     g.k_rows_per_batch = kper;
@@ -890,29 +897,31 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
                                                               gFEin ? gFEin + (size_t)n0 * P * D : nullptr, rows, P, D, d.K, GFE, RS);
       PASN_LAUNCH_CHECK();
       count_launch();
-      proto_bwd_reduce_kernel<<<dim3(P, nb >= 64 ? 16 : 1), 256, 0, st>>>(FE, w.prototypes, gLogits ? gLogits + (size_t)n0 * d.K : nullptr, RS, nb, P, D, d.K,
-                                                 gr.prototypes, gr.last_layer);
-      PASN_LAUNCH_CHECK();
-      count_launch();
+      if (gr.prototypes || gr.last_layer) {
+        proto_bwd_reduce_kernel<<<dim3(P, nb >= 64 ? 16 : 1), 256, 0, st>>>(FE, w.prototypes, gLogits ? gLogits + (size_t)n0 * d.K : nullptr, RS, nb, P, D, d.K,
+                                                   gr.prototypes, gr.last_layer);
+        PASN_LAUNCH_CHECK();
+        count_launch();
+      }
     }
     // ================= pooling backward
-    {  // gOpre[n][s][p] = ((F[n] gFE[n]^T)[s][p] + gOcc[n][p][s]) * sign(Opre[n][s][p])
+    if (need.gOpre) {  // gOpre[n][s][p] = ((F[n] gFE[n]^T)[s][p] + gOcc[n][p][s]) * sign(Opre[n][s][p])
       tcg::Gemm g = gemm(f.with((long long)S * f.ld, 0, false), gfe.with((long long)P * gfe.ld, 0, false), S, P, D, nb, pick_bn(P));
       if (gOcc) g.addin = {gOcc + (size_t)n0 * P * S, 1, (long long)P * S, (long long)S};
       g.signin = {OS, (long long)Pp, (long long)S * Pp, 0};
       g.out[0] = store(go.with((long long)S * go.ld, 0, false), Pp);
       if ((rc = tcg::launch(g, st))) return rc;
     }
-    {  // gF[n][s][d] = sum_p O[n][s][p] gFE[n][p][d]
+    if (need.gF) {  // gF[n][s][d] = sum_p O[n][s][p] gFE[n][p][d]
       tcg::Gemm g = gemm(oa.with((long long)S * oa.ld, 0, false), gfe.with((long long)P * gfe.ld, P, true), S, D, P, nb,
                          D >= 256 ? 256 : 128);
       g.out[0] = store(gf.with((long long)S * gf.ld, 0, false));
       if ((rc = tcg::launch(g, st))) return rc;
     }
     // ================= add-on branch
-    if ((rc = wgrad(gf, D, y, D, T, gr.addon_w2, D, nullptr))) return rc;     // gW2 += gF^T H1
-    if ((rc = colsum(gf, T, D, gr.addon_b2, D, nullptr))) return rc;
-    {  // gH1 = (gF W2) masked by H1 > 0   -> columns [0, D) of the [gH1 | gG1] planes
+    if (gr.addon_w2 && (rc = wgrad(gf, D, D, y, D, T, gr.addon_w2, D, nullptr))) return rc;     // gW2 += gF^T H1
+    if (gr.addon_b2 && (rc = colsum(gf, T, D, gr.addon_b2, D, nullptr))) return rc;
+    if (need.gH1) {  // gH1 = (gF W2) masked by H1 > 0   -> columns [0, D) of the [gH1 | gG1] planes
       tcg::Gemm g = gemm(gf, w2.with(0, D, true), (int)T, D, D, 1, D >= 256 ? 256 : 128);
       g.mask = {y.ptr, y.ld, 0, 0};
       g.out[0] = store(gy);
@@ -920,16 +929,16 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     }
     }   // !occ_only
     // ================= occurrence branch
-    if ((rc = wgrad(go, P, g2, D2, T, gr.occ_w3, P, nullptr))) return rc;      // gW5 += gOpre^T G2
-    {  // gG2 = (gOpre W5) masked by G2 > 0
+    if (gr.occ_w3 && (rc = wgrad(go, P, P, g2, D2, T, gr.occ_w3, P, nullptr))) return rc;      // gW5 += gOpre^T G2
+    if (need.gG2) {  // gG2 = (gOpre W5) masked by G2 > 0
       tcg::Gemm g = gemm(go, w5.with(0, P, true), (int)T, D2, P, 1, pick_bn(D2));
       g.mask = {g2.ptr, g2.ld, 0, 0};
       g.out[0] = store(gg2);
       if ((rc = tcg::launch(g, st))) return rc;
     }
-    if ((rc = wgrad(gg2, D2, y.at(D), D, T, gr.occ_w2, D2, nullptr))) return rc;   // gW4 += gG2^T G1
-    if ((rc = colsum(gg2, T, D2, gr.occ_b2, D2, nullptr))) return rc;
-    {  // gG1 = (gG2 W4) masked by G1 > 0   -> columns [D, 2D) of the [gH1 | gG1] planes
+    if (gr.occ_w2 && (rc = wgrad(gg2, D2, D2, y.at(D), D, T, gr.occ_w2, D2, nullptr))) return rc;   // gW4 += gG2^T G1
+    if (gr.occ_b2 && (rc = colsum(gg2, T, D2, gr.occ_b2, D2, nullptr))) return rc;
+    if (need.gG1) {  // gG1 = (gG2 W4) masked by G1 > 0   -> columns [D, 2D) of the [gH1 | gG1] planes
       tcg::Gemm g = gemm(gg2, w4.with(0, D2, true), (int)T, D, D2, 1, D >= 256 ? 256 : 128);
       g.mask = {y.at(D).ptr, y.ld, 0, 0};
       g.out[0] = store(gy.at(D), D);
@@ -937,11 +946,18 @@ int tiled_head_backward(const void* feat, const pasn_weights& w, const pasn_dims
     }
     // ================= first layer: g[W1; W3] += [gH1 | gG1]^T X, biases, feature-map gradient
     if (occ_only) {
-      if ((rc = wgrad(gy.at(D), D, xv, C, T, gr.occ_w1, D, nullptr))) return rc;
-      if ((rc = colsum(gy.at(D), T, D, gr.occ_b1, D, nullptr))) return rc;
-    } else {
-      if ((rc = wgrad(gy, 2 * D, xv, C, T, gr.addon_w1, D, gr.occ_w1))) return rc;
-      if ((rc = colsum(gy, T, 2 * D, gr.addon_b1, D, gr.occ_b1))) return rc;
+      if (want_w3 && (rc = wgrad(gy.at(D), D, D, xv, C, T, gr.occ_w1, D, nullptr))) return rc;
+      if (gr.occ_b1 && (rc = colsum(gy.at(D), T, D, gr.occ_b1, D, nullptr))) return rc;
+    } else {   // both halves in one call, or the wanted half alone
+      rc = PASN_OK;
+      if (want_w1 && want_w3) rc = wgrad(gy, 2 * D, 2 * D, xv, C, T, gr.addon_w1, D, gr.occ_w1);
+      else if (want_w1) rc = wgrad(gy, D, 2 * D, xv, C, T, gr.addon_w1, D, nullptr);
+      else if (want_w3) rc = wgrad(gy.at(D), D, 2 * D, xv, C, T, gr.occ_w1, D, nullptr);
+      if (rc) return rc;
+      if (gr.addon_b1 && gr.occ_b1) rc = colsum(gy, T, 2 * D, gr.addon_b1, D, gr.occ_b1);
+      else if (gr.addon_b1) rc = colsum(gy, T, D, gr.addon_b1, D, nullptr);
+      else if (gr.occ_b1) rc = colsum(gy.at(D), T, D, gr.occ_b1, D, nullptr);
+      if (rc) return rc;
     }
     if (gX) {   // gX[n][c][s] = sum_o [gH1|gG1][n,s][o] [W1;W3][o][c]   (occurrence only: the G1 half alone, gG1 [W3])
       const int bn = C >= 256 ? 256 : (C >= 128 ? 128 : 64);

@@ -183,10 +183,11 @@ _FORWARD_OUTPUTS = ("logits", "similarity", "occurrence_map")                   
 _PUSH_OUTPUTS = ("features_extracted", "distance", "occurrence_map", "logits")          # push_forward()
 
 
-def _library_backward(rt, x, upstream: Dict[str, Optional[torch.Tensor]], want_gx):
-    """pasn_head_backward_ex on (x, head parameters): returns (grad_x or None, [11 parameter gradients]).  ``upstream``
-    maps output names (the keys of _UPSTREAM) to their gradients; a missing or None entry contributes nothing.  When the
-    occurrence map's is the only one, only the occurrence branch is differentiated (compute_occurence_map)."""
+def _library_backward(rt, x, upstream: Dict[str, Optional[torch.Tensor]], want_gx, wanted):
+    """pasn_head_backward_ex on (x, head parameters): returns (grad_x or None, [11 parameter gradients, None where not
+    ``wanted``]).  ``upstream`` maps output names (the keys of _UPSTREAM) to their gradients; a missing or None entry
+    contributes nothing.  When the occurrence map's is the only one, only the occurrence branch is differentiated
+    (compute_occurence_map).  ``wanted``: 11 flags in _head_params order; the library skips the work of the others."""
     lib = _lib.load()
     m = rt.owner
     dims, xc, spatial = rt.make_dims(x, m.kernel_path)   # GENERIC keeps the CUDA-core backward, anything else lets the
@@ -194,8 +195,8 @@ def _library_backward(rt, x, upstream: Dict[str, Optional[torch.Tensor]], want_g
     with torch.cuda.device(dev), torch.no_grad():
         stream = torch.cuda.current_stream(dev).cuda_stream
         w, tensors = rt._weights_struct(m)
-        grads = [torch.zeros_like(t) for t in tensors]
-        gw = PasnGrads(*[g.data_ptr() for g in grads])
+        grads = [torch.zeros_like(t) if want else None for t, want in zip(tensors, wanted)]
+        gw = PasnGrads(*[_ptr(g) for g in grads])
         gx = torch.empty((dims.N, dims.C, dims.S), dtype=torch.float32, device=dev) if want_gx else None
 
         def prep(g, shape):
@@ -221,8 +222,25 @@ def _library_backward(rt, x, upstream: Dict[str, Optional[torch.Tensor]], want_g
     return gx, grads
 
 
-def _param_grads(grads, params, needed) -> tuple:
-    return tuple(g.reshape(p.shape) if need else None for g, p, need in zip(grads, params, needed))
+def _param_grads(grads, params) -> tuple:
+    return tuple(None if g is None else g.reshape(p.shape) for g, p in zip(grads, params))
+
+
+def _last_layer_backward(grad_logits: Optional[torch.Tensor], sim: torch.Tensor) -> Optional[torch.Tensor]:
+    """d(last_layer.weight) [K, P] = grad_logitsᵀ · sim from the forward's own similarity (pasn_last_layer_backward: one
+    kernel, nothing recomputed); None without a logits gradient."""
+    if grad_logits is None:
+        return None
+    lib = _lib.load()
+    N, P = sim.shape
+    K = grad_logits.shape[1]
+    dev = sim.device
+    with torch.cuda.device(dev), torch.no_grad():
+        gl = grad_logits.to(torch.float32).contiguous()
+        g = torch.zeros((K, P), dtype=torch.float32, device=dev)
+        _lib.check(lib.pasn_last_layer_backward(gl.data_ptr(), sim.data_ptr(), N, P, K, g.data_ptr(),
+                                                torch.cuda.current_stream(dev).cuda_stream), "pasn_last_layer_backward")
+    return g
 
 
 class _OccFunction(torch.autograd.Function):
@@ -242,28 +260,35 @@ class _OccFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_occ):
         x, *params = ctx.saved_tensors
-        gx, grads = _library_backward(ctx.rt, x, {"occurrence_map": g_occ}, ctx.needs_input_grad[1])
-        return (None, gx) + _param_grads(grads[_OCC_PARAMS], params, ctx.needs_input_grad[2:])
+        wanted = [False] * 11
+        wanted[_OCC_PARAMS] = ctx.needs_input_grad[2:]
+        gx, grads = _library_backward(ctx.rt, x, {"occurrence_map": g_occ}, ctx.needs_input_grad[1], wanted)
+        return (None, gx) + _param_grads(grads[_OCC_PARAMS], params)
 
 
 class _HeadFunction(torch.autograd.Function):
     """(features, 11 head parameters) -> the head outputs named by ``outputs`` (_FORWARD_OUTPUTS: forward()'s, or
     _PUSH_OUTPUTS: push_forward()'s): forward through the library's usual path, backward through
-    ``pasn_head_backward_ex`` with the gradient of every returned output (forward intermediates recomputed)."""
+    ``pasn_head_backward_ex`` with the gradient of every returned output (forward intermediates recomputed), for the
+    inputs that need one.  When last_layer.weight is the only one, its gradient comes from the forward's similarity
+    (kept by the forward, also when it is not an output) through pasn_last_layer_backward alone."""
 
     @staticmethod
     def forward(ctx, rt, outputs, x, *params):
         with torch.no_grad():
             r = rt.run(x, want_occ=True, want_feats="features_extracted" in outputs, want_dist="distance" in outputs)
         ctx.rt, ctx.outputs = rt, outputs
-        ctx.save_for_backward(x, *params)
+        ctx.save_for_backward(x, r["similarity"], *params)
         return tuple(r[k] for k in outputs)
 
     @staticmethod
     def backward(ctx, *grads):
-        x, *params = ctx.saved_tensors
-        gx, g = _library_backward(ctx.rt, x, dict(zip(ctx.outputs, grads)), ctx.needs_input_grad[2])
-        return (None, None, gx) + _param_grads(g, params, ctx.needs_input_grad[3:])
+        x, sim, *params = ctx.saved_tensors
+        want_gx, wanted = ctx.needs_input_grad[2], ctx.needs_input_grad[3:]
+        if wanted[10] and not want_gx and not any(wanted[:10]):   # last-layer-only stage
+            return (None, None, None) + (None,) * 10 + (_last_layer_backward(grads[ctx.outputs.index("logits")], sim),)
+        gx, g = _library_backward(ctx.rt, x, dict(zip(ctx.outputs, grads)), want_gx, wanted)
+        return (None, None, gx) + _param_grads(g, params)
 
 
 class HostPipeline:
